@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|torch_gpu]
                     [--config cfg3|cfg1|cfg2|cfg4|cfg5|k2] [--variant uniform|zipf|ragged] [--users B]
+                    [--dump-outputs DIR]
 
 Default = cfg3, the configuration the headline metric is quoted on (SURVEY.md section 8d): IRN influence-path
 generation, synthetic 1M-item catalog, history 200 => window L=201, d=128, 6 layers / 4 heads / ffn 256, reference
@@ -30,6 +31,9 @@ N=1 only) and `gpu_library_baseline` (the reference's own code on the same B200 
 --impl reference   the UNMODIFIED reference (oracle/_ref staged by __graft_entry__.build(), shims D1-D3 only) on the
                    host cores; falls back to the oracle port when the staged tree is absent.
 --impl torch_gpu   the same reference code with device='cuda' (cuBLAS/ATen, TF32 off) at the largest batch that fits.
+
+--dump-outputs DIR after the timed steps, writes what the timed path computed in its last step as DIR/<name>.npy.  The
+                   inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -209,6 +213,30 @@ def timed_steps(D: Dist, ops, step, steps, warmup, flush=None):
     kms = {k: (sum(sum(x[i].elapsed_time(x[i + 1]) for i in range(0, len(x), 2)) for x in v) / len(v), len(v) / steps)
            for k, v in timer.items()}
     return D.max(ms), launches, clocks, kms
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(args, D, arrays):
+    """--dump-outputs DIR: ``arrays`` (name -> tensor), what the timed path computed in its last step, as DIR/<name>.npy on
+    rank 0 -- float32 and float64 as they are, integer ids as float64 (exact).  All files together stay under 64 MB: an
+    array above its share is replaced by a fixed, seeded sample of its rows, whose ids go to DIR/<name>.rows.npy."""
+    if not args.dump_outputs or D.rank != 0:
+        return
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        t = torch.as_tensor(t).detach()
+        t = t.reshape(1) if t.dim() == 0 else t
+        dtype = t.dtype if t.dtype in (torch.float32, torch.float64) else torch.float64
+        row_bytes = t[0].numel() * dtype.itemsize
+        if t.shape[0] * row_bytes > share:
+            k = share // (row_bytes + 8)
+            rows = np.sort(np.random.default_rng(1234).choice(t.shape[0], k, replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+            np.save(os.path.join(args.dump_outputs, name + ".rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(args.dump_outputs, name + ".npy"), t.to(dtype).cpu().numpy())
 
 
 def roofline_blocks(alg, kms, step_ms, workload="cfg3"):
@@ -426,6 +454,10 @@ def run_cfg3(args, D):
             st["excl"] = irn.path_step(temp, users, paths, i, st["excl"])      # the product's own step (IRSNN.generate_on_device)
 
     ms, launches, clocks, kms = timed_steps(D, ops, step, args.steps, args.warmup)
+    if stepper is None:
+        dump_outputs(args, D, {"paths": paths, "windows": temp, "exclusions": st["excl"][0], "exclusion_counts": st["excl"][1]})
+    else:
+        dump_outputs(args, D, {"paths": paths, "windows": temp})
 
     # ---- end to end through the public API with HOST buffers (H2D of the batch + D2H of the paths inside)
     P_e2e = args.e2e_path_len
@@ -565,6 +597,7 @@ def run_cfg1(args, D):
             st["excl"] = irn.path_step(temp, users, paths, i, st["excl"])
 
     ms, launches, clocks, kms = timed_steps(D, ops, step, args.steps, args.warmup)
+    dump_outputs(args, D, {"paths": paths, "windows": temp, "exclusions": st["excl"][0], "exclusion_counts": st["excl"][1]})
     P = args.e2e_path_len
     sp, up = seqs.cpu().pin_memory(), users.cpu().pin_memory()
 
@@ -637,6 +670,7 @@ def run_cfg2(args, D):
         res["out"] = net.predict_topk(sd_, rd_, top_k=K, hist=sd_)
 
     ms, launches, clocks, kms = timed_steps(D, ops, step, args.steps, args.warmup)
+    dump_outputs(args, D, {"topk_scores": res["out"][0], "topk_items": res["out"][1]})
     sp, rp = seqs.pin_memory(), rats.pin_memory()
 
     def e2e_call():
@@ -719,6 +753,8 @@ def run_cfg4(args, D):
         losses.append(irn.train_batch(sd_, ud_))
 
     ms, launches, clocks, kms = timed_steps(D, ops, step, args.steps, args.warmup)
+    dump_outputs(args, D, {"loss": torch.tensor(losses[-1], dtype=torch.float64),
+                           **{"param." + k: p_ for k, p_ in net.named_parameters()}})
     sp, up = seqs.pin_memory(), users.pin_memory()
 
     def e2e_call():
@@ -852,6 +888,9 @@ def run_cfg5(args, D):
         res["caser"] = ops.score_topk_any(x, W2[1:], b2[1:], 50, None, 1)
 
     ms, launches, clocks, kms = timed_steps(D, ops, step, args.steps, args.warmup)
+    dump_outputs(args, D, {"path_probability": np.asarray(res["pp"]), "reciprocal_rank_increase": res["rr"][0],
+                           "rank_increase": res["rr"][1], "caser_topk_scores": res["caser"][0],
+                           "caser_topk_items": res["caser"][1]})
     t0 = time.perf_counter()
     ev.get_grad_in_batch(hd.clone(), nd, td, sd_, ld_)
     torch.cuda.synchronize()
@@ -944,25 +983,26 @@ def run_k2(args, D):
     for variant in ("uniform", "zipf"):
         ids, _ = synth_batch(B, cfg, g, device, variant)
 
-        def run(fn, reps=20):
-            for _ in range(3):
+        def run(fn):
+            for _ in range(args.warmup):
                 fn()
             torch.cuda.synchronize()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            for _ in range(reps):
-                fn()
+            for _ in range(args.steps):
+                last = fn()
             e1.record()
             torch.cuda.synchronize()
-            return e0.elapsed_time(e1) / reps
-        ms_g = run(lambda: ops.embed_gather_raw(ids, E, pe, math.sqrt(d)))
-        ms_s = run(lambda: ops.embed_scatter_add_raw(ids, dout, math.sqrt(d), dE, 0))
+            return e0.elapsed_time(e1) / args.steps, last
+        ms_g, gathered = run(lambda: ops.embed_gather_raw(ids, E, pe, math.sqrt(d)))
+        ms_s, _ = run(lambda: ops.embed_scatter_add_raw(ids, dout, math.sqrt(d), dE, 0))
         rows = B * L
         gb_g = rows * (8 + 8 * d) / 1e9
         gb_s = rows * (8 + 12 * d) / 1e9
         out[variant] = {"gather_ms": ms_g, "gather_GBps": gb_g / (ms_g / 1e3), "gather_frac": gb_g / (ms_g / 1e3) / pk["hbm"],
                         "scatter_add_ms": ms_s, "scatter_add_GBps": gb_s / (ms_s / 1e3), "scatter_add_frac": gb_s / (ms_s / 1e3) / pk["hbm"],
                         "distinct_ids": int(ids.unique().numel()), "rows": rows}
+    dump_outputs(args, D, {"gathered": gathered, "scatter_add_table": dE})
     # correctness of the scatter-add at the measured size: column sums survive (linearity), fp64 check on a sample of rows
     dE.zero_()
     ops.embed_scatter_add_raw(ids, dout, 1.0, dE, 0)
@@ -972,8 +1012,8 @@ def run_k2(args, D):
     if D.rank != 0:
         return None
     v = out["uniform"]
-    line = {"metric": "embedding scatter-add (K2) bandwidth", "value": v["scatter_add_GBps"], "unit": "GB/s", "n_gpus": 1, "steps": 20,
-            "warmup": 3, "ms_per_step": v["scatter_add_ms"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+    line = {"metric": "embedding scatter-add (K2) bandwidth", "value": v["scatter_add_GBps"], "unit": "GB/s", "n_gpus": 1,
+            "steps": args.steps, "warmup": args.warmup, "ms_per_step": v["scatter_add_ms"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic",
             "config": {"workload": f"k2: K1 gather and K2 scatter-add over [B={B}, L={L}] ids into a [{N}+1, {d}] fp32 table, uniform and "
                                    "Zipf(1) ids", "l2_policy": "table 512 MB > L2"},
@@ -1013,7 +1053,7 @@ def run_reference(args):
     kind = "port"
     t_all = []
     n_w = min(args.warmup, 1)
-    n = max(1, min(args.steps, 4))
+    n = max(1, args.steps)
     for i in range(n_w + n):
         off = (i % 64) * users_n
         _, dt, kind = reference_generate_cpu(cfg, state, seqs[off:off + users_n], us[off:off + users_n], steps, threads)
@@ -1053,7 +1093,7 @@ def run_torch_gpu(args):
     state = R.IntendedNet(SimpleNamespace(**cfg)).state_dict()
     g = torch.Generator().manual_seed(1234)
     seqs, us = synth_batch(args.users or 32, cfg, g, torch.device("cpu"), args.variant)
-    r = torch_gpu_reference(cfg, state, seqs, us, device, steps=max(2, min(args.steps, 4)), batch=args.users or 32)
+    r = torch_gpu_reference(cfg, state, seqs, us, device, steps=max(1, args.steps), batch=args.users or 32)
     r.pop("paths", None)
     print(json.dumps({"impl": "torch_gpu", "metric": "IRN influence-path generation throughput @1M items", "unit": "user-steps/s",
                       "value": r.get("value"), "n_gpus": 1, "higher_is_better": True, "dtype": "f32", "data": "synthetic",
@@ -1078,6 +1118,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = {"cfg3": 20, "cfg1": 20, "cfg2": 50, "cfg4": 3, "cfg5": 3, "k2": 20}[args.config]

@@ -46,7 +46,7 @@ def postpadded(B, L, n_item, g, min_len=3, max_fill=None):
     return seqs
 
 
-def irn_case(R, name, cfg, seqs, users, P, raw=None, labels=None, keep_rows=None, train=True):
+def irn_case(R, name, cfg, seqs, users, P, raw=None, labels=None, keep_rows=None, train=True, seeded=False):
     torch.manual_seed(1234)
     net = R.IntendedNet(cfg)
     net.eval()
@@ -83,6 +83,8 @@ def irn_case(R, name, cfg, seqs, users, P, raw=None, labels=None, keep_rows=None
         for k in ("item_embedder.weight", "project.weight", "project.bias", "user_mask_layer.weight",
                   "decoder.layers.0.self_attn.in_proj_weight", "decoder.layers.0.norm2.bias"):
             out["post." + k] = net.state_dict()[k].numpy().copy()         # after one Adam step
+    if seeded:
+        out = seeded_weights(out, 1234)
     np.savez_compressed(os.path.join(OUT, name + ".npz"), **out)
     print(name, {k: v.shape for k, v in out.items() if not k.startswith(("sd.", "grad.", "post."))})
 
@@ -100,12 +102,37 @@ def weight_fingerprint(sd):
     return keys, fp
 
 
+def seeded_weights(out, seed):
+    """Replace the state dict of an IRN fixture (``sd.<key>``, default initialisers under torch.manual_seed(seed)) by what
+    rebuilds it: the seed, a fingerprint of every tensor, and the two normal_-initialised embedding tables -- torch's CPU
+    normal_ stream depends on the host's vector ISA, so those cannot be rebuilt from the seed on another machine; the
+    uniform_-initialised tensors can.  Of the tables only the rows the fixture reads are kept (``rows.<key>`` ids,
+    ``sd.<key>`` values): the window items, the generated picks and PAD; the fixture's users.  That keeps fixtures at
+    catalog scale under 1 MB."""
+    sd = {k[3:]: torch.from_numpy(out.pop(k)) for k in [k for k in out if k.startswith("sd.")]}
+    keys, fp = weight_fingerprint(sd)
+    out.update(seed=np.array(seed), sd_keys=np.array(keys), sd_fingerprint=fp)
+    read = {"item_embedder.weight": np.union1d(np.union1d(out["seqs"], out["paths"].astype(np.int64)), [0]),
+            "user_embedder.weight": np.unique(out["users"])}
+    for k, ids in read.items():
+        out["rows." + k], out["sd." + k] = ids, sd[k][torch.from_numpy(ids)].numpy()
+    return out
+
+
+def sample_h_rows(out, n, seed):
+    """Keep a fixed, seeded sample of n decoder rows [B,L,d] at non-PAD positions: ``h_index`` (sorted flat b*L + position)
+    and ``h`` [n,d]."""
+    rng = np.random.default_rng(seed)
+    idx = np.sort(rng.choice(np.flatnonzero(out["seqs"].reshape(-1) != 0), n, replace=False))
+    out["h_index"], out["h"] = idx, out["h"].reshape(-1, out["h"].shape[-1])[idx]
+    return out
+
+
 def irn_cfg3_shape_case(R, name):
     """The BASELINE cfg3 decoder shape: window L=201 (200 history + objective), d=128, 4 heads, ffn 256, SIX layers;
     catalog 6000 items so that the fixture stays small.  Weights = the reference's default initialisers under
-    torch.manual_seed(1234) (what bench.py uses at N=1M).  Stored: a fingerprint of every tensor, plus the two
-    normal_-initialised embedding tables themselves (torch's CPU normal_ stream depends on the host's vector ISA, so those
-    cannot be rebuilt from the seed on another machine; the uniform_-initialised tensors can).  Full and ragged windows."""
+    torch.manual_seed(1234) (what bench.py uses at N=1M), stored as ``seeded_weights``.  Full and ragged windows; 320 of
+    the 1048 non-PAD decoder rows, all generation-row logits."""
     cfg = irn_config(n_item=6000, n_user=50, max_len=201, n_layers=6, n_heads=4, emb_dim=128, ffn_dim=256)
     g = torch.Generator().manual_seed(21)
     B, L, P = 8, 201, 4
@@ -115,23 +142,20 @@ def irn_cfg3_shape_case(R, name):
     net = R.IntendedNet(cfg)
     net.eval()
     irn = R.IRSNN(cfg, net, torch.device("cpu"))
-    keys, fp = weight_fingerprint(net.state_dict())
-    out = {"cfg": np.array([cfg.n_item, cfg.n_user, cfg.max_len, cfg.n_layers, cfg.n_heads, cfg.emb_dim,
-                            cfg.ffn_dim, cfg.u_emb_dim]),
-           "seed": np.array(1234), "sd_keys": np.array(keys), "sd_fingerprint": fp,
-           "seqs": seqs.numpy(), "users": users.numpy()}
-    for k in ("item_embedder.weight", "user_embedder.weight"):
-        out["sd." + k] = net.state_dict()[k].detach().clone().numpy()
+    out = dict(sd_arrays(net))
+    out.update(cfg=np.array([cfg.n_item, cfg.n_user, cfg.max_len, cfg.n_layers, cfg.n_heads, cfg.emb_dim,
+                             cfg.ffn_dim, cfg.u_emb_dim]), seqs=seqs.numpy(), users=users.numpy())
     targets = seqs[:, -1].clone()
     with torch.no_grad():
         h, r = net.decoding(seqs.clone(), users, return_pi=True)          # InfluentialNet.decoding
         logits = net.forward(seqs.clone(), users)                         # InfluentialNet.forward
-        out["h"] = h.numpy()                                              # every row [B,L,d]
+        out["h"] = h.numpy()                                              # [B,L,d], sampled below
         out["logits_row"] = logits[:, L - 2].numpy()                      # the row generation reads [B,N]
         out["r_u"] = r.numpy()
         out["eval_loss"] = np.array(irn.get_loss_on_eval_data(seqs, users))   # IRSNN.get_loss_on_eval_data
         p, t, hist, ne = irn.get_seq_in_batch(seqs, users, targets, max_path_len=P, gap_len=0)  # IRSNN.get_seq_in_batch
         out["paths"], out["targets"], out["n_early"] = p, t, np.array(ne)
+    out = sample_h_rows(seeded_weights(out, 1234), 320, seed=21)
     np.savez_compressed(os.path.join(OUT, name + ".npz"), **out)
     print(name, {k: v.shape for k, v in out.items()})
 
@@ -393,7 +417,7 @@ def main():
     dl = R.data_provider.DataLoaderIRS(ds, batch_size=Bm, shuffle=False, num_workers=0)
     seqs, users = next(iter(dl))                   # DataLoaderIRS collate (data_provider.py:568-575)
     cfg = irn_config(n_item=3415, n_user=6040, max_len=60, n_layers=2, n_heads=2, emb_dim=64, ffn_dim=128)
-    irn_case(R, "irn_ml1m", cfg, seqs, users, P=20, keep_rows=slice(58, 59), train=False)
+    irn_case(R, "irn_ml1m", cfg, seqs, users, P=20, keep_rows=slice(58, 59), train=False, seeded=True)
 
     evaluator_case(R, "evaluator_small")
     sas_case(R, "sas_small")

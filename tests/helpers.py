@@ -14,9 +14,36 @@ RTOL = 1e-3
 
 def load_golden(name):
     z = np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False)
+    rest = {k: z[k] for k in z.files if not k.startswith(("sd.", "rows."))}
+    if "sd_fingerprint" in z.files:
+        return seeded_state(z), rest
     sd = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd.")}
-    rest = {k: z[k] for k in z.files if not k.startswith("sd.")}
     return sd, rest
+
+
+def seeded_state(z):
+    """Rebuild the weights of a fixture stored by oracle/make_golden.py::seeded_weights: the reference's default
+    initialisers under the stored seed, through the drop-in InfluentialNet (it creates the same torch.nn modules in the
+    same order), every tensor checked bit for bit against the fingerprint the reference-side generator stored.  The two
+    normal_-initialised embedding tables come from the fixture (torch's CPU normal_ stream depends on the host's vector
+    ISA): the rows the fixture reads, NaN in every other row, so that a read of one shows in the results."""
+    from oracle.ref_shim import irn_config
+    from influentialrs_b200.irn import InfluentialNet
+    cfg = irn_config(*[int(x) for x in z["cfg"][:7]], u_emb_dim=int(z["cfg"][7]))
+    torch.manual_seed(int(z["seed"]))
+    sd = {k: v.detach().clone() for k, v in InfluentialNet(cfg).state_dict().items()}
+    keys = [str(k) for k in z["sd_keys"]]
+    assert sorted(sd.keys()) == keys
+    for i, k in enumerate(keys):
+        if "rows." + k in z.files:
+            sd[k] = torch.full_like(sd[k], float("nan"))
+            sd[k][torch.from_numpy(z["rows." + k])] = torch.from_numpy(z["sd." + k])
+            continue
+        bits = sd[k].contiguous().reshape(-1).view(torch.int32).to(torch.int64)
+        w = torch.arange(bits.numel(), dtype=torch.int64) % 8191 + 1
+        got = (int(bits.sum()), int((bits * w).sum()), bits.numel())
+        assert got == tuple(int(x) for x in z["sd_fingerprint"][i]), f"weights of {k} differ from the reference's"
+    return sd
 
 
 def max_rel(a, b):
@@ -29,28 +56,6 @@ def max_rel(a, b):
 def assert_close_rel(a, b, rtol=RTOL, what=""):
     r = max_rel(a, b)
     assert r <= rtol, f"{what}: max|a-b|/max|ref| = {r:.3e} > {rtol:g}"
-
-
-def cfg3_shape_state(g, module_cls, stored=None):
-    """Rebuild the weights of the ``irn_cfg3_shape`` fixture: the reference's default initialisers under the stored seed,
-    through ``module_cls`` (the drop-in InfluentialNet creates the same torch.nn modules in the same order), with the
-    normal_-initialised embedding tables taken from the fixture (``stored``: torch's CPU normal_ stream depends on the
-    host's vector ISA), and check the per-tensor fingerprint the reference-side generator stored -- bit for bit."""
-    from oracle.ref_shim import irn_config
-    cfg = irn_config(*[int(x) for x in g["cfg"][:7]], u_emb_dim=int(g["cfg"][7]))
-    torch.manual_seed(int(g["seed"]))
-    net = module_cls(cfg)
-    if stored:
-        net.load_state_dict(stored, strict=False)
-    sd = {k: v.detach().clone() for k, v in net.state_dict().items()}
-    keys = [str(k) for k in g["sd_keys"]]
-    assert sorted(sd.keys()) == keys
-    for i, k in enumerate(keys):
-        bits = sd[k].contiguous().reshape(-1).view(torch.int32).to(torch.int64)
-        w = torch.arange(bits.numel(), dtype=torch.int64) % 8191 + 1
-        got = (int(bits.sum()), int((bits * w).sum()), bits.numel())
-        assert got == tuple(int(x) for x in g["sd_fingerprint"][i]), f"weights of {k} differ from the reference's"
-    return cfg, net, sd
 
 
 def baseline_tail_scores(g, name):

@@ -47,6 +47,29 @@ def test_traffic_table_points_at_committed_captures():
         assert v["bytes_per_launch"] > 0 and os.path.exists(os.path.join(ROOT, v["source"]))
 
 
+def test_dump_outputs_types_sample_and_size_cap(tmp_path):
+    from types import SimpleNamespace
+    big = torch.arange(3 << 20, dtype=torch.int64).reshape(-1, 8)         # 24 MB as float64: above its quarter of 64 MB
+    arrays = {"ids": torch.tensor([[1, 2], [3, 1 << 40]]), "x": torch.rand(5), "loss": torch.tensor(0.5, dtype=torch.float64),
+              "big": big}
+    files = {}
+    for run in ("a", "b"):
+        out = tmp_path / run
+        bench.dump_outputs(SimpleNamespace(dump_outputs=str(out)), SimpleNamespace(rank=0), arrays)
+        files[run] = {p.name: np.load(p) for p in out.iterdir()}
+        assert sum(p.stat().st_size for p in out.iterdir()) <= bench.DUMP_BYTES
+    got = files["a"]
+    assert set(got) == {"ids.npy", "x.npy", "loss.npy", "big.npy", "big.rows.npy"}
+    assert got["ids.npy"].dtype == np.float64 and got["ids.npy"].tolist() == [[1, 2], [3, 1 << 40]]
+    assert got["x.npy"].dtype == np.float32 and np.array_equal(got["x.npy"], arrays["x"].numpy())
+    assert got["loss.npy"].dtype == np.float64 and got["loss.npy"].tolist() == [0.5]
+    rows = got["big.rows.npy"].astype(np.int64)
+    assert 0 < len(rows) < big.shape[0] and np.array_equal(got["big.npy"], big.numpy()[rows].astype(np.float64))
+    assert all(np.array_equal(got[k], files["b"][k]) for k in got)              # the sample is fixed
+    bench.dump_outputs(SimpleNamespace(dump_outputs=str(tmp_path / "r1")), SimpleNamespace(rank=1), arrays)
+    assert not (tmp_path / "r1").exists()                                       # rank 0 writes
+
+
 def test_reference_arm_runs_on_cpu_small():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--small", "--steps", "1",
                           "--warmup", "0"], capture_output=True, text=True, timeout=600, cwd=ROOT)
