@@ -81,15 +81,25 @@ struct Params {
 
 constexpr uint32_t kIdesc = make_idesc_bf16(BM, BN);
 
-// Rigorous bound on |s_true - s_hihi| for one bf16 MMA: each operand is rounded to nearest with relative error <= 2^-9, so a
-// product is off by <= |h_k w_k| (2^-8 + 2^-18) and the score by <= 2^-7.99 |h| |W_j| (Cauchy-Schwarz).  Two scores may
-// swap order only if they are within twice that; 2^-6.9 leaves margin for the fp32 accumulation.
-__device__ __forceinline__ float single_mma_band(float hnorm2, float wmax2) { return 0.00837f * sqrtf(hnorm2 * wmax2); }
+// Error bands, relative to sum_k |h_k w_k| <= |h| |W_j| <= |h| max_j |W_j| (Cauchy-Schwarz).  bf16 keeps 8 significant bits:
+// round to nearest has unit roundoff u = 2^-8 (1 + 2^-8 - 2^-20 rounds to 1).  tests/band_cases.py builds inputs that reach
+// each bound, tests/test_scorer_bands_cpu.py checks them against these figures.
+//
+// Single MMA (hi*hi): a product is off by <= (2u + u^2) |h_k w_k|, so a score by <= (2u + u^2) |h| |W_j| = 2^-6.99 |h| |W_j|.
+// Two scores may swap order only if they are within twice that, 2^-5.99; add for each score the fp32 accumulation of
+// <= 256 products in the tensor core (256 * 2^-23, truncating) and the engine's FMA chain (256 * 2^-24):
+// 2 (2u + u^2 + 256 * 2^-23 + 256 * 2^-24) = 0.015747, rounded up to 0.016 = 2^-5.97.
+__device__ __forceinline__ float single_mma_band(float hnorm2, float wmax2) { return 0.016f * sqrtf(hnorm2 * wmax2); }
 
-// Bound on |s_tensor_core - s_fp32_engine| for the three-MMA scheme: dropped lo*lo term and the rounding of the lo halves
-// (3 * 2^-18), fp32 accumulation of 3*128 products in the tensor core (384 * 2^-24) and the engine's own 128-term FMA chain
-// (128 * 2^-24), all relative to sum_k |h_k w_k| <= |h| |W_j|: 4.2e-5, rounded up.
-__device__ __forceinline__ float three_mma_band(float hnorm2, float wmax2) { return 5e-5f * sqrtf(hnorm2 * wmax2); }
+// Three MMAs (lo*hi + hi*lo + hi*hi): x = hi + lo + r with |lo| <= u |x| and |r| <= u^2 |x|; the dropped terms lo*lo, hi*r,
+// r*hi (+ smaller) are <= 3u^2 (1 + 2u) = 4.61e-5 of |h_k w_k| (x = 1 + 2^-8 + 2^-17 loses 3.03e-5).  Bound on
+// |s_tensor_core - s_fp32_engine| for d <= 128 (three-MMA schemes only exist there: KMAX): those terms + the fp32
+// accumulation in the tensor core, budgeted as one truncation per tcgen05.mma of K = 16 (3 * 128 / 16 * 2^-23 = 2.9e-6;
+// the accumulation probe in tests/test_gpu_scorer_bands.py measures 9.2e-7 on a B200 with worst-case inputs whose partial
+// sums all have one sign) + the engine's 128-term FMA chain (128 * 2^-24 = 7.6e-6): 5.66e-5, rounded up.
+// An arg-max compares two such scores.
+static_assert(KMAX <= 128, "three_mma_band() is derived for d <= 128");
+__device__ __forceinline__ float three_mma_band(float hnorm2, float wmax2) { return 5.7e-5f * sqrtf(hnorm2 * wmax2); }
 
 __device__ __forceinline__ float ex2f_approx(float x) {     // MUFU.EX2 (ftz): exp2(-inf) = 0
   float y;
@@ -495,8 +505,8 @@ score_tc_kernel(const Params p) {
         if (row_ok) {
           unsigned long long k0 = 0ull, k1 = 0ull, k2 = 0ull;
           if (best_c0 >= 0 && best_v > -INFINITY) {
-            float band = p.band_rel * fmaxf(1.0f, fabsf(best_v));
-            if (p.single) band += single_mma_band(hn2[row], *p.wmax2);
+            const float band = p.band_rel * fmaxf(1.0f, fabsf(best_v)) +
+                               (p.single ? single_mma_band(hn2[row], *p.wmax2) : 2.f * three_mma_band(hn2[row], *p.wmax2));
             const uint32_t flag = (best_v - fourth_v < band) ? 1u : 0u;
             k0 = pack_key(best_v, (uint32_t)best_c0 | flag);
             if (second_c0 >= 0 && second_v > -INFINITY) k1 = pack_key(second_v, (uint32_t)second_c0);
@@ -535,8 +545,8 @@ score_tc_kernel(const Params p) {
 
 // ---- exact re-scoring of the near-leaders -----------------------------------------------------------------
 // Candidates = for every (row, split, column half) the two 32-column chunks with the best tensor-core
-// chunk maxima.  Every candidate within `band` of the row's leader is re-scored column by column
-// with the fp32 FMA chain of the CUDA-core engine (excluded / out-of-range columns skipped); a flagged
+// chunk maxima.  The leader's chunk is re-scored first; every candidate whose chunk maximum is within the error bound of
+// one score below that exact score is then re-scored column by column with the fp32 FMA chain of the CUDA-core engine (excluded / out-of-range columns skipped); a flagged
 // candidate (third-best chunk of its slice inside the band) triggers an exact scan of its whole split.
 // The winner is the best exact (score desc, column asc) key.  One warp per row.
 __device__ __forceinline__ bool is_excluded(const int32_t* lst, int cnt, int64_t col) {
@@ -548,7 +558,8 @@ __device__ __forceinline__ bool is_excluded(const int32_t* lst, int cnt, int64_t
 __global__ void __launch_bounds__(256)
 rescore_finalize_kernel(const unsigned long long* __restrict__ slice_keys, int n_cand, const float* __restrict__ h,
                         int64_t ld_h, const float* __restrict__ W, const float* __restrict__ bias, int M, int64_t N, int d,
-                        int64_t item_base, float band_rel, const float* __restrict__ wmax2, const int32_t* __restrict__ excl_sorted,
+                        int64_t item_base, float band_rel, const float* __restrict__ wmax2, int single,
+                        const int32_t* __restrict__ excl_sorted,
                         const int32_t* __restrict__ excl_count, int Lx, int64_t tiles_per_split, int n_segs,
                         const float* __restrict__ ext_lead, float* __restrict__ vals, int64_t* __restrict__ items) {
   const int lane = threadIdx.x & 31;
@@ -569,12 +580,12 @@ rescore_finalize_kernel(const unsigned long long* __restrict__ slice_keys, int n
   // catalog-sharded call (phase 2): the leader is the best tensor-core score over ALL shards, so a shard that cannot hold
   // the row's winner finds no candidate inside the band and returns (-inf, -1) without reading W
   const float lead_s = ext_lead ? fmaxf(key_score(lead), ext_lead[m]) : key_score(lead);
-  float band = band_rel * fmaxf(1.0f, fabsf(lead_s));
-  if (wmax2 != nullptr) {                              // single-MMA pass: rigorous rounding-error band of this row
-    float hn = 0.f;
-    for (int kk = lane; kk < d; kk += 32) { const float x = h[(int64_t)m * ld_h + kk]; hn = fmaf(x, x, hn); }
-    band += single_mma_band(warp_sum(hn), *wmax2);
-  }
+  // rounding-error band of this row: the single-MMA or the (doubled) three-MMA bound, on top of the band_rel floor
+  float hn = 0.f;
+  for (int kk = lane; kk < d; kk += 32) { const float x = h[(int64_t)m * ld_h + kk]; hn = fmaf(x, x, hn); }
+  hn = warp_sum(hn);
+  // E bounds |s_tensor_core - s_fp32| of one score (plus the band_rel floor for the bias addition)
+  const float E = band_rel * fmaxf(1.0f, fabsf(lead_s)) + (single ? 0.5f * single_mma_band(hn, *wmax2) : three_mma_band(hn, *wmax2));
   const int32_t* lst = excl_sorted ? excl_sorted + (int64_t)m * Lx : nullptr;
   const int ecnt = excl_sorted ? excl_count[m] : 0;
   const float* hr = h + (int64_t)m * ld_h;
@@ -599,25 +610,48 @@ rescore_finalize_kernel(const unsigned long long* __restrict__ slice_keys, int n
     const unsigned long long ek = pack_key(acc, (uint32_t)col);
     best = ek > best ? ek : best;
   };
+  auto rescore = [&](unsigned long long key, int c) {   // whole warp: one candidate chunk, or its flagged segment
+    const uint32_t cf = key_col(key);
+    if (cf & 1u) {                                      // ambiguous slice: exact scan of its segment (both column halves)
+      const int split = (c / 6) / n_segs, seg = (c / 6) % n_segs;
+      const int64_t t0 = (int64_t)split * tiles_per_split + (int64_t)seg * SEG_TILES;
+      const int64_t t1 = min(t0 + SEG_TILES, (int64_t)(split + 1) * tiles_per_split);
+      const int64_t lo = t0 * BN, hi = min(t1 * BN, N);
+      for (int64_t col = lo + lane; col < hi; col += 32) exact(col);
+    } else {
+      exact((int64_t)(cf & ~31u) + lane);
+    }
+  };
+  auto warp_best = [&]() {
+    unsigned long long b = best;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const unsigned long long other = __shfl_xor_sync(0xffffffffu, b, o);
+      b = other > b ? other : b;
+    }
+    return b;
+  };
+  // The fp32 winner w scores >= any exact score L of a live column, and its chunk maximum is >= s_w - E >= L - E.  Whole
+  // catalog (phase 0): re-score the leader's chunk first, L = its best exact score (>= lead_s - E), then every candidate at
+  // or above L - E.  Phase 2 knows no exact score of the global leader: candidates at or above lead_s - 2E.
+  float thr = lead_s - 2.f * E;
+  if (!ext_lead) {
+    for (int c0 = 0; c0 < n_cand; c0 += 32) {
+      const unsigned long long mykey = (c0 + lane < n_cand) ? keys[c0 + lane] : 0ull;
+      const unsigned hit = __ballot_sync(0xffffffffu, mykey == lead);
+      if (hit) { rescore(lead, c0 + __ffs(hit) - 1); break; }
+    }
+    const unsigned long long b = warp_best();
+    if (b) thr = fmaxf(thr, key_score(b) - E);
+  }
   // 32 candidates at a time (one coalesced load), the few inside the band are then handled by the whole warp
   for (int c0 = 0; c0 < n_cand; c0 += 32) {
     const unsigned long long mykey = (c0 + lane < n_cand) ? keys[c0 + lane] : 0ull;
-    unsigned hits = __ballot_sync(0xffffffffu, mykey != 0ull && !(key_score(mykey) < lead_s - band));
+    unsigned hits = __ballot_sync(0xffffffffu, mykey != 0ull && !(key_score(mykey) < thr) && (ext_lead || mykey != lead));
     while (hits) {
       const int src = __ffs(hits) - 1;
       hits &= hits - 1;
-      const unsigned long long key = __shfl_sync(0xffffffffu, mykey, src);
-      const int c = c0 + src;
-      const uint32_t cf = key_col(key);
-      if (cf & 1u) {                                    // ambiguous slice: exact scan of its segment (both column halves)
-        const int split = (c / 6) / n_segs, seg = (c / 6) % n_segs;
-        const int64_t t0 = (int64_t)split * tiles_per_split + (int64_t)seg * SEG_TILES;
-        const int64_t t1 = min(t0 + SEG_TILES, (int64_t)(split + 1) * tiles_per_split);
-        const int64_t lo = t0 * BN, hi = min(t1 * BN, N);
-        for (int64_t col = lo + lane; col < hi; col += 32) exact(col);
-      } else {
-        exact((int64_t)(cf & ~31u) + lane);
-      }
+      rescore(__shfl_sync(0xffffffffu, mykey, src), c0 + src);
     }
   }
 #pragma unroll
@@ -765,8 +799,8 @@ rank_finalize_tc_kernel(const int* __restrict__ rank_above, const int* __restric
 }
 
 // ---- top-k (k > 1) finalisation ---------------------------------------------------------------------------------------
-// Input: the best single-MMA (hi*hi) score of every 32-column chunk of the row (MODE 3).  With E the rounding-error bound
-// of such a score (single_mma_band() is 2E plus margin):
+// Input: the best single-MMA (hi*hi) score of every 32-column chunk of the row (MODE 3).  With E the bound on
+// |s_hihi - s_fp32| of such a score, (2u + u^2) |h| max_j |W_j| plus accumulation, u = 2^-8 (single_mma_band() is 2E):
 //   * tau = the k-th largest chunk maximum.  k distinct chunks hold a column scoring >= tau on the tensor core, i.e.
 //     >= tau - E exactly, so the exact k-th best score T_k >= tau - E;
 //   * a column of the exact top-k scores >= T_k, hence >= tau - 2E on the tensor core: it lives in a chunk whose maximum is
@@ -978,7 +1012,7 @@ static int argmax_tc_run(int phase, const float* h, int64_t ld_h, const float* W
   p.timeline = g_scorer_timeline;
   p.single = (variant & 2) ? 1 : 0;
   p.wmax2 = (const float*)((const char*)prepared + (size_t)ceil_div(N, tc::BN) * p.n_chunks * tc::STAGE_BYTES);
-  // bf16x3 error: ~2^-16 relative per product over d terms, measured 2e-5 at |s|~3 (SURVEY 7): 1e-4 band
+  // floor of the band, relative to the leader's score: covers the fp32 rounding of the bias addition in both scores
   p.band_rel = 1e-4f;
   const int n_cand = p.n_splits * p.n_segs * 6;
   if (phase != 2) {
@@ -996,10 +1030,10 @@ static int argmax_tc_run(int phase, const float* h, int64_t ld_h, const float* W
     IRS_LAUNCHED();
     return 0;
   }
-  // the single-MMA error band of phase 2 uses the largest weight norm of ANY shard: the global leader may come from there
-  const float* wmax2 = p.single ? (phase == 2 ? lead + M : p.wmax2) : nullptr;
+  // the error band of phase 2 uses the largest weight norm of ANY shard: the global leader may come from there
+  const float* wmax2 = phase == 2 ? lead + M : p.wmax2;
   tc::rescore_finalize_kernel<<<(unsigned)ceil_div((int64_t)M * 32, 256), 256, 0, s>>>(
-      p.slice_keys, n_cand, h, ld_h, W, bias, M, N, d, item_base, p.band_rel, wmax2,
+      p.slice_keys, n_cand, h, ld_h, W, bias, M, N, d, item_base, p.band_rel, wmax2, p.single,
       excl_sorted, excl_count, Lx, p.tiles_per_split, p.n_segs, phase == 2 ? lead : nullptr, vals, items);
   IRS_LAUNCHED();
   return 0;
