@@ -253,7 +253,7 @@ int irs_score_argmax_tc_phase2(const float* h, int64_t ld_h, const float* W, con
  * exist).  Pass 2 (one CTA per row) = radix-select of the k-th largest chunk maximum tau, then every chunk whose maximum is
  * within the rigorous bf16 rounding bound of tau is re-scored column by column with the fp32 FMA chain of the CUDA-core
  * engine and the k best (score desc, id asc) are emitted.  `prepared` = irs_scorer_prepare_weights(W) (d <= 256).
- * replaces  softmax + topk(100) + filter + multinomial over k survivors  model/influentialRS.py:418-434 (sample=True),
+ * replaces  softmax + topk(100) + filter  model/influentialRS.py:418-434 (sample=True; irs_topk_sample then draws the pick),
  *           sort + delete_item_in_history + [:k]  model/sas.py:357-388, model/caser.py:273-299, model/baselines.py:527-550 */
 size_t irs_score_topk_tc_workspace_bytes(int M, int64_t N, int d, int k);
 int irs_score_topk_tc(const float* h, int64_t ld_h, const float* W, const void* prepared, const float* bias,
@@ -354,6 +354,25 @@ int irs_score_ce_bwd_tc(const float* h, int64_t ld_h, const float* W, const floa
  * item id asc).  G*k <= 4096. */
 int irs_topk_merge(const float* vals, const int64_t* items, int G, int M, int k,
                    float* out_vals, int64_t* out_items, void* stream);
+
+/* ---- a7 sample=True : one draw from the softmax over the k best (model/influentialRS.py:430-434) -------------------------
+ * vals/items [G, M, k] per-shard candidates in the layout of irs_topk_merge (G = 1 on one GPU) -> out_items[m], one item
+ * per row.  G*k <= 4096.  Per row m:
+ *   1. merge the G*k candidates to the best k by (score desc, item id asc), exactly as irs_topk_merge;
+ *   2. the finite survivors v_0 >= v_1 >= ... (in that order) get the weights w_i = exp(v_i - v_0), in fp64;
+ *   3. S = w_0 + w_1 + ... and C_i = w_0 + ... + w_i, both added one after another in that order (so S = C_last);
+ *   4. out = the first survivor with C_i > u*S, or the last finite survivor if rounding leaves none.
+ * The draw depends only on the merged list, never on G: sharded and single-GPU picks are equal.
+ * u is a 53-bit uniform in [0, 1), a pure function of (seed, step, row_key[m]); with 64-bit unsigned wrap-around,
+ * phi = 0x9E3779B97F4A7C15 and fmix64 the murmur3 finaliser
+ *   (x ^= x >> 33; x *= 0xff51afd7ed558ccd; x ^= x >> 33; x *= 0xc4ceb9fe1a85ec53; x ^= x >> 33):
+ *     x = fmix64(seed + phi * (step + 1));  x = fmix64(x + phi * (row_key[m] + 1));  u = (x >> 11) * 2^-53
+ * (step and row_key as two's-complement 64-bit words).  Edge rows: no finite candidate (every item excluded) -> -1, what
+ * the arg-max returns; any candidate carrying the overflow marker (NaN score or item -2) of irs_score_topk -> -2.
+ * replaces  softmax + multinomial over the k survivors (torch's RNG)  model/influentialRS.py:430-434 */
+int irs_topk_sample(const float* vals, const int64_t* items, int G, int M, int k,
+                    unsigned long long seed, int64_t step, const int64_t* row_key,
+                    int64_t* out_items, void* stream);
 
 /* ---- a7 window update (device-side, no host sync) ---------------------------------------------
  * seq[b,:] <- [seq[b,1:L-1], next[b], seq[b,L-1]];  paths[b,step] = (float)next[b]

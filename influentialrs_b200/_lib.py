@@ -68,6 +68,7 @@ SIGNATURES = {
     "irs_score_ce_bwd_tc_workspace_bytes": (_z, [_i, _l, _i]),
     "irs_score_ce_bwd_tc": (_i, [_p, _l, _p, _p, _p, _p, _f, _p, _p, _p, _i, _l, _i, _p, _z, _p]),
     "irs_topk_merge": (_i, [_p, _p, _i, _i, _i, _p, _p, _p]),
+    "irs_topk_sample": (_i, [_p, _p, _i, _i, _i, C.c_uint64, _l, _p, _p, _p]),
     "irs_window_shift": (_i, [_p, _p, _p, _i, _i, _i, _i, _p]),
 }
 

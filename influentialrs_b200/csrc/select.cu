@@ -196,11 +196,15 @@ rank_finalize_kernel(const int* __restrict__ rank_count, const int* __restrict__
 }
 
 // ---- shard merge --------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256)
-topk_merge_kernel(const float* __restrict__ vals, const int64_t* __restrict__ items, int G, int M, int k, int P,
-                  float* __restrict__ out_vals, int64_t* __restrict__ out_items) {
-  extern __shared__ unsigned long long sk[];
-  const int m = blockIdx.x;
+// Row m of the [G, M, k] per-shard candidates as keys sorted by (score desc, item id asc) in sk[0..P); candidates with a
+// negative item id or a NaN score become 0 (sorted last).  With `marker` non-null, *marker (shared) ends up 1 iff one of
+// the row's candidates is the overflow marker (NaN, -2) of irs_score_topk.  Every thread of the block calls this.
+__device__ void merge_row_candidates(const float* __restrict__ vals, const int64_t* __restrict__ items, int G, int M, int k,
+                                     int P, int m, unsigned long long* sk, int* marker) {
+  if (marker) {
+    if (threadIdx.x == 0) *marker = 0;
+    __syncthreads();
+  }
   for (int t = threadIdx.x; t < P; t += blockDim.x) {
     unsigned long long key = 0ull;
     if (t < G * k) {
@@ -208,15 +212,71 @@ topk_merge_kernel(const float* __restrict__ vals, const int64_t* __restrict__ it
       const int64_t it = items[((int64_t)g * M + m) * k + j];
       const float v = vals[((int64_t)g * M + m) * k + j];
       if (it >= 0 && it <= 0xfffffffell && !(v != v)) key = pack_key(v, (uint32_t)it);   // item id as the column
+      else if (marker && (it == -2 || v != v)) *marker = 1;   // racing threads all store 1; the sort's barriers publish it
     }
     sk[t] = key;
   }
-  block_bitonic_desc(sk, P);
+  block_bitonic_desc(sk, P);                    // starts and ends with a barrier: *marker is final on return
+}
+
+__global__ void __launch_bounds__(256)
+topk_merge_kernel(const float* __restrict__ vals, const int64_t* __restrict__ items, int G, int M, int k, int P,
+                  float* __restrict__ out_vals, int64_t* __restrict__ out_items) {
+  extern __shared__ unsigned long long sk[];
+  const int m = blockIdx.x;
+  merge_row_candidates(vals, items, G, M, k, P, m, sk, nullptr);
   for (int t = threadIdx.x; t < k; t += blockDim.x) {
     const unsigned long long key = sk[t];
     out_vals[(int64_t)m * k + t] = key ? key_score(key) : -INFINITY;
     out_items[(int64_t)m * k + t] = key ? (int64_t)key_col(key) : -1;
   }
+}
+
+// ---- top-k sampling (one draw from the softmax over the merged k best) -----------------------------------
+__device__ __forceinline__ unsigned long long fmix64(unsigned long long x) {      // murmur3 finaliser
+  x ^= x >> 33; x *= 0xff51afd7ed558ccdull; x ^= x >> 33; x *= 0xc4ceb9fe1a85ec53ull; x ^= x >> 33;
+  return x;
+}
+
+__global__ void __launch_bounds__(256)
+topk_sample_kernel(const float* __restrict__ vals, const int64_t* __restrict__ items, int G, int M, int k, int P,
+                   unsigned long long seed, int64_t step, const int64_t* __restrict__ row_key, int64_t* __restrict__ out_items) {
+  extern __shared__ unsigned long long sk[];
+  __shared__ int s_marker;
+  const int m = blockIdx.x;
+  merge_row_candidates(vals, items, G, M, k, P, m, sk, &s_marker);
+  if (threadIdx.x != 0) return;
+  if (s_marker) { out_items[m] = -2; return; }
+  // the uniform: a pure function of (seed, step, row key); the header states the definition
+  const unsigned long long phi = 0x9E3779B97F4A7C15ull;
+  unsigned long long x = fmix64(seed + phi * ((unsigned long long)step + 1ull));
+  x = fmix64(x + phi * ((unsigned long long)row_key[m] + 1ull));
+  const double u = (double)(x >> 11) * 0x1.0p-53;
+  // weights exp(v_i - v_0) of the finite survivors among the k best, summed one after another in sorted order
+  double v0 = 0.0, total = 0.0;
+  int n_live = 0;
+  for (int t = 0; t < k; ++t) {
+    const unsigned long long key = sk[t];
+    if (!key) break;                                   // keys sort last: no survivor after the first empty slot
+    const float v = key_score(key);
+    if (!isfinite(v)) continue;
+    if (n_live++ == 0) v0 = (double)v;
+    total += exp((double)v - v0);
+  }
+  if (n_live == 0) { out_items[m] = -1; return; }      // every item excluded: what the arg-max returns
+  const double target = u * total;
+  double run = 0.0;
+  int64_t pick = -1;
+  for (int t = 0; t < k; ++t) {
+    const unsigned long long key = sk[t];
+    if (!key) break;
+    const float v = key_score(key);
+    if (!isfinite(v)) continue;
+    pick = (int64_t)key_col(key);                      // rounding may leave no running sum above target: the last one
+    run += exp((double)v - v0);
+    if (run > target) break;
+  }
+  out_items[m] = pick;
 }
 
 // ---- window shift ---------------------------------------------------------------------------------------
@@ -483,6 +543,21 @@ extern "C" int irs_topk_merge(const float* vals, const int64_t* items, int G, in
   if ((int64_t)G * k > 4096) return IRS_E_SHAPE;
   const int P = next_pow2(G * k);
   topk_merge_kernel<<<M, 256, (size_t)P * 8, (cudaStream_t)stream>>>(vals, items, G, M, k, P, out_vals, out_items);
+  IRS_LAUNCHED();
+  return 0;
+}
+
+extern "C" int irs_topk_sample(const float* vals, const int64_t* items, int G, int M, int k,
+                               unsigned long long seed, int64_t step, const int64_t* row_key,
+                               int64_t* out_items, void* stream) {
+  if (!vals || !items || !row_key || !out_items) return IRS_E_BADARG;
+  if (G <= 0 || M <= 0 || k <= 0) return IRS_E_BADARG;
+  if ((int64_t)G * k > 4096) return IRS_E_SHAPE;
+  const int P = next_pow2(G * k);
+  int threads = next_pow2(P / 2);                       // one compare-exchange per thread and stage
+  threads = threads < 32 ? 32 : (threads > 256 ? 256 : threads);
+  topk_sample_kernel<<<M, threads, (size_t)P * 8, (cudaStream_t)stream>>>(vals, items, G, M, k, P, seed, step, row_key,
+                                                                          out_items);
   IRS_LAUNCHED();
   return 0;
 }

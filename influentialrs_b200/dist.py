@@ -9,6 +9,9 @@ Generation  -- users are split data-parallel AND the catalog (``project`` rows) 
                collective) and merged by (score desc,
                item id asc) with irs_topk_merge, and every rank shifts every user's window (so windows
                never have to be exchanged again).  Two small collectives per step.
+               Sampled generation: every shard sends its k best per row through the same one all-gather and every
+               rank draws the pick with irs_topk_sample, a pure function of (seed, step, global row) and of the
+               merged list -- the same picks on every rank, and the same as on one GPU, with no further collective.
 Training    -- plain data parallelism: local mean-CE gradients are rescaled by the local/global row
                counts and all-reduced in one flat bucket, so the update equals the single-GPU one.
 
@@ -49,11 +52,16 @@ def unpack_candidates(packed: torch.Tensor):
 
 
 class ShardedGenerator:
-    """Catalog-sharded, user-data-parallel influence-path generation (a7 across GPUs)."""
+    """Catalog-sharded, user-data-parallel influence-path generation (a7 across GPUs).
+
+    Compute callables (injectable): ``decode_fn(windows, users) -> h``; ``score_fn(h_all, windows_all[, k])`` -> (vals,
+    items) [G*B, 1] of this shard (the arg-max), or its k best when sampling passes ``k``; ``merge_fn(vals, items)`` ->
+    best (vals, items) of the [G, G*B, k] candidates; ``sample_fn(vals, items, seed, step, row_key)`` -> one pick [G*B]
+    per row (irs_topk_sample); ``shift_fn(windows_all, nxt_all, paths_local, step, row0, n_local)``."""
 
     def __init__(self, irn, rank: int, world: int, group=None, decode_fn: Optional[Callable] = None,
                  score_fn: Optional[Callable] = None, merge_fn: Optional[Callable] = None,
-                 shift_fn: Optional[Callable] = None):
+                 shift_fn: Optional[Callable] = None, sample_fn: Optional[Callable] = None):
         self.irn, self.rank, self.world, self.group = irn, rank, world, group
         self.n_item = irn.n_item
         self.lo, self.hi = shard_bounds(self.n_item, rank, world)
@@ -67,21 +75,31 @@ class ShardedGenerator:
         self.score_fn = score_fn or self._score_cuda
         self.merge_fn = merge_fn or self._merge_cuda
         self.shift_fn = shift_fn or self._shift_cuda
+        self.sample_fn = sample_fn or self._sample_cuda
 
     # ---- default CUDA operators -------------------------------------------------------------------
     def _decode_cuda(self, windows, users):
         return self.irn.net.decoding(windows, users, last_row=windows.shape[1] - 2)
 
-    def _score_cuda(self, h_all, windows_all):
+    def _prepared(self):
+        from . import ops
+        tag = ops.weight_tag(self.irn.net.project.weight)            # re-checked every call: training between two
+        if self._prep is None or self._prep[0] != tag:                # generations must not leave a stale image behind
+            self._prep = (tag, ops.scorer_prepare_weights(self.W))
+        return self._prep[1]
+
+    def _score_cuda(self, h_all, windows_all, k=None):
         from . import ops
         if self._excl is None:          # first step of a generation; afterwards the lists are updated incrementally (step())
             self._excl = ops.sort_exclusions(windows_all[:, :-1], self.hi - self.lo, self.lo + 1)
         excl = self._excl
+        if k is not None:               # sampling: the k best of my shard for every row
+            if (ops.USE_TC_TOPK and ops.score_topk_tc_supported(self.W.shape[1], k)
+                    and self.W.shape[0] >= ops.TC_TOPK_MIN_ITEMS):
+                return ops.score_topk_tc(h_all, self.W, self._prepared(), self.b, k, excl, self.lo + 1)
+            return ops.score_topk(h_all, self.W, self.b, k, excl, self.lo + 1)
         if ops.scorer_tc_supported(self.W.shape[1]):
-            tag = ops.weight_tag(self.irn.net.project.weight)        # re-checked every call: training between two
-            if self._prep is None or self._prep[0] != tag:            # generations must not leave a stale image behind
-                self._prep = (tag, ops.scorer_prepare_weights(self.W))
-            prep = self._prep[1]
+            prep = self._prepared()
             if self.world == 1:
                 return ops.score_argmax_tc(h_all, self.W, prep, self.b, excl, self.lo + 1)
             # two phases around one max-reduction: only the shard that can hold a row's winner re-scores it exactly
@@ -93,6 +111,10 @@ class ShardedGenerator:
     def _merge_cuda(self, vals, items):
         from . import ops
         return ops.topk_merge(vals, items)
+
+    def _sample_cuda(self, vals, items, seed, step, row_key):
+        from . import ops
+        return ops.topk_sample(vals, items, seed, step, row_key)
 
     def _shift_cuda(self, windows_all, nxt_all, paths_local, step, row0, n_local):
         from . import ops
@@ -122,8 +144,10 @@ class ShardedGenerator:
         self._all = _all_gather_cat(windows_local, self.world, self.group)
         self._excl = None
 
-    def step(self, windows_local, users_local, paths_local, step: int):
-        """Advance every user by one path position.  ``windows_local`` is updated in place."""
+    def step(self, windows_local, users_local, paths_local, step: int, sample=None):
+        """Advance every user by one path position.  ``windows_local`` is updated in place.  ``sample`` = (k, seed,
+        row_key [G*B] int64 of every rank's rows) draws each pick from the softmax over the k best of the whole catalog
+        (irs_topk_sample on the gathered per-shard lists: every rank computes the same picks) instead of the arg-max."""
         B = windows_local.shape[0]
         if self._all is None or self._all.shape[0] != B * self.world:
             self.begin(windows_local)
@@ -131,20 +155,27 @@ class ShardedGenerator:
         mine = self._all[row0:row0 + B]
         h = self.decode_fn(mine, users_local)                                   # [B,d]
         h_all = _all_gather_cat(h, self.world, self.group)                      # exchange 1
-        vals, items = self.score_fn(h_all, self._all)                           # [G*B,1] over my shard
+        if sample is None:
+            vals, items = self.score_fn(h_all, self._all)                       # [G*B,1] over my shard
+        else:
+            vals, items = self.score_fn(h_all, self._all, sample[0])            # [G*B,k] over my shard
         # exchange 2: (score, item) of every user from every shard in ONE collective -- the fp32 scores travel as the
         # low halves of int64 words next to the item ids ([G, G*B, k, 2] int64)
         packed_all = _all_gather_cat(pack_candidates(vals, items).unsqueeze(0), self.world, self.group)
         vals_all, items_all = unpack_candidates(packed_all)                     # [G, G*B, k] each
-        _, best = self.merge_fn(vals_all, items_all)
-        nxt_all = best[:, 0].contiguous()
+        if sample is None:
+            _, best = self.merge_fn(vals_all, items_all)
+            nxt_all = best[:, 0].contiguous()
+        else:
+            nxt_all = self.sample_fn(vals_all, items_all, sample[1], step, sample[2]).contiguous()
         self.shift_fn(self._all, nxt_all, paths_local, step, row0, B)
         windows_local.copy_(self._all[row0:row0 + B])
 
-    def generate(self, seqs_local, users_local, max_path_len=20):
+    def generate(self, seqs_local, users_local, max_path_len=20, sample=None):
         """Paths [B_local, P] of this rank's users.  Ranks may hold different numbers of users (a ragged last batch):
         every rank pads to the largest local batch with copies of its first row (or an all-PAD window when it holds no
-        user at all) and the pad rows are dropped from the result."""
+        user at all) and the pad rows are dropped from the result.  ``sample`` = (k, seed, first_key): sampled picks,
+        rank r's row i drawing with the key first_key[r] + i (a sequence of G ints, the same on every rank)."""
         n_local = seqs_local.shape[0]
         n_max = n_local
         if self.world > 1:
@@ -158,26 +189,48 @@ class ShardedGenerator:
             windows = torch.cat([windows, fill_w.expand(n_max - n_local, -1)]).contiguous()
             users_local = torch.cat([users_local, fill_u.expand(n_max - n_local)]).contiguous()
         paths = torch.zeros((n_max, max_path_len), dtype=torch.float32, device=seqs_local.device)
+        step_sample = None
+        if sample is not None:
+            k, seed, first_key = sample
+            first = torch.tensor(list(first_key), dtype=torch.int64, device=seqs_local.device)
+            keys = (first.view(-1, 1) + torch.arange(n_max, dtype=torch.int64, device=seqs_local.device)).reshape(-1)
+            step_sample = (k, seed, keys)
         self._all = None
         with torch.no_grad():
             for i in range(max_path_len):
-                self.step(windows, users_local, paths, i)
+                self.step(windows, users_local, paths, i, step_sample)
         self._all = None
         return paths[:n_local]
 
     def get_seq_in_batch(self, seqs, users, targets, max_path_len=20, gap_len=0, sample=False, sample_k=3):
-        """Same contract as IRSNN.get_seq_in_batch (model/influentialRS.py:392-470) for this rank's users."""
-        if gap_len != 0 or sample:
-            raise NotImplementedError("sharded generation implements the default greedy, gap_len=0 path")
+        """Same contract as IRSNN.get_seq_in_batch (model/influentialRS.py:392-470) for this rank's users.
+
+        ``sample``: every rank draws one seed from torch's CPU generator (as IRSNN does, so the generators stay in step)
+        and rank 0's is used; every row draws with its index in the batch of all ranks together (the ranks' local batches
+        in rank order).  So the paths equal those of IRSNN.get_seq_in_batch(sample=True) over that whole batch under the
+        same torch seed on rank 0, whatever the number of ranks."""
+        if gap_len != 0:
+            raise NotImplementedError("sharded generation implements the gap_len=0 path (SURVEY D6)")
         # device tiles of irn.user_tile users per rank (activation memory), the same number of tiles on every rank
         tile = int(getattr(self.irn, "user_tile", 4096))
         n_local = seqs.shape[0]
         n_max = n_local
-        if self.world > 1:
+        if sample:
+            # one collective per call: every rank's batch size (-> global row keys) and rank 0's seed
+            from .irn import _draw_seed
+            mine = torch.tensor([[n_local, _draw_seed()]], dtype=torch.int64, device=seqs.device)
+            info = _all_gather_cat(mine, self.world, self.group).cpu() if self.world > 1 else mine.cpu()
+            sizes, seed = info[:, 0].tolist(), int(info[0, 1])
+            offsets = [sum(sizes[:r]) for r in range(len(sizes))]
+            n_max = max(sizes)
+        elif self.world > 1:
             t = torch.tensor([n_local], dtype=torch.int64, device=seqs.device)
             dist.all_reduce(t, op=dist.ReduceOp.MAX, group=self.group)
             n_max = int(t.item())
-        parts = [self.generate(seqs[t0:t0 + tile], users[t0:t0 + tile], max_path_len) for t0 in range(0, max(n_max, 1), tile)]
+        parts = []
+        for t0 in range(0, max(n_max, 1), tile):
+            tile_sample = (int(sample_k), seed, [o + t0 for o in offsets]) if sample else None
+            parts.append(self.generate(seqs[t0:t0 + tile], users[t0:t0 + tile], max_path_len, tile_sample))
         paths = torch.cat(parts).cpu().numpy()
         return trim_paths(paths, targets.detach().cpu().numpy(), seqs[:, :-1].detach().cpu().numpy())
 

@@ -203,6 +203,11 @@ def _decoder_stack_fused(owner, x, ids, r_u, mask_mode, last_row=None):
 USE_FUSED_CHAIN = True      # tests flip it to compare against the layer-by-layer kernels
 
 
+def _draw_seed() -> int:
+    """Seed of one sampled generation, from torch's (CPU) generator: reproducible under torch.manual_seed, no device sync."""
+    return int(torch.randint(0, 2 ** 62, (1,)).item())
+
+
 def _decoder_stack(owner, x, ids, r_u, mask_mode, last_row=None):
     """Post-norm decoder over an all-zero memory (model/influentialRS.py:67-74,172-173,189-193).
 
@@ -430,12 +435,15 @@ class IRSNN(nn.Module):
         return hit_count, rr
 
     # -- influence-path generation ----------------------------------------------------------------------
-    def path_step(self, temp, users, paths, i, excl=None, sample=False, sample_k=3, h=None):
+    def path_step(self, temp, users, paths, i, excl=None, sample=False, sample_k=3, h=None, seed=None, row_key=None):
         """ONE generation step of a tile of windows ``temp`` [b,L] (updated in place; model/influentialRS.py:412-449):
-        decode (row L-2 only in the last layer) -> fused score + window mask + arg-max (or top-k + multinomial when
-        ``sample``) -> window shift, pick recorded in ``paths[:, i]``.  ``excl`` is the sorted exclusion state of the
-        windows (built on the first call, then updated incrementally: one id slides out, the pick comes in) and is
-        returned for the next step.  No host synchronisation."""
+        decode (row L-2 only in the last layer) -> fused score + window mask + arg-max (or, when ``sample``, top-k and one
+        draw from the softmax over the k survivors) -> window shift, pick recorded in ``paths[:, i]``.  ``excl`` is the
+        sorted exclusion state of the windows (built on the first call, then updated incrementally: one id slides out,
+        the pick comes in) and is returned for the next step.  The draw is a pure function of (``seed``, step ``i``,
+        ``row_key``[r]) -- ``row_key`` [b] int64 on the device names each row (default: its index in the tile).  ``seed`` is
+        required with ``sample``: one seed held for every step of a path (generate_on_device draws it once per call from
+        torch's CPU generator).  No host synchronisation."""
         L = temp.shape[1]
         p = L - 2
         if h is None:
@@ -447,26 +455,32 @@ class IRSNN(nn.Module):
         else:
             W, beta = self.net.project.weight, self.net.project.bias
             vals, items = ops.score_topk_any(h, W, beta, sample_k, excl, 1)              # tcgen05 top-k: one pass over W
-            prob = torch.softmax(vals, dim=1)      # softmax restricted to the k survivors == renormalised probs
-            pick = torch.multinomial(prob, 1, replacement=False)
-            nxt = items.gather(1, pick)[:, 0].contiguous()
+            if seed is None:
+                raise ValueError("path_step(sample=True) needs the seed of the whole path (see generate_on_device)")
+            if row_key is None:
+                row_key = torch.arange(temp.shape[0], dtype=torch.int64, device=temp.device)
+            nxt = ops.topk_sample(vals, items, seed, i, row_key)   # softmax over the k survivors, one counter-based draw
         ops.exclusions_update(excl, temp[:, 0], nxt, self.n_item, 1)                     # before the shift: temp[:,0] slides out
         ops.window_shift(temp, nxt, paths, i)
         return excl
 
     def generate_on_device(self, seqs, users, max_path_len=20, sample=False, sample_k=3, first_h=None):
         """Device loop of get_seq_in_batch: returns paths f32 [B,P] on the device, untrimmed.  ``first_h`` [B,d]
-        (optional) is the decoder row L-2 of the unmodified windows, if the caller already has it."""
+        (optional) is the decoder row L-2 of the unmodified windows, if the caller already has it.  With ``sample`` one
+        seed is drawn per call from torch's CPU generator (``torch.manual_seed`` makes runs reproducible) and row b of
+        ``seqs`` draws with the key b at every step, so the paths do not depend on ``user_tile`` or on the device."""
         B, L = seqs.shape
         paths = torch.zeros((B, max_path_len), dtype=torch.float32, device=seqs.device)
+        seed = _draw_seed() if sample else None
         for b0 in range(0, B, self.user_tile):
             temp = seqs[b0:b0 + self.user_tile].clone()
             us = users[b0:b0 + self.user_tile]
             pt = paths[b0:b0 + self.user_tile]
+            keys = torch.arange(b0, b0 + temp.shape[0], dtype=torch.int64, device=seqs.device) if sample else None
             excl = None
             for i in range(max_path_len):
                 h = first_h[b0:b0 + self.user_tile] if (i == 0 and first_h is not None) else None
-                excl = self.path_step(temp, us, pt, i, excl, sample, sample_k, h)
+                excl = self.path_step(temp, us, pt, i, excl, sample, sample_k, h, seed, keys)
         return paths
 
     def test_batch(self, raw, seqs, users, targets, labels, top_k=20, max_path_len=20, use_h=True, sample=False, sample_k=3):

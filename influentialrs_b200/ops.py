@@ -594,6 +594,30 @@ def topk_merge(vals, items):
     return ov, oi
 
 
+@_timed("sample")
+def topk_sample(vals, items, seed: int, step: int, row_key):
+    """One draw per row from the softmax over the k best candidates (score desc, item id asc) of ``vals`` / ``items``
+    [G,M,k] (per-shard lists as all-gathered) or [M,k] (G = 1).  The draw is a pure function of (seed, step, row_key[m])
+    and of the merged list, so it does not depend on G, on the device or on how rows are tiled (include/irs_b200.h states
+    the exact definition).  Returns items [M] int64: -1 for a row with no live candidate, -2 for a row that carries the
+    overflow marker of score_topk."""
+    vals = _need(vals, torch.float32, "vals")
+    items = _need(items, torch.int64, "items")
+    row_key = _need(row_key, torch.int64, "row_key")
+    if vals.dim() == 2:
+        vals, items = vals.unsqueeze(0), items.unsqueeze(0)
+    G, M, k = vals.shape
+    if tuple(items.shape) != (G, M, k) or row_key.shape != (M,):
+        raise ValueError(f"topk_sample: items {tuple(items.shape)} and row_key {tuple(row_key.shape)} must be "
+                         f"[{G},{M},{k}] and [{M}]")
+    out = torch.empty((M,), dtype=torch.int64, device=vals.device)
+    if M == 0:
+        return out
+    check(lib().irs_topk_sample(_ptr(vals), _ptr(items), G, M, k, int(seed) & (2 ** 64 - 1), int(step), _ptr(row_key),
+                                _ptr(out), _stream()), "topk_sample")
+    return out
+
+
 def window_shift(seq, nxt, paths=None, step: int = 0) -> None:
     """In place: seq[b] <- [seq[b,1:L-1], nxt[b], seq[b,L-1]]; paths[b,step] = nxt[b]."""
     B, L = seq.shape
