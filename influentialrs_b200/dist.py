@@ -2,23 +2,26 @@
 
 Generation  -- users are split data-parallel AND the catalog (``project`` rows) is sharded: rank g owns
                item ids [lo_g+1, hi_g].  Per path step every rank decodes its own users, the decoded
-               rows are all-gathered (B*d floats per rank), each rank runs the fused scorer over ITS
-               catalog shard for ALL users (window mask applied in-kernel with item_base = lo_g+1),
-               (two phases around a max-reduction of the per-row shard leaders, so that only the shard that can hold a
-               row's winner re-scores it exactly), the per-shard (score, item) candidates are all-gathered (one
-               collective) and merged by (score desc,
-               item id asc) with irs_topk_merge, and every rank shifts every user's window (so windows
-               never have to be exchanged again).  Two small collectives per step.
+               rows are all-gathered (B*d floats per rank), each rank runs the fused arg-max over ITS
+               catalog shard for ALL users (window mask applied in-kernel with item_base = lo_g+1; on the
+               tensor cores in two phases around a MAX all-reduce of the per-row shard leaders, so that only
+               the shard that can hold a row's winner re-scores it exactly), the per-shard (score, item)
+               candidates are all-gathered (one collective) and merged by (score desc, item id asc) with
+               irs_topk_merge, and every rank shifts every user's window (so windows never have to be
+               exchanged again).  Two small collectives per step, three on the tensor cores.
                Sampled generation: every shard sends its k best per row through the same one all-gather and every
                rank draws the pick with irs_topk_sample, a pure function of (seed, step, global row) and of the
                merged list -- the same picks on every rank, and the same as on one GPU, with no further collective.
+Scoring     -- ShardedScorer: rank, log-sum-exp and top-k over a row-sharded catalog for data-parallel rows.
 Training    -- plain data parallelism: local mean-CE gradients are rescaled by the local/global row
                counts and all-reduced in one flat bucket, so the update equals the single-GPU one.
 
 The reference has only nn.DataParallel (pipeline.py:43-44), which gathers [B,L,N] logits on GPU 0.
 
-The collective plumbing is torch.distributed; the compute callables default to the CUDA operators and
-can be injected, which is how tests/test_dist_cpu.py drives the same host logic on CPU over gloo.
+The collective plumbing is torch.distributed.  The compute callables default to the dispatching scorer ops of ops.py,
+which choose the engine (tcgen05 or fp32 CUDA cores) by the same rules as on one GPU and keep the weight image of each
+shard in the same process-wide cache.  They can be injected, which is how tests/test_dist_cpu.py drives the same host
+logic on CPU over gloo (ops loads the CUDA library only at the first kernel call).
 """
 from __future__ import annotations
 
@@ -27,6 +30,8 @@ from typing import Callable, Optional
 import numpy as np
 import torch
 import torch.distributed as dist
+
+from . import ops
 
 
 def shard_bounds(n_item: int, rank: int, world: int):
@@ -68,7 +73,6 @@ class ShardedGenerator:
         W, b = irn.net.project.weight, irn.net.project.bias
         self.W = W.detach()[self.lo:self.hi]            # a deployment loads only these rows
         self.b = b.detach()[self.lo:self.hi]
-        self._prep = None                               # (weight tag, prepared image of my catalog rows)
         self._excl = None                               # sorted exclusion lists of every window for MY catalog shard
         self._all = None                                # every user's window, kept in step on every rank
         self.decode_fn = decode_fn or self._decode_cuda
@@ -81,43 +85,21 @@ class ShardedGenerator:
     def _decode_cuda(self, windows, users):
         return self.irn.net.decoding(windows, users, last_row=windows.shape[1] - 2)
 
-    def _prepared(self):
-        from . import ops
-        tag = ops.weight_tag(self.irn.net.project.weight)            # re-checked every call: training between two
-        if self._prep is None or self._prep[0] != tag:                # generations must not leave a stale image behind
-            self._prep = (tag, ops.scorer_prepare_weights(self.W))
-        return self._prep[1]
-
     def _score_cuda(self, h_all, windows_all, k=None):
-        from . import ops
         if self._excl is None:          # first step of a generation; afterwards the lists are updated incrementally (step())
             self._excl = ops.sort_exclusions(windows_all[:, :-1], self.hi - self.lo, self.lo + 1)
-        excl = self._excl
         if k is not None:               # sampling: the k best of my shard for every row
-            if (ops.USE_TC_TOPK and ops.score_topk_tc_supported(self.W.shape[1], k)
-                    and self.W.shape[0] >= ops.TC_TOPK_MIN_ITEMS):
-                return ops.score_topk_tc(h_all, self.W, self._prepared(), self.b, k, excl, self.lo + 1)
-            return ops.score_topk(h_all, self.W, self.b, k, excl, self.lo + 1)
-        if ops.scorer_tc_supported(self.W.shape[1]):
-            prep = self._prepared()
-            if self.world == 1:
-                return ops.score_argmax_tc(h_all, self.W, prep, self.b, excl, self.lo + 1)
-            # two phases around one max-reduction: only the shard that can hold a row's winner re-scores it exactly
-            lead, ws = ops.score_argmax_tc_phase1(h_all, self.W, prep, self.b, excl, self.lo + 1)
-            dist.all_reduce(lead, op=dist.ReduceOp.MAX, group=self.group)
-            return ops.score_argmax_tc_phase2(h_all, self.W, prep, self.b, excl, self.lo + 1, lead, ws)
-        return ops.score_topk(h_all, self.W, self.b, 1, excl, self.lo + 1)
+            return ops.score_topk_any(h_all, self.W, self.b, k, self._excl, self.lo + 1)
+        reduce_lead = None if self.world == 1 else (lambda t: dist.all_reduce(t, op=dist.ReduceOp.MAX, group=self.group))
+        return ops.score_argmax(h_all, self.W, self.b, self._excl, self.lo + 1, reduce_lead)
 
     def _merge_cuda(self, vals, items):
-        from . import ops
         return ops.topk_merge(vals, items)
 
     def _sample_cuda(self, vals, items, seed, step, row_key):
-        from . import ops
         return ops.topk_sample(vals, items, seed, step, row_key)
 
     def _shift_cuda(self, windows_all, nxt_all, paths_local, step, row0, n_local):
-        from . import ops
         if self._excl is not None:      # the id that slides out leaves the list, the pick enters (instead of a re-sort)
             ops.exclusions_update(self._excl, windows_all[:, 0], nxt_all, self.hi - self.lo, self.lo + 1)
         ops.window_shift(windows_all, nxt_all, None, 0)
@@ -125,9 +107,8 @@ class ShardedGenerator:
             paths_local[:, step] = nxt_all[row0:row0 + n_local].float()
 
     def invalidate_prepared(self):
-        """Forget the prepared image of this rank's catalog rows (after editing project.weight through ``.data``)."""
-        self._prep = None
-        self.irn.invalidate_prepared()
+        """Forget every cached weight image (after editing project.weight through ``.data``)."""
+        ops.invalidate_prepared()
 
     # ---- one path step ------------------------------------------------------------------------------
     def begin(self, windows_local: torch.Tensor):
@@ -255,10 +236,8 @@ class ShardedScorer:
         self.rank_id, self.world, self.group = rank, world, group
         self.n_item = W.shape[0]
         self.lo, self.hi = shard_bounds(self.n_item, rank, world)
-        self.W_full = W
         self.W = W.detach()[self.lo:self.hi]            # a deployment loads only these rows
         self.b = None if bias is None else bias.detach()[self.lo:self.hi]
-        self._prep = None
         self.select_fn = select_fn or self._select_cuda
         self.count_fn = count_fn or self._count_cuda
         self.lse_fn = lse_fn or self._lse_cuda
@@ -266,45 +245,27 @@ class ShardedScorer:
         self.merge_fn = merge_fn or self._merge_cuda
 
     # ---- default CUDA operators -------------------------------------------------------------------
-    def _prepared(self):
-        from . import ops
-        if not ops.scorer_tc_supported(self.W.shape[1]):
-            return None
-        tag = ops.weight_tag(self.W_full)
-        if self._prep is None or self._prep[0] != tag:
-            self._prep = (tag, ops.scorer_prepare_weights(self.W))
-        return self._prep[1]
-
     def invalidate_prepared(self):
-        self._prep = None
+        """Forget every cached weight image (after editing the catalog weights through ``.data``)."""
+        ops.invalidate_prepared()
 
     def _excl(self, ids_all):
-        from . import ops
         return None if ids_all is None else ops.sort_exclusions(ids_all, self.hi - self.lo, self.lo + 1)
 
     def _select_cuda(self, h_all, sel_all):
-        from . import ops
         return ops.score_select(h_all, self.W, self.b, sel_all, self.lo + 1)
 
     def _count_cuda(self, h_all, label_all, score_all, ids_all):
-        from . import ops
-        return ops.score_count_ahead(h_all, self.W, self.b, label_all, score_all, self._excl(ids_all), self.lo + 1,
-                                     prepared=self._prepared())
+        return ops.score_count_ahead(h_all, self.W, self.b, label_all, score_all, self._excl(ids_all), self.lo + 1)
 
     def _lse_cuda(self, h_all):
-        from . import ops
         sel0 = torch.zeros((h_all.shape[0], 1), dtype=torch.int64, device=h_all.device)
         return ops.score_lse_gather(h_all, self.W, self.b, sel0, self.lo + 1)[0]
 
     def _topk_cuda(self, h_all, k, ids_all):
-        from . import ops
-        prep = self._prepared() if ops.USE_TC_TOPK else None
-        if prep is not None:
-            return ops.score_topk_tc(h_all, self.W, prep, self.b, k, self._excl(ids_all), self.lo + 1)
-        return ops.score_topk(h_all, self.W, self.b, k, self._excl(ids_all), self.lo + 1)
+        return ops.score_topk_any(h_all, self.W, self.b, k, self._excl(ids_all), self.lo + 1)
 
     def _merge_cuda(self, vals, items):
-        from . import ops
         return ops.topk_merge(vals, items)
 
     # ---- plumbing ------------------------------------------------------------------------------------

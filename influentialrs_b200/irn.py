@@ -54,15 +54,14 @@ def _tc_ok(d, ffn):
     return d % 4 == 0 and ffn % 4 == 0 and d <= 256 and ffn <= 256
 
 
+def _cached(owner, key, ws, make):
+    """``make()``, derived from the weights ``ws``, cached on the module ``owner`` per weight version (ops.cached_image)."""
+    return ops.cached_image(owner.__dict__.setdefault("_tc_cache", {}), key, ws, make)
+
+
 def _prepared(owner, key, W):
-    """Weight matrix re-tiled for the tensor-core kernels, cached per weight version (ops.weight_tag)."""
-    cache = owner.__dict__.setdefault("_tc_cache", {})
-    tag = ops.weight_tag(W)
-    hit = cache.get(key)
-    if hit is None or hit[0] != tag:
-        hit = (tag, ops.linear_prepare(W.detach().contiguous()))
-        cache[key] = hit
-    return hit[1]
+    """Weight matrix re-tiled for the tensor-core kernels."""
+    return _cached(owner, key, (W,), lambda: ops.linear_prepare(W.detach().contiguous()))
 
 
 def _tc_in_proj(owner, li, sa, x):
@@ -96,18 +95,12 @@ def _tc_layer_tail(owner, li, layer, x, a, c):
     return x2.view(shape)
 
 
-def _chain_prepared(owner, li, layer, nxt):
-    """Weight stream of the fused decoder-chain kernel for layer ``li`` (+ in_proj of the next layer)."""
+def _chain_prepared(owner, key, layer, nxt):
+    """Weight stream of the fused decoder-chain kernel for ``layer`` (+ in_proj of the layer ``nxt``)."""
     ws = [layer.self_attn.out_proj.weight, layer.linear1.weight, layer.linear2.weight]
     if nxt is not None:
         ws.append(nxt.self_attn.in_proj_weight)
-    cache = owner.__dict__.setdefault("_tc_cache", {})
-    tag = ops.weight_tag(*ws)
-    hit = cache.get(("chain", li))
-    if hit is None or hit[0] != tag:
-        hit = (tag, ops.decoder_chain_prepare(*[w.detach() for w in ws]))
-        cache[("chain", li)] = hit
-    return hit[1]
+    return _cached(owner, key, ws, lambda: ops.decoder_chain_prepare(*[w.detach() for w in ws]))
 
 
 def _cross_const(owner, li, layer):
@@ -120,14 +113,9 @@ def _cross_const(owner, li, layer):
     ws = (ca.in_proj_bias, ca.out_proj.weight, ca.out_proj.bias)
     if torch.is_grad_enabled() and any(w.requires_grad for w in ws):
         return F.linear(ca.in_proj_bias[2 * d:], ca.out_proj.weight, ca.out_proj.bias)
-    cache = owner.__dict__.setdefault("_tc_cache", {})
-    tag = ops.weight_tag(*ws)
-    hit = cache.get(("cross", li))
-    if hit is None or hit[0] != tag:
-        with torch.no_grad():
-            hit = (tag, F.linear(ca.in_proj_bias[2 * d:], ca.out_proj.weight, ca.out_proj.bias).contiguous())
-        cache[("cross", li)] = hit
-    return hit[1]
+    with torch.no_grad():
+        return _cached(owner, ("cross", li), ws,
+                       lambda: F.linear(ca.in_proj_bias[2 * d:], ca.out_proj.weight, ca.out_proj.bias).contiguous())
 
 
 def _cross_rows_dropout(owner, layer, B, L, p_drop, device):
@@ -161,14 +149,7 @@ def _decoder_stack_fused(owner, x, ids, r_u, mask_mode, last_row=None):
     if use_img:
         images = ops.qkv_images_buffer(B, L, H, x.device, slot=1)
         l0 = layers[0]
-        cache = owner.__dict__.setdefault("_tc_cache", {})
-        ws = [l0.self_attn.out_proj.weight, l0.linear1.weight, l0.linear2.weight, l0.self_attn.in_proj_weight]
-        tag = ops.weight_tag(*ws)
-        hit = cache.get("chain_in0")
-        if hit is None or hit[0] != tag:
-            hit = (tag, ops.decoder_chain_prepare(*[w.detach() for w in ws]))
-            cache["chain_in0"] = hit
-        ops.in_proj_images_tc(x, hit[1], l0.self_attn.in_proj_bias, images, L, mask_mode)
+        ops.in_proj_images_tc(x, _chain_prepared(owner, "chain_in0", l0, l0), l0.self_attn.in_proj_bias, images, L, mask_mode)
         qkv = None
     else:
         qkv = _tc_in_proj(owner, 0, layers[0].self_attn, x)
@@ -187,7 +168,7 @@ def _decoder_stack_fused(owner, x, ids, r_u, mask_mode, last_row=None):
         else:
             a = ops.pim_attention(qkv, ids, r_u, H, mask_mode, W_H, W_OBJ)
         nxt = None if last else layers[li + 1]
-        x, q2 = ops.decoder_chain_tc(a, x, _chain_prepared(owner, li, layer, nxt), sa.out_proj.bias,
+        x, q2 = ops.decoder_chain_tc(a, x, _chain_prepared(owner, ("chain", li), layer, nxt), sa.out_proj.bias,
                                      layer.norm1.weight, layer.norm1.bias, c, layer.norm2.weight, layer.norm2.bias,
                                      layer.linear1.bias, layer.linear2.bias, layer.norm3.weight, layer.norm3.bias,
                                      None if last else nxt.self_attn.in_proj_bias,
@@ -343,30 +324,11 @@ class IRSNN(nn.Module):
         self.grad_sync = None        # set by dist.make_data_parallel(): all-reduce of gradients
         self.scorer = None           # dist.ShardedScorer: catalog-sharded label ranks across GPUs (SURVEY 8e row 3)
 
-    def prepared_project(self):
-        """project.weight in the tcgen05 scorer's streaming layout (ONE cache for the arg-max, rank and log-sum-exp
-        paths: ops.prepared_scorer_weights), rebuilt when the weights change; None if the embedding size is outside
-        the tensor-core kernel."""
-        W = self.net.project.weight
-        if not ops.scorer_tc_supported(W.shape[1]):
-            return None
-        return ops.prepared_scorer_weights(W)
-
     def invalidate_prepared(self):
         """Forget every cached weight image (call after editing weights through ``.data``; see ops.weight_tag)."""
         if hasattr(self.net, "invalidate_prepared"):
             self.net.invalidate_prepared()
         ops.invalidate_prepared()
-
-    def next_items(self, h, excl):
-        """Greedy pick: arg-max over the catalog of h W^T + b among items not in the window."""
-        W, beta = self.net.project.weight, self.net.project.bias
-        prep = self.prepared_project()
-        if prep is not None:
-            _, items = ops.score_argmax_tc(h, W, prep, beta, excl, 1)
-        else:
-            _, items = ops.score_topk(h, W, beta, 1, excl, 1)
-        return items[:, 0].contiguous()
 
     # -- loss ---------------------------------------------------------------------------------------
     def _ce(self, seqs, users):
@@ -450,10 +412,10 @@ class IRSNN(nn.Module):
             h = self.net.decoding(temp, users, last_row=p)                              # [b,d]
         if excl is None:
             excl = ops.sort_exclusions(temp[:, : p + 1], self.n_item, 1)
+        W, beta = self.net.project.weight, self.net.project.bias
         if not sample:
-            nxt = self.next_items(h, excl)
+            nxt = ops.score_argmax(h, W, beta, excl, 1)[1][:, 0].contiguous()          # greedy: the best item not in the window
         else:
-            W, beta = self.net.project.weight, self.net.project.bias
             vals, items = ops.score_topk_any(h, W, beta, sample_k, excl, 1)              # tcgen05 top-k: one pass over W
             if seed is None:
                 raise ValueError("path_step(sample=True) needs the seed of the whole path (see generate_on_device)")

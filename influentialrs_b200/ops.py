@@ -45,7 +45,7 @@ def _error_flag(device):
 # Every tensor-core kernel streams a re-tiled bf16 hi/lo IMAGE of its weight matrix, cached per weight version.  The
 # version tag is (data_ptr, Tensor._version, shape, epoch): optimizer steps, load_state_dict and every in-place op on
 # the parameter bump _version, but edits through ``p.data`` (p.data.copy_ / mul_ / EMA swaps / clipping) do NOT.  After
-# such an edit call ``invalidate_prepared()`` (also a method of InfluentialNet / SampleNet / IRSNN / ShardedGenerator);
+# such an edit call ``invalidate_prepared()`` (also a method of InfluentialNet / SampleNet / IRSNN / the sharded classes);
 # IRS_VERIFY_PREPARED=1 adds a checksum of the weights to the tag (one host sync per lookup: a debug mode).
 _prepared_epoch = 0
 _VERIFY_PREPARED = __import__("os").environ.get("IRS_VERIFY_PREPARED", "0") == "1"
@@ -64,6 +64,19 @@ def weight_tag(*ws):
     if _VERIFY_PREPARED:
         tag += tuple(float(w.detach().double().sum()) for w in ws)
     return tag
+
+
+def cached_image(cache: dict, key, ws, make):
+    """``make()``, a value derived from the weights ``ws`` (a re-tiled image, a folded constant), cached in ``cache`` under
+    ``key`` and rebuilt when weight_tag(*ws) changes.  An entry is (tag, value, weights): it keeps the weights referenced,
+    so while it is cached their storage cannot be freed and the address cannot come back as a different tensor with the
+    same shape and a fresh version counter (which would silently hit a stale value)."""
+    tag = weight_tag(*ws)
+    hit = cache.get(key)
+    if hit is None or hit[0] != tag:
+        hit = (tag, make(), tuple(w.detach() for w in ws))
+        cache[key] = hit
+    return hit[1]
 
 
 # bench.py sets this to a dict: kernel class -> list of (start, stop) CUDA events on the launching stream
@@ -351,6 +364,45 @@ def _rows(h):
     return h, h.stride(0)
 
 
+def _excl(excl):
+    """C arguments (sorted ids, counts, Lx) of an exclusion state from sort_exclusions; None = no exclusions."""
+    return (None, None, 0) if excl is None else (_ptr(excl[0]), _ptr(excl[1]), excl[0].shape[1])
+
+
+def _workspace(nbytes: int, like: torch.Tensor) -> torch.Tensor:
+    return torch.empty((nbytes,), dtype=torch.uint8, device=like.device)
+
+
+def _no_rows(h, k: int):
+    """(vals [0,k], items [0,k]) of a scorer call without rows: nothing to launch, whichever engine it would pick."""
+    return (torch.empty((0, k), dtype=torch.float32, device=h.device),
+            torch.empty((0, k), dtype=torch.int64, device=h.device))
+
+
+# ---- which engine scores a call ------------------------------------------------------------------------------------
+# The dispatching ops (score_argmax, score_topk_any, score_rank, score_count_ahead, score_lse_gather and the softmax-CE
+# backward) choose between the tcgen05 kernels and the fp32 CUDA-core engine with these rules and nothing else, and take
+# the tcgen05 weight image from prepared_scorer_weights.  The arg-max rule is scorer_tc_supported(d).
+# Below TC_TOPK_MIN_ITEMS the two-kernel tcgen05 top-k loses to the fp32 engine (measured r2: N=3,706 x 1,024 users, k=50:
+# 0.55 ms vs 0.14 ms -- the catalog is 15 tiles, the launch is latency; N=1M x 8,192 users, d=256: 19.6 ms vs 214 ms).
+TC_TOPK_MIN_ITEMS = 32768
+TC_THREE_MMA_MAX_D = 128    # the three-MMA (hi/lo split) kernels hold hi and lo images of h only for d <= 128
+USE_TC_TOPK = True          # top-k (k > 1) on the tensor cores where the shape allows (tests flip each flag to compare)
+USE_TC_LSE = True           # log-sum-exp over the catalog on the tensor cores when d <= TC_THREE_MMA_MAX_D
+USE_TC_RANK = True          # rank / count-ahead by counting on the tensor cores when d <= TC_THREE_MMA_MAX_D
+USE_TC_CE_BWD = True        # softmax-CE backward on the tensor cores when d <= TC_THREE_MMA_MAX_D
+
+
+def _tc_topk(d: int, k: int, N: int) -> bool:
+    # May differ between the catalog shards of one call (their sizes differ by a row): harmless, there is no collective
+    # inside the top-k and both engines return the same values, ids and tie order.
+    return USE_TC_TOPK and score_topk_tc_supported(d, k) and N >= TC_TOPK_MIN_ITEMS
+
+
+def _tc_three_mma(flag: bool, d: int) -> bool:
+    return flag and d <= TC_THREE_MMA_MAX_D
+
+
 @_timed("topk")
 def score_topk(h, W, bias, k: int = 1, excl: Optional[Tuple[torch.Tensor, torch.Tensor]] = None, item_base: int = 1):
     """Top-k (score desc, item id asc) of h W^T + bias per row among non-excluded items.
@@ -361,24 +413,18 @@ def score_topk(h, W, bias, k: int = 1, excl: Optional[Tuple[torch.Tensor, torch.
     N = W.shape[0]
     vals = torch.empty((M, k), dtype=torch.float32, device=h.device)
     items = torch.empty((M, k), dtype=torch.int64, device=h.device)
-    nbytes = lib().irs_score_topk_workspace_bytes(M, N, d, k)
-    ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
-    es, ec, Lx = (None, None, 0) if excl is None else (excl[0], excl[1], excl[0].shape[1])
-    check(lib().irs_score_topk(_ptr(h), ld, _ptr(W), _ptr(bias), item_base, _ptr(es), _ptr(ec), Lx, k,
-                               _ptr(vals), _ptr(items), M, N, d, _ptr(ws), nbytes, _stream()), "score_topk")
+    ws = _workspace(lib().irs_score_topk_workspace_bytes(M, N, d, k), h)
+    check(lib().irs_score_topk(_ptr(h), ld, _ptr(W), _ptr(bias), item_base, *_excl(excl), k,
+                               _ptr(vals), _ptr(items), M, N, d, _ptr(ws), ws.numel(), _stream()), "score_topk")
     return vals, items
-
-
-# Below this catalog size the two-kernel tcgen05 top-k loses to the fp32 engine (measured r2: N=3,706 x 1,024 users, k=50:
-# 0.55 ms vs 0.14 ms -- the catalog is 15 tiles, the launch is latency; N=1M x 8,192 users, d=256: 19.6 ms vs 214 ms).
-TC_TOPK_MIN_ITEMS = 32768
-USE_TC_TOPK = True          # top-k (k > 1) on the tensor cores where the shape allows (tests flip it to compare)
 
 
 def score_topk_any(h, W, bias, k: int = 1, excl=None, item_base: int = 1):
     """Top-k through the fastest engine that covers the shape: the tcgen05 scorer (same values, ids and tie order as the
     fp32 engine) when available, else ``score_topk`` (fp32 CUDA cores)."""
-    if USE_TC_TOPK and score_topk_tc_supported(h.shape[-1], k) and W.shape[0] >= TC_TOPK_MIN_ITEMS:
+    if h.numel() == 0:
+        return _no_rows(h, k)
+    if _tc_topk(h.shape[-1], k, W.shape[0]):
         return score_topk_tc(h, W, prepared_scorer_weights(W), bias, k, excl, item_base)
     return score_topk(h, W, bias, k, excl, item_base)
 
@@ -399,33 +445,23 @@ def score_topk_tc(h, W, prepared, bias, k: int, excl=None, item_base: int = 1):
     items = torch.empty((M, k), dtype=torch.int64, device=h.device)
     if M == 0:
         return vals, items
-    nbytes = lib().irs_score_topk_tc_workspace_bytes(M, N, d, k)
-    ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
-    es, ec, Lx = (None, None, 0) if excl is None else (excl[0], excl[1], excl[0].shape[1])
-    check(lib().irs_score_topk_tc(_ptr(h), ld, _ptr(W), _ptr(prepared), _ptr(bias), item_base, _ptr(es), _ptr(ec), Lx, k,
-                                  _ptr(vals), _ptr(items), M, N, d, _ptr(ws), nbytes, _stream()), "score_topk_tc")
+    ws = _workspace(lib().irs_score_topk_tc_workspace_bytes(M, N, d, k), h)
+    check(lib().irs_score_topk_tc(_ptr(h), ld, _ptr(W), _ptr(prepared), _ptr(bias), item_base, *_excl(excl), k,
+                                  _ptr(vals), _ptr(items), M, N, d, _ptr(ws), ws.numel(), _stream()), "score_topk_tc")
     return vals, items
 
 
-USE_TC_LSE = True           # log-sum-exp over the catalog on the tensor cores when d <= 128 (tests flip it to compare)
 _prepared_scorer_cache = {}
 
 
 def prepared_scorer_weights(W) -> torch.Tensor:
-    """W [N,d] re-tiled for the tcgen05 scorer family, cached per (address, version, shape): training changes the
-    weights every step (one extra pass over W), inference prepares once.  The entry keeps a reference to W: while it
-    is cached its storage cannot be freed, so the address cannot come back as a different tensor with the same shape
-    and a fresh version counter (which would silently hit a stale image)."""
-    key = W.data_ptr()
-    tag = weight_tag(W)
-    hit = _prepared_scorer_cache.get(key)
-    if hit is None or hit[0] != tag:
-        if len(_prepared_scorer_cache) >= 4:
-            _prepared_scorer_cache.clear()
-        Wd = W.detach()
-        hit = (tag, scorer_prepare_weights(Wd), Wd)
-        _prepared_scorer_cache[key] = hit
-    return hit[1]
+    """W [N,d] re-tiled for the tcgen05 scorer family, cached per (address, shape) and weight version (cached_image):
+    training changes the weights every step (one extra pass over W), inference prepares once.  A catalog shard W[lo:hi]
+    gets its own entry next to W's, and shares W's version counter, so an optimizer step on W reaches it too."""
+    key = (W.data_ptr(), tuple(W.shape))
+    if key not in _prepared_scorer_cache and len(_prepared_scorer_cache) >= 4:
+        _prepared_scorer_cache.clear()
+    return cached_image(_prepared_scorer_cache, key, (W,), lambda: scorer_prepare_weights(W.detach()))
 
 
 @_timed("lse")
@@ -435,25 +471,22 @@ def score_lse_gather(h, W, bias, sel, item_base: int = 1):
     W = _need(W, torch.float32, "W")
     M, d = h.shape
     N = W.shape[0]
-    sel = _need(sel.reshape(M, -1), torch.int64, "sel")
+    sel = _need(sel.reshape(M, -1 if M else sel.shape[-1]), torch.int64, "sel")      # -1 is ambiguous without rows
     s = sel.shape[1]
     lse = torch.empty((M,), dtype=torch.float32, device=h.device)
     logit = torch.empty((M, s), dtype=torch.float32, device=h.device)
-    if USE_TC_LSE and d <= 128 and M > 0:
-        prep = prepared_scorer_weights(W)
-        nbytes = lib().irs_score_lse_gather_tc_workspace_bytes(M, N, d)
-        ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
-        check(lib().irs_score_lse_gather_tc(_ptr(h), ld, _ptr(W), _ptr(prep), _ptr(bias), item_base, _ptr(sel), s, _ptr(lse),
-                                            _ptr(logit), M, N, d, _ptr(ws), nbytes, _stream()), "score_lse_gather_tc")
+    if M == 0:
         return lse, logit
-    nbytes = lib().irs_score_lse_gather_workspace_bytes(M, N, d, s)
-    ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
+    if _tc_three_mma(USE_TC_LSE, d):
+        ws = _workspace(lib().irs_score_lse_gather_tc_workspace_bytes(M, N, d), h)
+        check(lib().irs_score_lse_gather_tc(_ptr(h), ld, _ptr(W), _ptr(prepared_scorer_weights(W)), _ptr(bias), item_base,
+                                            _ptr(sel), s, _ptr(lse), _ptr(logit), M, N, d, _ptr(ws), ws.numel(), _stream()),
+              "score_lse_gather_tc")
+        return lse, logit
+    ws = _workspace(lib().irs_score_lse_gather_workspace_bytes(M, N, d, s), h)
     check(lib().irs_score_lse_gather(_ptr(h), ld, _ptr(W), _ptr(bias), item_base, _ptr(sel), s, _ptr(lse), _ptr(logit),
-                                     M, N, d, _ptr(ws), nbytes, _stream()), "score_lse_gather")
+                                     M, N, d, _ptr(ws), ws.numel(), _stream()), "score_lse_gather")
     return lse, logit
-
-
-USE_TC_RANK = True          # rank by counting on the tensor cores when d <= 128 (tests flip it to compare)
 
 
 @_timed("rank")
@@ -465,23 +498,18 @@ def score_rank(h, W, bias, label, excl=None, item_base: int = 1) -> torch.Tensor
     N = W.shape[0]
     label = _need(label.reshape(-1), torch.int64, "label")
     rank = torch.empty((M,), dtype=torch.int64, device=h.device)
-    if USE_TC_RANK and d <= 128 and M > 0:
-        prep = prepared_scorer_weights(W)
-        nbytes = lib().irs_score_rank_tc_workspace_bytes(M, N, d)
-        ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
-        es, ec, Lx = (None, None, 0) if excl is None else (excl[0], excl[1], excl[0].shape[1])
-        check(lib().irs_score_rank_tc(_ptr(h), ld, _ptr(W), _ptr(prep), _ptr(bias), item_base, _ptr(label), _ptr(es), _ptr(ec), Lx,
-                                      _ptr(rank), M, N, d, _ptr(ws), nbytes, _stream()), "score_rank_tc")
+    if M == 0:
         return rank
-    nbytes = lib().irs_score_rank_workspace_bytes(M, N, d)
-    ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
-    es, ec, Lx = (None, None, 0) if excl is None else (excl[0], excl[1], excl[0].shape[1])
-    check(lib().irs_score_rank(_ptr(h), ld, _ptr(W), _ptr(bias), item_base, _ptr(label), _ptr(es), _ptr(ec), Lx,
-                               _ptr(rank), M, N, d, _ptr(ws), nbytes, _stream()), "score_rank")
+    if _tc_three_mma(USE_TC_RANK, d):
+        ws = _workspace(lib().irs_score_rank_tc_workspace_bytes(M, N, d), h)
+        check(lib().irs_score_rank_tc(_ptr(h), ld, _ptr(W), _ptr(prepared_scorer_weights(W)), _ptr(bias), item_base,
+                                      _ptr(label), *_excl(excl), _ptr(rank), M, N, d, _ptr(ws), ws.numel(), _stream()),
+              "score_rank_tc")
+        return rank
+    ws = _workspace(lib().irs_score_rank_workspace_bytes(M, N, d), h)
+    check(lib().irs_score_rank(_ptr(h), ld, _ptr(W), _ptr(bias), item_base, _ptr(label), *_excl(excl),
+                               _ptr(rank), M, N, d, _ptr(ws), ws.numel(), _stream()), "score_rank")
     return rank
-
-
-USE_TC_CE_BWD = True       # softmax-CE backward on the tensor cores when d <= 128 (tests flip it to compare)
 
 
 class _SoftmaxCE(torch.autograd.Function):
@@ -517,11 +545,10 @@ class _SoftmaxCE(torch.autograd.Function):
 
     @staticmethod
     def _backward(h, W, bias, target, lse, gscale, d_h, d_W, d_b, M, N, d):
-        if USE_TC_CE_BWD and d <= 128:
-            nbytes = lib().irs_score_ce_bwd_tc_workspace_bytes(M, N, d)
-            ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
+        if _tc_three_mma(USE_TC_CE_BWD, d):
+            ws = _workspace(lib().irs_score_ce_bwd_tc_workspace_bytes(M, N, d), h)
             check(lib().irs_score_ce_bwd_tc(_ptr(h), h.stride(0), _ptr(W), _ptr(bias), _ptr(target), _ptr(lse), gscale,
-                                            _ptr(d_h), _ptr(d_W), _ptr(d_b), M, N, d, _ptr(ws), nbytes, _stream()),
+                                            _ptr(d_h), _ptr(d_W), _ptr(d_b), M, N, d, _ptr(ws), ws.numel(), _stream()),
                   "score_ce_bwd_tc")
             return d_h, d_W, d_b, None
         check(lib().irs_score_ce_bwd(_ptr(h), h.stride(0), _ptr(W), _ptr(bias), _ptr(target), _ptr(lse), gscale,
@@ -556,10 +583,10 @@ def score_select(h, W, bias, sel, item_base: int = 1) -> torch.Tensor:
 
 
 @_timed("rank")
-def score_count_ahead(h, W, bias, label, label_score, excl=None, item_base: int = 1, prepared=None):
+def score_count_ahead(h, W, bias, label, label_score, excl=None, item_base: int = 1):
     """(count [M] int64, label_excluded [M] int32): items of THIS catalog shard ahead of (label_score, label id); the label
-    may belong to another shard.  rank = 0 if any shard flags the label, else 1 + sum of the counts.  Tensor cores when a
-    prepared image is given (d <= 128), fp32 CUDA cores otherwise -- the same integers either way."""
+    may belong to another shard.  rank = 0 if any shard flags the label, else 1 + sum of the counts.  The engine is chosen
+    as in score_rank -- the same integers either way."""
     h, ld = _rows(h)
     W = _need(W, torch.float32, "W")
     M, d = h.shape
@@ -568,18 +595,18 @@ def score_count_ahead(h, W, bias, label, label_score, excl=None, item_base: int 
     label_score = _need(label_score.reshape(-1), torch.float32, "label_score")
     count = torch.empty((M,), dtype=torch.int64, device=h.device)
     flag = torch.empty((M,), dtype=torch.int32, device=h.device)
-    es, ec, Lx = (None, None, 0) if excl is None else (excl[0], excl[1], excl[0].shape[1])
-    if prepared is not None and USE_TC_RANK:
-        nbytes = lib().irs_score_rank_tc_workspace_bytes(M, N, d)
-        ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
-        check(lib().irs_score_count_ahead_tc(_ptr(h), ld, _ptr(W), _ptr(prepared), _ptr(bias), item_base, _ptr(label),
-                                             _ptr(label_score), _ptr(es), _ptr(ec), Lx, _ptr(count), _ptr(flag), M, N, d,
-                                             _ptr(ws), nbytes, _stream()), "score_count_ahead_tc")
+    if M == 0:
         return count, flag
-    nbytes = lib().irs_score_count_ahead_workspace_bytes(M, N, d)
-    ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
-    check(lib().irs_score_count_ahead(_ptr(h), ld, _ptr(W), _ptr(bias), item_base, _ptr(label), _ptr(label_score), _ptr(es), _ptr(ec),
-                                      Lx, _ptr(count), _ptr(flag), M, N, d, _ptr(ws), nbytes, _stream()), "score_count_ahead")
+    if _tc_three_mma(USE_TC_RANK, d):
+        ws = _workspace(lib().irs_score_rank_tc_workspace_bytes(M, N, d), h)
+        check(lib().irs_score_count_ahead_tc(_ptr(h), ld, _ptr(W), _ptr(prepared_scorer_weights(W)), _ptr(bias), item_base,
+                                             _ptr(label), _ptr(label_score), *_excl(excl), _ptr(count), _ptr(flag), M, N, d,
+                                             _ptr(ws), ws.numel(), _stream()), "score_count_ahead_tc")
+        return count, flag
+    ws = _workspace(lib().irs_score_count_ahead_workspace_bytes(M, N, d), h)
+    check(lib().irs_score_count_ahead(_ptr(h), ld, _ptr(W), _ptr(bias), item_base, _ptr(label), _ptr(label_score),
+                                      *_excl(excl), _ptr(count), _ptr(flag), M, N, d, _ptr(ws), ws.numel(), _stream()),
+          "score_count_ahead")
     return count, flag
 
 
@@ -629,7 +656,7 @@ def window_shift(seq, nxt, paths=None, step: int = 0) -> None:
 # tensor-core (tcgen05) arg-max scorer
 # ------------------------------------------------------------------------------------------------
 def scorer_prepare_weights(W) -> torch.Tensor:
-    """Re-tile the catalog matrix W [N,d] (d <= 128) into the bf16 hi/lo shared-memory image the
+    """Re-tile the catalog matrix W [N,d] (d <= 256) into the bf16 hi/lo shared-memory image the
     tcgen05 scorer streams (one 32 KB bulk copy per stage).  Do this once per weight version."""
     W = _need(W, torch.float32, "W")
     N, d = W.shape
@@ -658,12 +685,10 @@ def score_argmax_tc(h, W, prepared, bias, excl=None, item_base: int = 1, variant
     N = W.shape[0]
     vals = torch.empty((M, 1), dtype=torch.float32, device=h.device)
     items = torch.empty((M, 1), dtype=torch.int64, device=h.device)
-    nbytes = lib().irs_score_argmax_tc_workspace_bytes(M, N, d)
-    ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
-    es, ec, Lx = (None, None, 0) if excl is None else (excl[0], excl[1], excl[0].shape[1])
-    check(lib().irs_score_argmax_tc(_ptr(h), ld, _ptr(W), _ptr(prepared), _ptr(bias), item_base, _ptr(es), _ptr(ec), Lx,
-                                    _ptr(vals), _ptr(items), M, N, d, ARGMAX_VARIANT if variant is None else variant, _ptr(ws), nbytes,
-                                    _stream()), "score_argmax_tc")
+    ws = _workspace(lib().irs_score_argmax_tc_workspace_bytes(M, N, d), h)
+    check(lib().irs_score_argmax_tc(_ptr(h), ld, _ptr(W), _ptr(prepared), _ptr(bias), item_base, *_excl(excl),
+                                    _ptr(vals), _ptr(items), M, N, d, ARGMAX_VARIANT if variant is None else variant, _ptr(ws),
+                                    ws.numel(), _stream()), "score_argmax_tc")
     return vals, items
 
 
@@ -678,17 +703,15 @@ def score_argmax_tc_phase1(h, W, prepared, bias, excl=None, item_base: int = 1, 
     M, d = h.shape
     N = W.shape[0]
     lead = torch.empty((M + 1,), dtype=torch.float32, device=h.device)
-    nbytes = lib().irs_score_argmax_tc_workspace_bytes(M, N, d)
-    ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
-    es, ec, Lx = (None, None, 0) if excl is None else (excl[0], excl[1], excl[0].shape[1])
+    ws = _workspace(lib().irs_score_argmax_tc_workspace_bytes(M, N, d), h)
     global _pending_phase1
     ev = None
     if _timer is not None:
         ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
         ev[0].record()
-    check(lib().irs_score_argmax_tc_phase1(_ptr(h), ld, _ptr(W), _ptr(prepared), _ptr(bias), item_base, _ptr(es), _ptr(ec), Lx,
-                                           _ptr(lead), M, N, d, ARGMAX_VARIANT if variant is None else variant, _ptr(ws), nbytes,
-                                           _stream()), "score_argmax_tc_phase1")
+    check(lib().irs_score_argmax_tc_phase1(_ptr(h), ld, _ptr(W), _ptr(prepared), _ptr(bias), item_base, *_excl(excl),
+                                           _ptr(lead), M, N, d, ARGMAX_VARIANT if variant is None else variant, _ptr(ws),
+                                           ws.numel(), _stream()), "score_argmax_tc_phase1")
     if ev is not None:
         ev[1].record()
     _pending_phase1 = ev
@@ -704,13 +727,12 @@ def score_argmax_tc_phase2(h, W, prepared, bias, excl, item_base, lead_global, w
     lead_global = _need(lead_global, torch.float32, "lead_global")
     vals = torch.empty((M, 1), dtype=torch.float32, device=h.device)
     items = torch.empty((M, 1), dtype=torch.int64, device=h.device)
-    es, ec, Lx = (None, None, 0) if excl is None else (excl[0], excl[1], excl[0].shape[1])
     global _pending_phase1
     ev = None
     if _timer is not None:
         ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
         ev[0].record()
-    check(lib().irs_score_argmax_tc_phase2(_ptr(h), ld, _ptr(W), _ptr(prepared), _ptr(bias), item_base, _ptr(es), _ptr(ec), Lx,
+    check(lib().irs_score_argmax_tc_phase2(_ptr(h), ld, _ptr(W), _ptr(prepared), _ptr(bias), item_base, *_excl(excl),
                                            _ptr(lead_global), _ptr(vals), _ptr(items), M, N, d,
                                            ARGMAX_VARIANT if variant is None else variant, _ptr(ws), ws.numel(), _stream()),
           "score_argmax_tc_phase2")
@@ -720,6 +742,27 @@ def score_argmax_tc_phase2(h, W, prepared, bias, excl, item_base, lead_global, w
         _timer.setdefault("scorer", []).append(((_pending_phase1 or ()) + ev))
         _pending_phase1 = None
     return vals, items
+
+
+def score_argmax(h, W, bias, excl=None, item_base: int = 1, reduce_lead=None):
+    """Arg-max (k = 1) of h W^T + bias among non-excluded items: (vals [M,1], items [M,1]), the same as score_topk(k=1).
+    On the tensor cores when scorer_tc_supported(d), else on the fp32 engine.
+
+    ``reduce_lead``: W is this rank's shard of a catalog split over ranks that all score the same rows h.  The tcgen05
+    engine then runs in two phases around ``reduce_lead(lead)``, which must MAX-reduce ``lead`` over the ranks in place,
+    so that only the shard that can hold a row's winner re-scores it exactly; rows won in another shard come back as
+    (-inf, -1).  So the engine must depend on d alone, never on N: the tcgen05 branch holds that collective, and the
+    shards of one catalog differ in size by a row, so a rule on N could leave one rank out of it."""
+    if h.numel() == 0:
+        return _no_rows(h, 1)
+    if not scorer_tc_supported(h.shape[-1]):
+        return score_topk(h, W, bias, 1, excl, item_base)
+    prep = prepared_scorer_weights(W)
+    if reduce_lead is None:
+        return score_argmax_tc(h, W, prep, bias, excl, item_base)
+    lead, ws = score_argmax_tc_phase1(h, W, prep, bias, excl, item_base)
+    reduce_lead(lead)
+    return score_argmax_tc_phase2(h, W, prep, bias, excl, item_base, lead, ws)
 
 
 # ------------------------------------------------------------------------------------------------

@@ -671,14 +671,15 @@ def test_ce_backward_tensor_core_skips_negative_targets(ops):
 
 
 @pytest.mark.parametrize("tc", [False, True])
-@pytest.mark.parametrize("M,N,d,Lx,shards", [(130, 5000, 128, 60, 2), (300, 70001, 128, 40, 3), (64, 3415, 64, 0, 4), (9, 700, 30, 5, 2)])
+@pytest.mark.parametrize("M,N,d,Lx,shards", [(130, 5000, 128, 60, 2), (300, 70001, 128, 40, 3), (64, 3415, 64, 0, 4), (9, 700, 30, 5, 2),
+                                             (40, 40000, 192, 20, 3), (17, 9001, 256, 9, 2), (128, 5000, 160, 0, 4),
+                                             (9, 700, 129, 5, 2)])
 def test_sharded_rank_select_and_count_equal_unsharded(ops, M, N, d, Lx, shards, tc, monkeypatch):
     """Catalog-sharded rank (SURVEY 8e row 3), shards emulated on one GPU: label score = MAX over shards of irs_score_select,
     rank = 1 + SUM over shards of irs_score_count_ahead[_tc] -- the same integers as irs_score_rank over the whole catalog,
     with exact ties of the label straddling shard boundaries, excluded labels and uneven shards; irs_score_select is
-    bit-identical to the scorer's own label scores."""
-    if tc and d > 128:
-        pytest.skip("tensor-core scorer covers d <= 128")
+    bit-identical to the scorer's own label scores.  ``tc`` sets USE_TC_RANK; for d > 128 both count-ahead and rank take
+    the fp32 engine whatever the flag."""
     monkeypatch.setattr(ops, "USE_TC_RANK", tc)
     h, W, bias, excl = _score_case(M, N, d, max(Lx, 1), 61)
     g = _gen(62)
@@ -703,8 +704,7 @@ def test_sharded_rank_select_and_count_equal_unsharded(ops, M, N, d, Lx, shards,
     for lo, hi in bounds:
         Ws, bs = Wd[lo:hi].contiguous(), bd[lo:hi].contiguous()
         e = ops.sort_exclusions(ed, hi - lo, lo + 1) if Lx else None
-        prep = ops.scorer_prepare_weights(Ws) if tc else None
-        c, f = ops.score_count_ahead(hd, Ws, bs, ld_, score, e, lo + 1, prepared=prep)
+        c, f = ops.score_count_ahead(hd, Ws, bs, ld_, score, e, lo + 1)
         total += c
         flags += f.long()
     got = torch.where(flags > 0, torch.zeros_like(total), total + 1)

@@ -135,10 +135,12 @@ def test_rank_three_mma(ops, d, crowded, monkeypatch):
     _healthy(ops)
 
 
+@pytest.mark.parametrize("tc", [True, False])
 @pytest.mark.parametrize("d", [64, 128])
-def test_count_ahead_three_mma_across_shards(ops, d, monkeypatch):
-    """rank = 1 + sum over two catalog shards of score_count_ahead(prepared=...), label score = MAX of score_select."""
-    monkeypatch.setattr(ops, "USE_TC_RANK", True)
+def test_count_ahead_three_mma_across_shards(ops, d, tc, monkeypatch):
+    """rank = 1 + sum over two catalog shards of score_count_ahead, label score = MAX of score_select, on the tensor-core
+    count-ahead (tc) and on the fp32 engine."""
+    monkeypatch.setattr(ops, "USE_TC_RANK", tc)
     case = B.rank_three(d, False)
     h, W, b, _ = _dev(case, ops)
     lab = case.label.to(DEV)
@@ -150,7 +152,7 @@ def test_count_ahead_three_mma_across_shards(ops, d, monkeypatch):
     total = torch.zeros((case.M,), dtype=torch.int64, device=DEV)
     for lo, hi in bounds:
         Ws, bs = W[lo:hi].contiguous(), b[lo:hi].contiguous()
-        c, f = ops.score_count_ahead(h, Ws, bs, lab, score, None, lo + 1, prepared=ops.scorer_prepare_weights(Ws))
+        c, f = ops.score_count_ahead(h, Ws, bs, lab, score, None, lo + 1)
         assert int(f.sum()) == 0
         total += c
     assert torch.equal((total + 1).cpu(), case.expected)
