@@ -75,7 +75,11 @@ int irs_pif_fwd(const int64_t* users, const float* user_table, const float* w, c
  * A query row whose keys are all masked yields NaN, as torch's softmax does.
  * p_drop > 0 (training): attention-probability dropout, out_i = sum_j softmax(s)_ij m_ij V_j with m_ij in {0, 1/(1-p)}
  * a counter-based function of (seed, b*H+h, i, j) -- what nn.MultiheadAttention(dropout=p) does in train mode
- * (model/influentialRS.py:67-74); irs_pim_attn_bwd regenerates the same mask from the same (p_drop, seed). */
+ * (model/influentialRS.py:67-74); irs_pim_attn_bwd regenerates the same mask from the same (p_drop, seed).
+ * Windows of up to IRS_ATTN_MAX_L positions: every attention entry point returns IRS_E_SHAPE above it.  The whole
+ * head's K and V stay in shared memory while that layout fits 227 KB (L <= 582 for dh = 32, <= 346 for dh = 64);
+ * longer windows run the key-blocked kernel of irs_pim_attn_fwd_blocked, with the same results up to rounding. */
+#define IRS_ATTN_MAX_L      2048
 #define IRS_MASK_PIM        0
 #define IRS_MASK_CAUSAL_PAD 1
 #define IRS_MASK_CAUSAL     2
@@ -83,16 +87,34 @@ int irs_pim_attn_fwd(const float* q, const float* k, const float* v, int64_t ld_
                      const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
                      float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
                      float p_drop, unsigned long long seed, void* stream);
+/* Key-blocked fp32 forward with the same contract (dropout mask included, bit for bit), for 1 <= L <= 2048 and
+ * 1 <= dh <= 256; shared memory holds one 64-key block at a time, so it does not depend on L.  Online softmax:
+ * results equal irs_pim_attn_fwd's up to fp32 rounding.  irs_pim_attn_fwd calls it when its own layout exceeds
+ * 227 KB; it is exported for tests and benchmarks. */
+int irs_pim_attn_fwd_blocked(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
+                             const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
+                             float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
+                             float p_drop, unsigned long long seed, void* stream);
 
-/* Tensor-core (tcgen05) forward with the same contract, for dh in {16,32,48,64} and L <= 223
- * (irs_pim_attn_tc_supported); bf16 hi/lo split MMAs with fp32 accumulation, ~1e-5 relative.
+/* Tensor-core (tcgen05) forward with the same contract, for dh in {16,32,48,64} and 1 <= L <= 2048
+ * (irs_pim_attn_tc_supported); bf16 hi/lo split MMAs with fp32 accumulation, ~1e-5 relative.  No dropout.
  * lse (optional, [B,H,n_q]) as for irs_pim_attn_fwd: the training forward (dropout 0) runs here and hands lse to
- * irs_pim_attn_bwd. */
+ * irs_pim_attn_bwd.  L <= 223 runs the kernel that keeps the head's K and V^T in shared memory, as before;
+ * longer windows run irs_pim_attn_fwd_tc_blocked. */
 int irs_pim_attn_tc_supported(int L, int dh);
 int irs_pim_attn_fwd_tc(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
                         const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
                         float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
                         int* error_flag, void* stream);
+/* Key-blocked tcgen05 forward, same contract and shapes as irs_pim_attn_fwd_tc (any 1 <= L <= 2048).  One CTA per
+ * (batch, head, 128-row query tile); K and V stream through shared memory in blocks of 128 keys, so shared memory
+ * and tensor memory (256 columns) do not depend on L.  Two passes per tile: the row max of the masked scores, then
+ * P = exp2(s - max) and O += P V.  The PIM objective key L-1 is an exact fp32 term of every row.  q/k/v rows and
+ * out must be 16-byte aligned. */
+int irs_pim_attn_fwd_tc_blocked(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
+                                const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
+                                float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
+                                int* error_flag, void* stream);
 
 /* Persistent tcgen05 forward for full windows of 129..223 positions with 32-wide heads
  * (irs_pim_attn_img_supported), the BASELINE cfg3/cfg5 decoder shape.  Its input is the q/k/v projection in
@@ -113,12 +135,20 @@ int irs_pim_attn_fwd_img(const void* images, const int64_t* ids, const float* r_
 
 /* backward of the above (all rows).  d_q/d_k/d_v are written (not accumulated) with the same
  * leading dimensions as q/k/v;  d_r_u[b] += w_obj * sum_{h,i} dS[b,h,i,L-1]   (PIM mode only; the
- * caller zeroes d_r_u once per step and every layer accumulates into it). */
+ * caller zeroes d_r_u once per step and every layer accumulates into it).  Windows whose q, k, v and dO do not
+ * fit 227 KB of shared memory (L > 286 for dh = 32, > 171 for dh = 64) run irs_pim_attn_bwd_blocked. */
 int irs_pim_attn_bwd(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
                      const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
                      const float* out, const float* lse, const float* d_out,
                      float* d_q, float* d_k, float* d_v, float* d_r_u,
                      int B, int L, int H, int dh, float p_drop, unsigned long long seed, void* stream);
+/* Key-blocked fp32 backward, same contract (1 <= L <= 2048, 1 <= dh <= 256, shared memory independent of L): one
+ * kernel per 32-row query tile gives dQ and the objective's d_r_u, one per 32-key tile gives dK and dV. */
+int irs_pim_attn_bwd_blocked(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
+                             const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
+                             const float* out, const float* lse, const float* d_out,
+                             float* d_q, float* d_k, float* d_v, float* d_r_u,
+                             int B, int L, int H, int dh, float p_drop, unsigned long long seed, void* stream);
 
 /* ---- a4 : fused (bias +) residual + LayerNorm, optionally followed by "+ const, LayerNorm" ----
  * t = x + y (+ y_bias);  o = LN(t; g1,b1,eps);  if g2: o = LN(o + c2; g2,b2,eps)

@@ -24,13 +24,16 @@ SIGNATURES = {
     "irs_embed_scatter_add_bwd": (_i, [_p, _p, _f, _p, _l, _i, _l, _l, _p]),
     "irs_pif_fwd": (_i, [_p, _p, _p, _p, _p, _i, _i, _l, _p]),
     "irs_pim_attn_fwd": (_i, [_p, _p, _p, _l, _l, _l, _p, _p, _f, _f, _i, _p, _p, _i, _i, _i, _i, _i, _i, _f, C.c_uint64, _p]),
+    "irs_pim_attn_fwd_blocked": (_i, [_p, _p, _p, _l, _l, _l, _p, _p, _f, _f, _i, _p, _p, _i, _i, _i, _i, _i, _i, _f, C.c_uint64, _p]),
     "irs_pim_attn_tc_supported": (_i, [_i, _i]),
     "irs_pim_attn_fwd_tc": (_i, [_p, _p, _p, _l, _l, _l, _p, _p, _f, _f, _i, _p, _p, _i, _i, _i, _i, _i, _i, _p, _p]),
+    "irs_pim_attn_fwd_tc_blocked": (_i, [_p, _p, _p, _l, _l, _l, _p, _p, _f, _f, _i, _p, _p, _i, _i, _i, _i, _i, _i, _p, _p]),
     "irs_pim_attn_img_supported": (_i, [_i, _i]),
     "irs_qkv_images_bytes": (_z, [_i, _i, _i, _i]),
     "irs_qkv_to_images": (_i, [_p, _p, _p, _l, _l, _l, _p, _i, _i, _i, _i, _i, _p]),
     "irs_pim_attn_fwd_img": (_i, [_p, _p, _p, _f, _f, _i, _p, _i, _i, _i, _i, _i, _i, _p, _p]),
     "irs_pim_attn_bwd": (_i, [_p, _p, _p, _l, _l, _l, _p, _p, _f, _f, _i, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _f, C.c_uint64, _p]),
+    "irs_pim_attn_bwd_blocked": (_i, [_p, _p, _p, _l, _l, _l, _p, _p, _f, _f, _i, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _f, C.c_uint64, _p]),
     "irs_residual_layernorm": (_i, [_p, _p, _p, _p, _p, _p, _p, _p, _f, _p, _l, _i, _p]),
     "irs_linear_prepared_bytes": (_z, [_i, _i]),
     "irs_linear_prepare_weights": (_i, [_p, _i, _i, _p, _p]),

@@ -382,18 +382,346 @@ pim_attn_tc_kernel(const Params p) {
 }
 
 }  // namespace tca
+
+// ---------------------------------------------------------------------------------------------------------
+// Key-blocked variant for windows of any length up to 2048.  One CTA per (batch, head, 128-row query tile);
+// thread r (< 128) owns query row r of the tile (TMEM lane r), thread 0 also issues the MMAs.  Q is staged once;
+// K and V^T stream through shared memory in blocks of KB = 128 keys, converted to the same bf16 hi/lo core-matrix
+// images the resident kernel uses.  Tile t visits key blocks 0..t only (causality):
+//   pass 1   S_blk = Q K_blk^T (TMEM columns [0,128)), running row max of the masked scores (no exp)
+//   pass 2   S_blk again; P = exp2(s - max) as hi/lo 32-key sub-blocks (double buffered),
+//            O += P V_blk (TMEM columns [128, 128+dh)) and the row sum
+//   epilogue O / sum, lse
+// The objective key L-1 of PIM mode is not in any block: each row adds it as an exact fp32 term
+// (q_i . k_{L-1}, weight exp2(s_obj - max), v_{L-1} added in the epilogue), so no tile visits extra blocks.
+// Shared memory: Q, K, V^T at most 32 KB each (dh = 64), P 32 KB, independent of L.  Two CTAs per SM for dh <= 48
+// overlap one CTA's staging with the other's MMAs.
+// ---------------------------------------------------------------------------------------------------------
+namespace tcb {
+
+using namespace irs::tc;
+
+constexpr int BM = 128;
+constexpr int KB = 128;              // keys per block
+constexpr int PB = 32;               // keys per P sub-block
+constexpr int THREADS = 128;
+constexpr uint32_t SBO = 128;
+constexpr uint32_t TMEM_COLS = 256;
+constexpr uint32_t O_COL = KB;
+
+struct Layout {
+  uint32_t off_q_hi, off_q_lo, off_k_hi, off_k_lo, off_v_hi, off_v_lo, off_p, p_buf_bytes, off_kb, off_bars, off_tmem, total;
+};
+__host__ __device__ inline Layout make_layout(int dh) {
+  Layout l;
+  const uint32_t part = (uint32_t)BM * dh * 2;                  // one bf16 part of a [128][dh] operand
+  l.off_q_hi = 0; l.off_q_lo = part;
+  l.off_k_hi = 2 * part; l.off_k_lo = 3 * part;                  // K   : [dh/8][128 keys][8]
+  l.off_v_hi = 4 * part; l.off_v_lo = 5 * part;                  // V^T : [128/8 key groups][dh][8]
+  l.off_p = 6 * part;
+  l.p_buf_bytes = 2u * (PB / 8) * BM * 16;                       // hi + lo of one 32-key sub-block: 16384
+  l.off_kb = l.off_p + 2 * l.p_buf_bytes;                        // float [128] key bias of the block
+  l.off_bars = l.off_kb + KB * 4;                                // s, v, pfree[2]
+  l.off_tmem = l.off_bars + 4 * 8;
+  l.total = l.off_tmem + 16;
+  return l;
+}
+
+__global__ void __launch_bounds__(THREADS, 2)
+pim_attn_tc_blocked_kernel(const tca::Params p) {
+  extern __shared__ __align__(128) uint8_t smem[];
+  const uint32_t sbase = smem_u32(smem);
+  const Layout lay = make_layout(p.dh);
+  const int tid = threadIdx.x, warp = tid >> 5;
+  const int b = blockIdx.x / p.H, h = blockIdx.x % p.H;
+  const int tile = p.q_row0 / BM + blockIdx.y;
+  const int L = p.L, dh = p.dh, slabs = dh / 8;
+  const bool pim = (p.mode == IRS_MASK_PIM);
+  const int Lk = pim ? L - 1 : L;                  // keys held in blocks (PIM: all but the objective key)
+  const float l2e = 1.4426950408889634f;
+  const float qscale = l2e / sqrtf((float)dh);
+  const float base_w = l2e * (pim ? p.w_h : 0.f);
+  float* kb = reinterpret_cast<float*>(smem + lay.off_kb);
+
+  const uint32_t bar_s = sbase + lay.off_bars, bar_v = bar_s + 8;
+  auto bar_pfree = [&](int i) { return bar_s + 16 + 8u * i; };
+  volatile uint32_t* tmem_holder = reinterpret_cast<volatile uint32_t*>(smem + lay.off_tmem);
+  if (tid == 0) {
+    mbar_init(bar_s, 1); mbar_init(bar_v, 1); mbar_init(bar_pfree(0), 1); mbar_init(bar_pfree(1), 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
+                 :: "r"(sbase + lay.off_tmem), "r"(TMEM_COLS) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+
+  const uint32_t k_lbo = (uint32_t)KB * 16, v_lbo = (uint32_t)dh * 16, q_lbo = (uint32_t)BM * 16;
+  const float* qbase = p.q + (int64_t)b * L * p.ld_q + h * dh;
+  const float* kbase = p.k + (int64_t)b * L * p.ld_k + h * dh;
+  const float* vbase = p.v + (int64_t)b * L * p.ld_v + h * dh;
+  const int i = tile * BM + tid;                   // this thread's query row
+  const bool row_ok = i < L;
+
+  // Q tile, pre-scaled into the log2 domain; the objective score in fp32 from the same scaled q
+  float s_obj = -INFINITY;
+  {
+    const float* qk = kbase + (int64_t)(L - 1) * p.ld_k;
+    float dot = 0.f;
+    for (int s = 0; s < slabs; ++s) {
+      float x[8];
+      if (row_ok) {
+        const float* src = qbase + (int64_t)i * p.ld_q + s * 8;
+        const float4 v0 = *reinterpret_cast<const float4*>(src), v1 = *reinterpret_cast<const float4*>(src + 4);
+        x[0] = v0.x * qscale; x[1] = v0.y * qscale; x[2] = v0.z * qscale; x[3] = v0.w * qscale;
+        x[4] = v1.x * qscale; x[5] = v1.y * qscale; x[6] = v1.z * qscale; x[7] = v1.w * qscale;
+        if (pim) {
+          const float4 k0 = *reinterpret_cast<const float4*>(qk + s * 8), k1 = *reinterpret_cast<const float4*>(qk + s * 8 + 4);
+          dot = fmaf(x[0], k0.x, dot); dot = fmaf(x[1], k0.y, dot); dot = fmaf(x[2], k0.z, dot); dot = fmaf(x[3], k0.w, dot);
+          dot = fmaf(x[4], k1.x, dot); dot = fmaf(x[5], k1.y, dot); dot = fmaf(x[6], k1.z, dot); dot = fmaf(x[7], k1.w, dot);
+        }
+      } else {
+#pragma unroll
+        for (int e = 0; e < 8; ++e) x[e] = 0.f;
+      }
+      uint4 hi, lo;
+      split8(x, hi, lo);
+      *reinterpret_cast<uint4*>(smem + lay.off_q_hi + s * q_lbo + tid * 16) = hi;
+      *reinterpret_cast<uint4*>(smem + lay.off_q_lo + s * q_lbo + tid * 16) = lo;
+    }
+    if (pim && p.ids[(int64_t)b * L + L - 1] != 0) s_obj = dot + l2e * p.w_obj * p.r_u[b];
+  }
+
+  // blocks this tile visits: keys 0 .. min(last row of the tile, Lk - 1)
+  const int nblk = (min(BM * (tile + 1), Lk) + KB - 1) / KB;
+  auto stage_k = [&](int blk) {                                  // thread <-> key column of the block
+    const int j = blk * KB + tid;
+    const bool ok = j < Lk;
+    const float* src = kbase + (int64_t)(ok ? j : 0) * p.ld_k;
+    for (int s = 0; s < slabs; ++s) {
+      float x[8];
+      if (ok) {
+        const float4 v0 = *reinterpret_cast<const float4*>(src + s * 8), v1 = *reinterpret_cast<const float4*>(src + s * 8 + 4);
+        x[0] = v0.x; x[1] = v0.y; x[2] = v0.z; x[3] = v0.w; x[4] = v1.x; x[5] = v1.y; x[6] = v1.z; x[7] = v1.w;
+      } else {
+#pragma unroll
+        for (int e = 0; e < 8; ++e) x[e] = 0.f;
+      }
+      uint4 hi, lo;
+      split8(x, hi, lo);
+      *reinterpret_cast<uint4*>(smem + lay.off_k_hi + s * k_lbo + tid * 16) = hi;
+      *reinterpret_cast<uint4*>(smem + lay.off_k_lo + s * k_lbo + tid * 16) = lo;
+    }
+    kb[tid] = (!ok || (p.mode != IRS_MASK_CAUSAL && p.ids[(int64_t)b * L + j] == 0)) ? -INFINITY : base_w;
+  };
+  auto stage_v = [&](int blk) {                                  // warp <-> group of 8 keys, lane <-> head dim
+    const int lane = tid & 31;
+    for (int ks = warp; ks < KB / 8; ks += THREADS / 32) {
+      for (int c = lane; c < dh; c += 32) {
+        float x[8];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) {
+          const int j = blk * KB + ks * 8 + e;
+          x[e] = (j < Lk) ? vbase[(int64_t)j * p.ld_v + c] : 0.f;
+        }
+        uint4 hi, lo;
+        split8(x, hi, lo);
+        *reinterpret_cast<uint4*>(smem + lay.off_v_hi + ks * v_lbo + c * 16) = hi;
+        *reinterpret_cast<uint4*>(smem + lay.off_v_lo + ks * v_lbo + c * 16) = lo;
+      }
+    }
+  };
+
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_holder;
+  const uint32_t trow = tmem_base + ((uint32_t)(warp * 32) << 16);
+  const uint32_t idesc_s = make_idesc_bf16(BM, KB);
+  const uint32_t idesc_o = make_idesc_bf16(BM, dh);
+  uint32_t ph_s = 0, ph_v = 0, ph_pfree[2] = {0, 0};
+
+  // S_blk = Q K_blk^T once the K image of the block is in shared memory; every thread waits for it
+  auto score_block = [&]() {
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    tc_fence_before();
+    __syncthreads();
+    if (tid == 0) {
+      tc_fence_after();
+      for (int kk = 0; kk < dh / 16; ++kk) {
+        const uint64_t q_hi = make_desc(sbase + lay.off_q_hi + (uint32_t)(kk * 2) * q_lbo, q_lbo, SBO);
+        const uint64_t q_lo = make_desc(sbase + lay.off_q_lo + (uint32_t)(kk * 2) * q_lbo, q_lbo, SBO);
+        const uint64_t k_hi = make_desc(sbase + lay.off_k_hi + (uint32_t)(kk * 2) * k_lbo, k_lbo, SBO);
+        const uint64_t k_lo = make_desc(sbase + lay.off_k_lo + (uint32_t)(kk * 2) * k_lbo, k_lbo, SBO);
+        tc_mma_bf16(tmem_base, q_lo, k_hi, idesc_s, kk != 0 ? 1u : 0u);
+        tc_mma_bf16(tmem_base, q_hi, k_lo, idesc_s, 1u);
+        tc_mma_bf16(tmem_base, q_hi, k_hi, idesc_s, 1u);
+      }
+      tc_commit(bar_s);
+    }
+    mbar_wait(bar_s, ph_s, p.error_flag, 40);
+    ph_s ^= 1u;
+    tc_fence_after();
+  };
+
+  // ---- pass 1: row max
+  float mx = s_obj;
+  for (int blk = 0; blk < nblk; ++blk) {
+    __syncthreads();                                             // every thread is done with the previous block's kb
+    stage_k(blk);
+    score_block();
+    const bool full = (blk + 1) * KB <= min(tile * BM + 1, Lk);  // every key of the block visible to every row
+    for (int sb = 0; sb < KB / PB; ++sb) {
+      uint32_t v[32];
+      tc_ld32(trow + sb * PB, v);
+      const float4* cw4 = reinterpret_cast<const float4*>(kb + sb * PB);
+      tc_wait_ld();
+      const int c0 = blk * KB + sb * PB;
+      float m0 = -INFINITY, m1 = -INFINITY, m2 = -INFINITY, m3 = -INFINITY;
+      if (full) {
+#pragma unroll
+        for (int j4 = 0; j4 < 8; ++j4) {
+          const float4 w = cw4[j4];
+          m0 = fmaxf(m0, __uint_as_float(v[4 * j4 + 0]) + w.x); m1 = fmaxf(m1, __uint_as_float(v[4 * j4 + 1]) + w.y);
+          m2 = fmaxf(m2, __uint_as_float(v[4 * j4 + 2]) + w.z); m3 = fmaxf(m3, __uint_as_float(v[4 * j4 + 3]) + w.w);
+        }
+      } else {
+#pragma unroll
+        for (int j4 = 0; j4 < 8; ++j4) {
+          const float4 w = cw4[j4];
+          const int c = c0 + 4 * j4;
+          if (c + 0 <= i) m0 = fmaxf(m0, __uint_as_float(v[4 * j4 + 0]) + w.x);
+          if (c + 1 <= i) m1 = fmaxf(m1, __uint_as_float(v[4 * j4 + 1]) + w.y);
+          if (c + 2 <= i) m2 = fmaxf(m2, __uint_as_float(v[4 * j4 + 2]) + w.z);
+          if (c + 3 <= i) m3 = fmaxf(m3, __uint_as_float(v[4 * j4 + 3]) + w.w);
+        }
+      }
+      mx = fmaxf(mx, fmaxf(fmaxf(m0, m1), fmaxf(m2, m3)));
+    }
+  }
+
+  // ---- pass 2: P and O += P V
+  float sum = pim ? exp2f(s_obj - mx) : 0.f;                     // fully masked row: -inf - -inf = NaN, as torch
+  for (int blk = 0; blk < nblk; ++blk) {
+    if (blk > 0) { mbar_wait(bar_v, ph_v, p.error_flag, 41); ph_v ^= 1u; }   // the previous block's O MMAs read V and P
+    __syncthreads();
+    stage_k(blk);
+    stage_v(blk);
+    score_block();
+    const bool full = (blk + 1) * KB <= min(tile * BM + 1, Lk);
+    for (int sb = 0; sb < KB / PB; ++sb) {
+      const int g = blk * (KB / PB) + sb, pb = g & 1;
+      uint32_t v[32];
+      tc_ld32(trow + sb * PB, v);
+      if (g >= 2) { mbar_wait(bar_pfree(pb), ph_pfree[pb], p.error_flag, 42); ph_pfree[pb] ^= 1u; }
+      uint8_t* pdst = smem + lay.off_p + pb * lay.p_buf_bytes;
+      const float4* cw4 = reinterpret_cast<const float4*>(kb + sb * PB);
+      tc_wait_ld();
+      const int c0 = blk * KB + sb * PB;
+#pragma unroll
+      for (int s8 = 0; s8 < PB / 8; ++s8) {
+        float x[8];
+#pragma unroll
+        for (int hq = 0; hq < 2; ++hq) {
+          const float4 w = cw4[s8 * 2 + hq];
+          const float ww[4] = {w.x, w.y, w.z, w.w};
+          const int c = c0 + s8 * 8 + hq * 4;
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            float pv = exp2f(__uint_as_float(v[s8 * 8 + hq * 4 + e]) + ww[e] - mx);
+            if (!full && c + e > i) pv = 0.f;
+            x[hq * 4 + e] = pv;
+            sum += pv;
+          }
+        }
+        uint4 hi, lo;
+        split8(x, hi, lo);
+        *reinterpret_cast<uint4*>(pdst + s8 * q_lbo + tid * 16) = hi;
+        *reinterpret_cast<uint4*>(pdst + lay.p_buf_bytes / 2 + s8 * q_lbo + tid * 16) = lo;
+      }
+      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      tc_fence_before();
+      __syncthreads();
+      if (tid == 0) {
+        tc_fence_after();
+        const uint32_t ps = sbase + lay.off_p + pb * lay.p_buf_bytes;
+#pragma unroll
+        for (int kk = 0; kk < PB / 16; ++kk) {
+          const uint64_t p_hi = make_desc(ps + (uint32_t)(kk * 2) * q_lbo, q_lbo, SBO);
+          const uint64_t p_lo = make_desc(ps + lay.p_buf_bytes / 2 + (uint32_t)(kk * 2) * q_lbo, q_lbo, SBO);
+          const uint32_t vo = (uint32_t)(sb * (PB / 8) + kk * 2) * v_lbo;
+          const uint64_t v_hi = make_desc(sbase + lay.off_v_hi + vo, v_lbo, SBO);
+          const uint64_t v_lo = make_desc(sbase + lay.off_v_lo + vo, v_lbo, SBO);
+          tc_mma_bf16(tmem_base + O_COL, p_lo, v_hi, idesc_o, (g | kk) != 0 ? 1u : 0u);
+          tc_mma_bf16(tmem_base + O_COL, p_hi, v_lo, idesc_o, 1u);
+          tc_mma_bf16(tmem_base + O_COL, p_hi, v_hi, idesc_o, 1u);
+        }
+        tc_commit(bar_pfree(pb));
+        if (sb == KB / PB - 1) tc_commit(bar_v);
+      }
+    }
+  }
+  if (nblk > 0) { mbar_wait(bar_v, ph_v, p.error_flag, 43); ph_v ^= 1u; }
+  tc_fence_after();
+
+  // ---- epilogue: O / sum (+ the objective term), lse
+  {
+    const bool write = row_ok && (i >= p.q_row0) && (i < p.q_row0 + p.n_q);
+    const float inv = 1.0f / sum;
+    const float w_obj_row = pim ? exp2f(s_obj - mx) : 0.f;
+    const float* vobj = vbase + (int64_t)(L - 1) * p.ld_v;
+    float* dst = p.out + ((int64_t)b * p.n_q + (i - p.q_row0)) * (p.H * dh) + h * dh;
+    if (write && p.lse != nullptr)
+      p.lse[((int64_t)b * p.H + h) * p.n_q + (i - p.q_row0)] = 0.6931471805599453f * (mx + log2f(sum));
+    for (int c0 = 0; c0 < dh; c0 += 16) {
+      uint32_t v[16];
+      if (nblk > 0) {
+        asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 "
+                     "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+                     : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
+                       "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
+                     : "r"(trow + O_COL + c0));
+        tc_wait_ld();
+      } else {
+#pragma unroll
+        for (int j = 0; j < 16; ++j) v[j] = 0u;
+      }
+      if (write) {
+#pragma unroll
+        for (int j = 0; j < 16; j += 4) {
+          float4 o4 = make_float4(__uint_as_float(v[j]), __uint_as_float(v[j + 1]), __uint_as_float(v[j + 2]), __uint_as_float(v[j + 3]));
+          if (pim) {
+            const float4 vo = *reinterpret_cast<const float4*>(vobj + c0 + j);
+            o4.x = fmaf(w_obj_row, vo.x, o4.x); o4.y = fmaf(w_obj_row, vo.y, o4.y);
+            o4.z = fmaf(w_obj_row, vo.z, o4.z); o4.w = fmaf(w_obj_row, vo.w, o4.w);
+          }
+          *reinterpret_cast<float4*>(dst + c0 + j) = make_float4(o4.x * inv, o4.y * inv, o4.z * inv, o4.w * inv);
+        }
+      }
+    }
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 0) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem_base), "r"(TMEM_COLS) : "memory");
+  }
+}
+
+}  // namespace tcb
 }  // namespace irs
 
 using namespace irs;
 
 extern "C" int irs_pim_attn_tc_supported(int L, int dh) {
-  return (dh % 16 == 0 && dh >= 16 && dh <= 64 && L >= 1 && L <= tca::KEYS_MAX - 1) ? 1 : 0;
+  return (dh % 16 == 0 && dh >= 16 && dh <= 64 && L >= 1 && L <= IRS_ATTN_MAX_L) ? 1 : 0;
 }
 
-extern "C" int irs_pim_attn_fwd_tc(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
-                                   const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
-                                   float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
-                                   int* error_flag, void* stream) {
+static int attn_tc_check(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
+                         const int64_t* ids, const float* r_u, int mode, const float* out, int B, int L, int H, int dh,
+                         int q_row0, int n_q) {
   if (!q || !k || !v || !out) return IRS_E_BADARG;
   if (B <= 0 || L <= 0 || H <= 0 || dh <= 0 || q_row0 < 0 || n_q <= 0 || q_row0 + n_q > L) return IRS_E_BADARG;
   if (mode < 0 || mode > 2) return IRS_E_BADARG;
@@ -403,17 +731,59 @@ extern "C" int irs_pim_attn_fwd_tc(const float* q, const float* k, const float* 
   if ((ld_q & 3) || (ld_k & 3) || (ld_v & 3) || ((uintptr_t)q & 15) || ((uintptr_t)k & 15) || ((uintptr_t)v & 15) ||
       ((uintptr_t)out & 15))
     return IRS_E_SHAPE;
+  return 0;
+}
+
+static tca::Params attn_tc_params(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
+                                  const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
+                                  float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q, int* error_flag) {
+  tca::Params p = {};
+  p.q = q; p.k = k; p.v = v; p.ld_q = ld_q; p.ld_k = ld_k; p.ld_v = ld_v; p.ids = ids; p.r_u = r_u;
+  p.w_h = w_h; p.w_obj = w_obj; p.mode = mode; p.out = out; p.B = B; p.L = L; p.H = H; p.dh = dh;
+  p.q_row0 = q_row0; p.n_q = n_q; p.error_flag = error_flag; p.lse = lse;
+  return p;
+}
+
+static int attn_tc_blocked_launch(const tca::Params& p, void* stream) {
+  const tcb::Layout lay = tcb::make_layout(p.dh);
+  static uint32_t configured = 0;
+  if (lay.total > configured) {
+    IRS_CUDA(cudaFuncSetAttribute(tcb::pim_attn_tc_blocked_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.total));
+    configured = lay.total;
+  }
+  const int tiles = (p.q_row0 + p.n_q - 1) / tcb::BM - p.q_row0 / tcb::BM + 1;
+  dim3 grid((unsigned)(p.B * p.H), (unsigned)tiles);
+  tcb::pim_attn_tc_blocked_kernel<<<grid, tcb::THREADS, lay.total, (cudaStream_t)stream>>>(p);
+  IRS_LAUNCHED();
+  return 0;
+}
+
+extern "C" int irs_pim_attn_fwd_tc(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
+                                   const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
+                                   float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
+                                   int* error_flag, void* stream) {
+  const int rc = attn_tc_check(q, k, v, ld_q, ld_k, ld_v, ids, r_u, mode, out, B, L, H, dh, q_row0, n_q);
+  if (rc) return rc;
+  const tca::Params p = attn_tc_params(q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, B, L, H, dh,
+                                       q_row0, n_q, error_flag);
+  if (L > tca::KEYS_MAX - 1) return attn_tc_blocked_launch(p, stream);    // the head's K / V^T no longer fit on chip
   const tca::Layout lay = tca::make_layout(dh);
   static uint32_t configured = 0;
   if (lay.total > configured) {
     IRS_CUDA(cudaFuncSetAttribute(tca::pim_attn_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.total));
     configured = lay.total;
   }
-  tca::Params p = {};
-  p.q = q; p.k = k; p.v = v; p.ld_q = ld_q; p.ld_k = ld_k; p.ld_v = ld_v; p.ids = ids; p.r_u = r_u;
-  p.w_h = w_h; p.w_obj = w_obj; p.mode = mode; p.out = out; p.B = B; p.L = L; p.H = H; p.dh = dh;
-  p.q_row0 = q_row0; p.n_q = n_q; p.error_flag = error_flag; p.lse = lse;
   tca::pim_attn_tc_kernel<<<(unsigned)(B * H), tca::THREADS, lay.total, (cudaStream_t)stream>>>(p);
   IRS_LAUNCHED();
   return 0;
+}
+
+extern "C" int irs_pim_attn_fwd_tc_blocked(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
+                                           const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
+                                           float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
+                                           int* error_flag, void* stream) {
+  const int rc = attn_tc_check(q, k, v, ld_q, ld_k, ld_v, ids, r_u, mode, out, B, L, H, dh, q_row0, n_q);
+  if (rc) return rc;
+  return attn_tc_blocked_launch(attn_tc_params(q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, B, L, H, dh,
+                                               q_row0, n_q, error_flag), stream);
 }
