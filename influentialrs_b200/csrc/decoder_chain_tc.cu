@@ -164,6 +164,34 @@ __device__ __forceinline__ void pair_barrier(int quad) {          // the two epi
   asm volatile("bar.sync %0, 64;" :: "r"(1 + quad) : "memory");
 }
 
+// LayerNorm statistics of a row held by the two epilogue threads of a lane quadrant, 64 columns each, in two passes:
+// each thread centres its values on its own half mean m (t <- t - m, in place) and sums their squares q; the pair
+// exchanges (m, q) and merges them with Chan's formula (n_a = n_b = 64): mean = (m_a + m_b) / 2,
+// M2 = q_a + q_b + 32 (m_b - m_a)^2.  The merge is symmetric in a and b, so both threads get the same mean and rstd.
+// Unlike E[t^2] - mean^2 this keeps its accuracy on rows whose mean is large next to their spread.  Both sums run in
+// four interleaved partial sums (column j into j % 4): the epilogue warps are latency bound, and a 64-long dependent
+// chain per pass would cost more than the pass itself.
+// Returns (rstd, (m - mean) rstd): the normalised value of a centred element c is c rstd + .y.
+__device__ __forceinline__ float2 ln_pair_stats(float (&t)[64], float2* mine, const float2* other, int quad, float eps) {
+  float s[4] = {0.f, 0.f, 0.f, 0.f}, q[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+  for (int j = 0; j < 64; ++j) s[j & 3] += t[j];
+  const float m = ((s[0] + s[1]) + (s[2] + s[3])) * (1.0f / 64.0f);
+#pragma unroll
+  for (int j = 0; j < 64; ++j) {
+    t[j] -= m;
+    q[j & 3] = fmaf(t[j], t[j], q[j & 3]);
+  }
+  const float qs = (q[0] + q[1]) + (q[2] + q[3]);
+  *mine = make_float2(m, qs);
+  pair_barrier(quad);
+  const float2 o = *other;
+  const float delta = o.x - m;
+  const float mean = 0.5f * (m + o.x);
+  const float rstd = rsqrtf(fmaf(32.f * delta, delta, qs + o.y) * (1.0f / (float)D) + eps);
+  return make_float2(rstd, (m - mean) * rstd);
+}
+
 __global__ void __launch_bounds__(THREADS, 1)
 decoder_chain_kernel(const Params p) {
   extern __shared__ __align__(128) uint8_t smem[];
@@ -374,7 +402,6 @@ decoder_chain_kernel(const Params p) {
     const int row = quad * 32 + lane;
     const uint32_t tlane = tmem_base + (((uint32_t)(quad * 32)) << 16);
     float2* xch = reinterpret_cast<float2*>(smem + OFF_XCH);
-    const float inv_n = 1.0f / (float)D;
     const int c0 = half * 64;                        // this thread's columns of a 128-wide row
     // ---------------- E4: qkv' = acc + bin -> HBM, one piece (0: columns [0,256) in T_H, 1: [256,384) in T_D3) ----------------
     // fp32 rows [R, 384], or operand images: q (pre-scaled) / k / v of every head as bf16 hi/lo 16-byte pieces.
@@ -470,7 +497,6 @@ decoder_chain_kernel(const Params p) {
       mbar_wait(bar(B_D1), ph, p.error_flag, 41);
       tc_fence_after();
       if (warp == 0) IRS_TL(1, 1);
-      float s1 = 0.f, s2 = 0.f;
 #pragma unroll
       for (int ch = 0; ch < 2; ++ch) {
         uint32_t v[32];
@@ -478,44 +504,25 @@ decoder_chain_kernel(const Params p) {
         tc_wait_ld();
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
-          const float tt = __uint_as_float(v[j]) + vecs[V_BO + c0 + ch * 32 + j] + t[ch * 32 + j];
-          s1 += tt; s2 = fmaf(tt, tt, s2);
-          t[ch * 32 + j] = tt;
+          t[ch * 32 + j] = __uint_as_float(v[j]) + vecs[V_BO + c0 + ch * 32 + j] + t[ch * 32 + j];
         }
       }
-      xch[(0 * 2 + half) * 128 + row] = make_float2(s1, s2);
-      pair_barrier(quad);
-      {
-        const float2 o = xch[(0 * 2 + (half ^ 1)) * 128 + row];
-        s1 += o.x; s2 += o.y;
-      }
-      const float mean1 = s1 * inv_n;
-      const float rstd1 = rsqrtf(fmaxf(s2 * inv_n - mean1 * mean1, 0.f) + p.eps1);
-      const float nmr1 = -mean1 * rstd1;
-      float u1 = 0.f, u2 = 0.f;
+      const float2 st1 = ln_pair_stats(t, &xch[(0 * 2 + half) * 128 + row], &xch[(0 * 2 + (half ^ 1)) * 128 + row],
+                                       quad, p.eps1);
 #pragma unroll
       for (int j = 0; j < 64; ++j) {
         const int n = c0 + j;
-        const float y = fmaf(fmaf(t[j], rstd1, nmr1), vecs[V_G1 + n], vecs[V_B1 + n]);      // V_B1 holds b1 + c2
-        u1 += y; u2 = fmaf(y, y, u2);
-        t[j] = y;
+        t[j] = fmaf(fmaf(t[j], st1.x, st1.y), vecs[V_G1 + n], vecs[V_B1 + n]);      // V_B1 holds b1 + c2
       }
-      xch[(1 * 2 + half) * 128 + row] = make_float2(u1, u2);
-      pair_barrier(quad);
-      {
-        const float2 o = xch[(1 * 2 + (half ^ 1)) * 128 + row];
-        u1 += o.x; u2 += o.y;
-      }
-      const float mean2 = u1 * inv_n;
-      const float rstd2 = rsqrtf(fmaxf(u2 * inv_n - mean2 * mean2, 0.f) + p.eps2);
-      const float nmr2 = -mean2 * rstd2;
+      const float2 st2 = ln_pair_stats(t, &xch[(1 * 2 + half) * 128 + row], &xch[(1 * 2 + (half ^ 1)) * 128 + row],
+                                       quad, p.eps2);
 #pragma unroll
       for (int ch = 0; ch < 2; ++ch) {
         uint32_t v[32];
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
           const int n = c0 + ch * 32 + j;
-          const float y = fmaf(fmaf(t[ch * 32 + j], rstd2, nmr2), vecs[V_G2 + n], vecs[V_B2 + n]);
+          const float y = fmaf(fmaf(t[ch * 32 + j], st2.x, st2.y), vecs[V_G2 + n], vecs[V_B2 + n]);
           t[ch * 32 + j] = y;
           v[j] = __float_as_uint(y);
         }
@@ -566,7 +573,6 @@ decoder_chain_kernel(const Params p) {
       mbar_wait(bar(B_D3), ph, p.error_flag, 44);
       tc_fence_after();
       if (warp == 0) IRS_TL(1, 11);
-      float w1 = 0.f, w2 = 0.f;
 #pragma unroll
       for (int ch = 0; ch < 2; ++ch) {
         uint32_t v[32], y[32];
@@ -575,27 +581,18 @@ decoder_chain_kernel(const Params p) {
         tc_wait_ld();
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
-          const float tt = __uint_as_float(v[j]) + vecs[V_BF2 + c0 + ch * 32 + j] + __uint_as_float(y[j]);
-          w1 += tt; w2 = fmaf(tt, tt, w2);
-          t[ch * 32 + j] = tt;
+          t[ch * 32 + j] = __uint_as_float(v[j]) + vecs[V_BF2 + c0 + ch * 32 + j] + __uint_as_float(y[j]);
         }
       }
-      xch[(2 * 2 + half) * 128 + row] = make_float2(w1, w2);
-      pair_barrier(quad);
-      {
-        const float2 o = xch[(2 * 2 + (half ^ 1)) * 128 + row];
-        w1 += o.x; w2 += o.y;
-      }
-      const float mean3 = w1 * inv_n;
-      const float rstd3 = rsqrtf(fmaxf(w2 * inv_n - mean3 * mean3, 0.f) + p.eps3);
-      const float nmr3 = -mean3 * rstd3;
+      const float2 st3 = ln_pair_stats(t, &xch[(2 * 2 + half) * 128 + row], &xch[(2 * 2 + (half ^ 1)) * 128 + row],
+                                       quad, p.eps3);
       float* xo = p.x_out + (row_ok ? r : 0) * D + c0;
 #pragma unroll
       for (int ch = 0; ch < 2; ++ch) {
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
           const int n = c0 + ch * 32 + j;
-          t[ch * 32 + j] = fmaf(fmaf(t[ch * 32 + j], rstd3, nmr3), vecs[V_G3 + n], vecs[V_B3 + n]);
+          t[ch * 32 + j] = fmaf(fmaf(t[ch * 32 + j], st3.x, st3.y), vecs[V_G3 + n], vecs[V_B3 + n]);
         }
         if (row_ok) {
 #pragma unroll

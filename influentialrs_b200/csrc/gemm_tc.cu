@@ -79,6 +79,18 @@ prepare_linear_kernel(const float* __restrict__ W, int Nout, int K, int n_pad, i
   }
 }
 
+// Chan's parallel-variance merge: fold the statistics of nb more values (mean mb, sum of squared deviations qb) into the
+// running (n, mean, m2) of a row.  Each 32-column chunk is centred on its own mean before it is squared, so the row
+// statistics stay accurate when the mean is large next to the spread (E[t^2] - mean^2 would cancel).
+__device__ __forceinline__ void chan_merge(float& n, float& mean, float& m2, float nb, float mb, float qb) {
+  const float nn = n + nb;
+  const float delta = mb - mean;
+  const float w = nb / nn;
+  mean = fmaf(delta, w, mean);
+  m2 += qb + delta * delta * (n * w);
+  n = nn;
+}
+
 template <int EPI>
 __global__ void __launch_bounds__(THREADS, 1)
 linear_tc_kernel(const Params p) {
@@ -259,11 +271,12 @@ linear_tc_kernel(const Params p) {
           }
         }
       } else {
-        // pass 1: t = resid + acc + bias, written back into the accumulator (TMEM as row scratch);
-        // sum and sum of squares.  pass 2 (optional): statistics of LN1(t)+c2.  pass 3: normalise, store.
+        // pass 1: t = resid + acc + bias, written back into the accumulator (TMEM as row scratch); mean and squared
+        // deviations of each chunk, merged into the row's.  pass 2 (optional): the same statistics of LN1(t)+c2.
+        // pass 3: normalise, store.
         const float inv_n = 1.0f / (float)p.Nout;
         const float* rsd = p.resid + (row_ok ? r : 0) * p.ldr;
-        float s1 = 0.f, s2 = 0.f;
+        float n1 = 0.f, mean1 = 0.f, q1 = 0.f;
         for (int ch = 0; ch < n_ch; ++ch) {
           uint32_t v[32];
           tc_ld32(tbase + ch * 32, v);
@@ -276,37 +289,54 @@ linear_tc_kernel(const Params p) {
             rr[j] = q.x; rr[j + 1] = q.y; rr[j + 2] = q.z; rr[j + 3] = q.w;
           }
           tc_wait_ld();
+          const int nc = min(32, p.Nout - ch * 32);
+          float cs[4] = {0.f, 0.f, 0.f, 0.f}, cq[4] = {0.f, 0.f, 0.f, 0.f};     // four partial sums: short dependent chains
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
             const int n = ch * 32 + j;
             float t = 0.f;
-            if (n < p.Nout) { t = __uint_as_float(v[j]) + bias_s[n] + rr[j]; s1 += t; s2 = fmaf(t, t, s2); }
+            if (n < p.Nout) { t = __uint_as_float(v[j]) + bias_s[n] + rr[j]; cs[j & 3] += t; }
             v[j] = __float_as_uint(t);
           }
           tc_st32(tbase + ch * 32, v);
+          const float cm = ((cs[0] + cs[1]) + (cs[2] + cs[3])) / (float)nc;
+#pragma unroll
+          for (int j = 0; j < 32; ++j) {
+            const float e = __uint_as_float(v[j]) - cm;
+            if (ch * 32 + j < p.Nout) cq[j & 3] = fmaf(e, e, cq[j & 3]);
+          }
+          chan_merge(n1, mean1, q1, (float)nc, cm, (cq[0] + cq[1]) + (cq[2] + cq[3]));
         }
         tc_wait_st();
-        const float mean1 = s1 * inv_n;
-        const float rstd1 = rsqrtf(fmaxf(s2 * inv_n - mean1 * mean1, 0.f) + p.eps);
+        const float rstd1 = rsqrtf(q1 * inv_n + p.eps);
         float mean2 = 0.f, rstd2 = 1.f;
         const bool two = (p.g2 != nullptr);
         if (two) {
-          float u1 = 0.f, u2 = 0.f;
+          float n2 = 0.f, q2 = 0.f;
           for (int ch = 0; ch < n_ch; ++ch) {
             uint32_t v[32];
             tc_ld32(tbase + ch * 32, v);
             tc_wait_ld();
+            const int nc = min(32, p.Nout - ch * 32);
+            float y[32], cs[4] = {0.f, 0.f, 0.f, 0.f}, cq[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
             for (int j = 0; j < 32; ++j) {
               const int n = ch * 32 + j;
+              y[j] = 0.f;
               if (n < p.Nout) {
-                const float y = (__uint_as_float(v[j]) - mean1) * rstd1 * vecs[1 * NMAX + n] + vecs[2 * NMAX + n] + vecs[3 * NMAX + n];
-                u1 += y; u2 = fmaf(y, y, u2);
+                y[j] = (__uint_as_float(v[j]) - mean1) * rstd1 * vecs[1 * NMAX + n] + vecs[2 * NMAX + n] + vecs[3 * NMAX + n];
+                cs[j & 3] += y[j];
               }
             }
+            const float cm = ((cs[0] + cs[1]) + (cs[2] + cs[3])) / (float)nc;
+#pragma unroll
+            for (int j = 0; j < 32; ++j) {
+              const float e = y[j] - cm;
+              if (ch * 32 + j < p.Nout) cq[j & 3] = fmaf(e, e, cq[j & 3]);
+            }
+            chan_merge(n2, mean2, q2, (float)nc, cm, (cq[0] + cq[1]) + (cq[2] + cq[3]));
           }
-          mean2 = u1 * inv_n;
-          rstd2 = rsqrtf(fmaxf(u2 * inv_n - mean2 * mean2, 0.f) + p.eps);
+          rstd2 = rsqrtf(q2 * inv_n + p.eps);
         }
         for (int ch = 0; ch < n_ch; ++ch) {
           uint32_t v[32];
