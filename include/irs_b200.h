@@ -362,7 +362,7 @@ int irs_score_count_ahead_tc(const float* h, int64_t ld_h, const float* W, const
 /* ---- a6 backward : softmax-CE gradient with logits recomputed tile by tile --------------------
  * p = exp(s - lse);  g[m,j] = (p - [j == target[m]]) * gscale;   target is a 0-based column, or <0
  * to skip the row.   d_h[m,:] = sum_j g W[j,:];  d_W[j,:] += sum_m g h[m,:];  d_bias[j] += sum_m g.
- * d_h is written; d_W / d_bias are accumulated into (caller zeroes them).
+ * d_h is written; d_W / d_bias are accumulated into (caller zeroes them); any of the three may be NULL.
  * replaces autograd of project + CrossEntropyLoss  model/influentialRS.py:214,303,307 */
 int irs_score_ce_bwd(const float* h, int64_t ld_h, const float* W, const float* bias,
                      const int64_t* target, const float* lse, float gscale,

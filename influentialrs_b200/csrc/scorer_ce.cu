@@ -3,8 +3,8 @@
 //   g[m,j] = (exp(s[m,j] - lse[m]) - [j == target[m]]) * gscale
 //   d_h = g W          (kernel OWNER_M: a CTA owns 128 rows of h and sweeps the catalog)
 //   d_W += g^T h, d_bias += colsum(g)   (kernel OWNER_N: a CTA owns 128 catalog rows and sweeps M)
-// Each owner accumulates its 128 x d output tile in registers, so there are no global atomics and
-// the result is deterministic.
+// Each owner accumulates its 128 x d output tile in registers (one 128-row tile at a time, then into the
+// running sum), so there are no global atomics and the result is deterministic.  Any of d_h, d_W, d_bias may be NULL.
 //   reference: autograd of self.project + nn.CrossEntropyLoss, model/influentialRS.py:214,303,307.
 #include "common.cuh"
 
@@ -144,7 +144,14 @@ ce_bwd_kernel(const float* __restrict__ h, int64_t ld_h, const float* __restrict
       for (int j = 0; j < 8; ++j) atomicAdd(&sm.colsum[cn[j]], csum[j]);
     }
     __syncthreads();
-    // ---- second GEMM: acc2[owner, c] += sum_r Gs[r][owner] * Bt[r][c]
+    // ---- second GEMM: acc2[owner, c] += sum_r Gs[r][owner] * Bt[r][c], the tile summed on its own first: added one by one
+    // to a running sum over 500k items, the terms of tail items (p ~ 1e-6 and below) fall under half an ulp of it and are
+    // rounded away -- the same way every time, ~1e-3 of |d_h| on a catalog whose embeddings share a direction
+    float part[8][8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i)
+#pragma unroll
+      for (int j = 0; j < 8; ++j) part[i][j] = 0.f;
 #pragma unroll 4
     for (int r = 0; r < 128; ++r) {
       const float4 a0 = *reinterpret_cast<const float4*>(&sm.Gs[r][ty * 4]);
@@ -156,8 +163,12 @@ ce_bwd_kernel(const float* __restrict__ h, int64_t ld_h, const float* __restrict
 #pragma unroll
       for (int i = 0; i < 8; ++i)
 #pragma unroll
-        for (int j = 0; j < 8; ++j) acc2[i][j] = fmaf(a[i], b[j], acc2[i][j]);
+        for (int j = 0; j < 8; ++j) part[i][j] = fmaf(a[i], b[j], part[i][j]);
     }
+#pragma unroll
+    for (int i = 0; i < 8; ++i)
+#pragma unroll
+      for (int j = 0; j < 8; ++j) acc2[i][j] += part[i][j];
     __syncthreads();
   }
 
@@ -171,7 +182,7 @@ ce_bwd_kernel(const float* __restrict__ h, int64_t ld_h, const float* __restrict
       const int c = cn[j];
       if (c >= d) continue;
       if (OWNER_M) d_h[o * d + c] = acc2[i][j];
-      else d_W[o * d + c] += acc2[i][j];
+      else if (d_W != nullptr) d_W[o * d + c] += acc2[i][j];
     }
   }
   if (!OWNER_M && d_bias != nullptr && tid < 128 && own0 + tid < N) d_bias[own0 + tid] += sm.colsum[tid];
@@ -199,7 +210,7 @@ extern "C" int irs_score_ce_bwd(const float* h, int64_t ld_h, const float* W, co
         h, ld_h, W, bias, target, lse, gscale, d_h, nullptr, nullptr, M, N, d);
     IRS_LAUNCHED();
   }
-  if (d_W != nullptr) {
+  if (d_W != nullptr || d_bias != nullptr) {             // d_bias comes out of the d_W pass
     ce_bwd_kernel<false><<<(unsigned)ceil_div(N, 128), ce::kThreads, bytes, s>>>(
         h, ld_h, W, bias, target, lse, gscale, nullptr, d_W, d_bias, M, N, d);
     IRS_LAUNCHED();

@@ -12,8 +12,11 @@
 //   ACC += G Y   (A operand from TMEM; Y consumed a second time from the same shared-memory tile as an MN-major
 //                 B operand, so neither a transpose nor a second copy exists)
 // For d_h: rowb = -lse[m], rowid = target[m], colb = bias[j], colid = j.  For d_W the two sides swap and the row
-// sums of G give d_bias.  A CTA owning an X tile needs no atomics; when there are fewer X tiles than SMs the Y range
-// is split and the partial results are added with red.global.
+// sums of G give d_bias.  A CTA owning an X tile needs no atomics; when there are fewer X tiles than SMs, or when the Y
+// range is longer than MAX_RUN_TILES, the Y range is split and the partial results are added with red.global.
+// Accumulation: every tcgen05.mma into ACC loses up to one fp32 ulp of the running partial (truncation-like when the
+// partials have one sign), 24 MMAs per Y tile.  One run of 3,907 tiles (the d_h pass at 500k items) would lose ~3e-3 of
+// |d_h| on coherent sums (an anisotropic catalog); runs of <= 256 tiles keep it near 2e-4 (tests/ce_cases.py).
 // Operand format ("row images", one per 128 rows): [part hi|lo][16 slabs of 8 columns][128 rows][8 bf16] = 64 KB,
 // built once per call by prepare_rows_kernel for h and for W (K is zero-padded to 128).
 // Warps: 0-7 epilogue (TMEM lane quadrant = warp % 4, 64-column half = warp / 4), 8 producer (bulk copies + the
@@ -41,6 +44,7 @@ constexpr uint32_t SMEM_BYTES = OFF_TMEM + 16;
 constexpr int THREADS = 10 * 32;
 constexpr int WARP_PROD = 8, WARP_MMA = 9;
 constexpr uint32_t T_ACC = 256;
+constexpr int MAX_RUN_TILES = 256;                           // Y tiles one ACC accumulation may span
 
 struct Params {
   const uint8_t* ximg; const uint8_t* yimg;      // row images
@@ -50,7 +54,7 @@ struct Params {
   int64_t RX, RY;                                // valid rows on each side
   int n_x_tiles, n_y_tiles, n_splits, tiles_per_split;
   float gscale;
-  float* out; int64_t ld_out; int d;             // [RX, d] accumulated (+=)
+  float* out; int64_t ld_out; int d;             // [RX, d] accumulated (+=) or null
   float* rowsum;                                 // [RX] accumulated (+=) or null
   int use_atomics;
   int* error_flag;
@@ -275,7 +279,7 @@ ce_bwd_tc_kernel(const Params p) {
         uint32_t v[32];
         tc_ld32(tlane + T_ACC + c0, v);
         tc_wait_ld();
-        if (row_ok) {
+        if (row_ok && p.out) {
           float* dst = p.out + xr * p.ld_out + c0;
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
@@ -308,6 +312,7 @@ static void plan(int64_t RX, int64_t RY, int& n_x, int& n_y, int& n_splits, int&
   const int64_t max_splits = ceil_div(n_y, 16) > 0 ? ceil_div(n_y, 16) : 1;
   if (splits > max_splits) splits = max_splits;
   tps = (int)ceil_div(n_y, splits);
+  if (tps > MAX_RUN_TILES) tps = MAX_RUN_TILES;              // bound the fp32 error of one TMEM accumulation
   n_splits = (int)ceil_div(n_y, tps);
 }
 
@@ -354,7 +359,7 @@ extern "C" int irs_score_ce_bwd_tc(const float* h, int64_t ld_h, const float* W,
     cet::ce_bwd_tc_kernel<<<(unsigned)(p.n_x_tiles * p.n_splits), cet::THREADS, cet::SMEM_BYTES, s>>>(p);
     IRS_LAUNCHED();
   }
-  if (d_W != nullptr) {                                  // X = items, Y = users
+  if (d_W != nullptr || d_bias != nullptr) {             // X = items, Y = users (d_bias = the row sums of this pass)
     cet::Params p = {};
     p.ximg = wimg; p.yimg = himg; p.rowb = bias; p.row_neg = 0; p.rowid64 = nullptr; p.colb = lse; p.col_neg = 1; p.colid64 = target;
     p.RX = N; p.RY = M; p.gscale = gscale; p.out = d_W; p.ld_out = d; p.d = d; p.rowsum = d_bias; p.error_flag = error_flag;

@@ -218,9 +218,10 @@ score_simt_kernel(const ScoreParams p) {
         for (int t = 0; t < p.n_sel; ++t) {
           const int64_t c = p.sel[(int64_t)m * p.n_sel + t] - p.item_base - n0;
           if (c >= 0 && c < BN) {
+            // an id past the catalog but inside its last partial tile keeps the 0.0 it was given (acc is -inf there)
 #pragma unroll
             for (int j = 0; j < 8; ++j)
-              if (c == cn[j]) p.sel_logit[(int64_t)m * p.n_sel + t] = acc[i][j];
+              if (c == cn[j] && col_ok[j]) p.sel_logit[(int64_t)m * p.n_sel + t] = acc[i][j];
           }
         }
       }

@@ -316,7 +316,8 @@ class ShardedScorer:
         return r[mine].contiguous()
 
     def lse_gather(self, h, sel):
-        """(lse [B], logit [B,s]) over the full catalog: logit[m,t] = exact score of item sel[m,t] (0 -> 0.0)."""
+        """(lse [B], logit [B,s]) over the full catalog: logit[m,t] = exact score of item sel[m,t] (0.0 for an id outside
+        1 .. n_item, PAD included)."""
         sel = sel.reshape(h.shape[0], -1).long()
         (h_all, sel_all), mine, _ = self._gather_rows(h, sel)
         lse_loc = self.lse_fn(h_all)
@@ -327,7 +328,8 @@ class ShardedScorer:
         else:
             lse_all = lse_loc.unsqueeze(0)
         lse = torch.logsumexp(lse_all.double(), dim=0).float()
-        logit = torch.where(sel_all == 0, torch.zeros_like(logit), logit)
+        # ids outside the catalog (0 = PAD, negative, > n_item) select 0.0, as score_lse_gather does
+        logit = torch.where((sel_all < 1) | (sel_all > self.n_item), torch.zeros_like(logit), logit)
         return lse[mine].contiguous(), logit[mine].contiguous()
 
     def topk(self, h, k: int, excl_ids=None):

@@ -466,7 +466,8 @@ def prepared_scorer_weights(W) -> torch.Tensor:
 
 @_timed("lse")
 def score_lse_gather(h, W, bias, sel, item_base: int = 1):
-    """(lse [M], logit [M,s]) with logit[m,t] = score of item sel[m,t] (0 -> 0.0)."""
+    """(lse [M], logit [M,s]) with logit[m,t] = score of item sel[m,t] (0.0 for an id outside [item_base, item_base + N),
+    PAD = 0 included)."""
     h, ld = _rows(h)
     W = _need(W, torch.float32, "W")
     M, d = h.shape
