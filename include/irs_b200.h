@@ -168,6 +168,8 @@ int irs_residual_layernorm(const float* x, const float* y, const float* y_bias,
  *   epilogue 2: LN(resid + acc + bias; g1,b1,eps) and, if g2, LN(. + c2; g2,b2,eps)
  *                                     out_proj + norm1 (+ zero-memory cross-attention constant + norm2),
  *                                     linear2 + norm3
+ *               resid [R,Nout] row-major with leading dimension ldr: ldr a multiple of 4 and resid
+ *               16-byte aligned (it is read with 16-byte vector loads), else IRS_E_SHAPE.
  * error_flag: device int, set non-zero if the kernel's pipeline watchdog fires (never in normal use). */
 size_t irs_linear_prepared_bytes(int Nout, int K);
 int irs_linear_prepare_weights(const float* W, int Nout, int K, void* prepared, void* stream);

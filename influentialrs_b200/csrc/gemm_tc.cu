@@ -409,6 +409,8 @@ extern "C" int irs_linear_tc(const float* A, int64_t lda, const void* prepared, 
   if ((lda & 3) || (K & 3) || ((uintptr_t)A & 15) || (ldc & 3) || ((uintptr_t)C & 15)) return IRS_E_SHAPE;
   if (epilogue < 0 || epilogue > 2) return IRS_E_BADARG;
   if (epilogue == tcg::EPI_RESID_LN && (!resid || !g1 || !b1 || (g2 && !b2))) return IRS_E_BADARG;
+  // epilogue 2 reads resid rows with float4 loads
+  if (epilogue == tcg::EPI_RESID_LN && ((ldr & 3) || ((uintptr_t)resid & 15))) return IRS_E_SHAPE;
   cudaStream_t s = (cudaStream_t)stream;
   tcg::Params p = {};
   p.A = A; p.lda = lda; p.Wt = (const uint4*)prepared; p.bias = bias; p.resid = resid; p.ldr = ldr;

@@ -795,8 +795,11 @@ def linear_tc(A, prepared, Nout: int, bias=None, epilogue: int = EPI_BIAS, resid
     R, K = A.shape
     if out is None:
         out = torch.empty((R, Nout), dtype=torch.float32, device=A.device)
-    if resid is not None and (resid.dim() != 2 or resid.stride(1) != 1):
-        resid = resid.contiguous()
+    if resid is not None and (resid.dim() != 2 or resid.stride(1) != 1 or resid.stride(0) % 4 != 0
+                              or resid.data_ptr() % 16 != 0):
+        # the kernel reads resid rows with 16-byte vector loads: a fresh copy is aligned (contiguous() would return a
+        # misaligned contiguous view unchanged)
+        resid = resid.clone(memory_format=torch.contiguous_format)
     check(lib().irs_linear_tc(_ptr(A), A.stride(0), _ptr(prepared), _ptr(bias), int(epilogue),
                               _ptr(resid), 0 if resid is None else resid.stride(0), _ptr(g1), _ptr(b1), _ptr(c2), _ptr(g2),
                               _ptr(b2), float(eps), _ptr(out), out.stride(0), R, K, Nout, _ptr(_error_flag(A.device)),

@@ -17,7 +17,8 @@ bias shared by every row (``y_bias`` / ``bias`` / ``bo`` / ``c2`` / ``bf2``, pla
 
 The band (``ln_band``) bounds |out - LN(t)| per row, LN in fp64 of the exact t:
   KAPPA u (max_j |t_j| rstd max|g| + max|b|)   -- what holding t (and the output) in fp32 costs any implementation;
-  + TC_REL P rstd max|g|                      -- tensor-core paths: the bf16x3 product error, P = max_j sum_k |a_k w_jk|;
+  + MARGIN G(K) P rstd max|g|                 -- tensor-core paths: the bf16x3 product error of a K-deep GEMM,
+                                                 P = max_j sum_k |a_k w_jk| (G and MARGIN: tests/gemm_cases.py);
   + e rstd max|g| (2 + max_j |z_j|)           -- an error e of t from upstream (LN2 after LN1, LN3 after the FFN).
 KAPPA comes from the two-pass and Chan emulators below (KAPPA_MARGIN times the largest ratio they reach on these
 cases, tests/test_layernorm_cond_cpu.py), not from GPU output.
@@ -29,10 +30,11 @@ from typing import Optional
 
 import numpy as np
 
+from tests.gemm_cases import band_rel
+
 U = 2.0 ** -24                  # fp32 unit roundoff
 KAPPA = 24.0                    # >= KAPPA_MARGIN x the largest error of the emulators in units of the band: 11.1
 KAPPA_MARGIN = 2.0
-TC_REL = 3e-5                   # bf16x3 product error, relative to sum_k |a_k w_k| (the suite's band for these kernels)
 RATIOS = (1.0, 10.0, 30.0, 100.0, 1e3, 1e4)
 DISCRIMINATING = 30.0           # the one-pass statistics leave the band at every |mean|/std >= this
 
@@ -111,21 +113,50 @@ def ln64(t64: np.ndarray, g, b, eps: float) -> np.ndarray:
     return (t64 - m) / np.sqrt(v + eps) * np.asarray(g, np.float64) + np.asarray(b, np.float64)
 
 
-def ln_band(t64: np.ndarray, g, b, eps: float, prod: Optional[np.ndarray] = None,
+def ln_band(t64: np.ndarray, g, b, eps: float, prod: Optional[np.ndarray] = None, k: Optional[int] = None,
             upstream: Optional[np.ndarray] = None) -> np.ndarray:
-    """Per-row bound on |out - ln64(t64)| (module docstring).  ``prod`` [R]: product scale of a tensor-core GEMM inside
-    t; ``upstream`` [R]: a bound on the error of t itself."""
+    """Per-row bound on |out - ln64(t64)| (module docstring).  ``prod`` [R]: product scale of a tensor-core GEMM of depth
+    ``k`` inside t; ``upstream`` [R]: a bound on the error of t itself."""
     m = t64.mean(1, keepdims=True)
     rstd = 1.0 / np.sqrt(((t64 - m) ** 2).mean(1) + eps)
     gmax = float(np.abs(np.asarray(g, np.float64)).max())
     bmax = float(np.abs(np.asarray(b, np.float64)).max())
     band = KAPPA * U * (np.abs(t64).max(1) * rstd * gmax + bmax)
     if prod is not None:
-        band = band + TC_REL * prod * rstd * gmax
+        band = band + band_rel(k) * prod * rstd * gmax
     if upstream is not None:
         zmax = (np.abs(t64 - m).max(1)) * rstd
         band = band + upstream * rstd * gmax * (2.0 + zmax)
     return band
+
+
+def abs_prod(a, w) -> np.ndarray:
+    """P = max_j sum_k |a_k w_jk| per row."""
+    return (np.abs(np.asarray(a, np.float64)) @ np.abs(np.asarray(w, np.float64)).T).max(1)
+
+
+def inf_norm(w) -> float:
+    return float(np.abs(np.asarray(w, np.float64)).sum(1).max())
+
+
+def chain_bands(attn, x, P, eps=1e-5):
+    """fp64 decoder chain (out_proj + LN1 + LN2, linear1 + relu + linear2 + LN3, next in_proj) and the per-row bands of
+    x' and qkv', each GEMM's error propagated with the band of its own depth (128, or 256 for linear2).  P holds the
+    float32 parameters by name."""
+    D = lambda k: np.asarray(P[k], np.float64)
+    t1 = x.astype(np.float64) + attn.astype(np.float64) @ D("Wo").T + D("bo")
+    band1 = ln_band(t1, P["g1"], P["b1"], eps, prod=abs_prod(attn, P["Wo"]), k=128)
+    t2 = ln64(t1, P["g1"], P["b1"], eps) + D("c2")
+    band2 = ln_band(t2, P["g2"], P["b2"], eps, upstream=band1)
+    y = ln64(t2, P["g2"], P["b2"], eps)
+    f = np.maximum(y @ D("W1").T + D("bf1"), 0.0)
+    e_f = inf_norm(P["W1"]) * band2 + band_rel(128) * abs_prod(y, P["W1"]) + 2 * U * np.abs(f).max(1)  # relu: 1-Lipschitz
+    t3 = y + f @ D("W2").T + D("bf2")
+    band3 = ln_band(t3, P["g3"], P["b3"], eps, prod=abs_prod(f, P["W2"]), k=256, upstream=band2 + inf_norm(P["W2"]) * e_f)
+    xo = ln64(t3, P["g3"], P["b3"], eps)
+    qkv = xo @ D("Win").T + D("bin")
+    band_q = inf_norm(P["Win"]) * band3 + band_rel(128) * abs_prod(xo, P["Win"]) + 2 * U * np.abs(qkv).max(1)
+    return xo, band3, qkv, band_q
 
 
 def row_err(out, want) -> np.ndarray:

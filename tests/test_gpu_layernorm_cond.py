@@ -39,15 +39,6 @@ def _check(got, want, band, what, ratio=None):
                              f"err {err[w]:.3e} band {band[w]:.3e}")
 
 
-def _abs_prod(a, w):
-    """P = max_j sum_k |a_k w_jk| per row."""
-    return (np.abs(np.asarray(a, np.float64)) @ np.abs(np.asarray(w, np.float64)).T).max(1)
-
-
-def _inf_norm(w):
-    return float(np.abs(np.asarray(w, np.float64)).sum(1).max())
-
-
 # ---------------------------------------------------------------------------------------------- residual_layernorm
 @pytest.mark.parametrize("two", [False, True])
 @pytest.mark.parametrize("eps", [1e-5, 1e-8])
@@ -89,7 +80,7 @@ def test_linear_tc_layernorm_large_mean(ops, K, Nout, placement, two):
         g2, b2 = C.ln_params(Nout, seed=1)
         c2 = np.full(Nout, sign * 1e3, np.float32)
         t = rows.x.astype(np.float64) + A.astype(np.float64) @ W.astype(np.float64).T + rows.bias
-        band1 = C.ln_band(t, g1, b1, eps, prod=_abs_prod(A, W))
+        band1 = C.ln_band(t, g1, b1, eps, prod=C.abs_prod(A, W), k=K)
         prep = ops.linear_prepare(_d(W))
         if not two:
             got = ops.linear_tc(_d(A), prep, Nout, _d(rows.bias), ops.EPI_RESID_LN, resid=_d(rows.x), g1=_d(g1), b1=_d(b1),
@@ -129,31 +120,13 @@ def _chain_case(stage, placement, v, R=333, d=128, ffn=256):
     return attn, x, P, ratio
 
 
-def _chain_bands(attn, x, P, eps=1e-5):
-    """fp64 chain (as _chain_reference in test_gpu_kernels.py) and the per-row bands of x' and qkv'."""
-    D = lambda k: P[k].astype(np.float64)
-    t1 = x.astype(np.float64) + attn.astype(np.float64) @ D("Wo").T + D("bo")
-    band1 = C.ln_band(t1, P["g1"], P["b1"], eps, prod=_abs_prod(attn, P["Wo"]))
-    t2 = C.ln64(t1, P["g1"], P["b1"], eps) + D("c2")
-    band2 = C.ln_band(t2, P["g2"], P["b2"], eps, upstream=band1)
-    y = C.ln64(t2, P["g2"], P["b2"], eps)
-    f = np.maximum(y @ D("W1").T + D("bf1"), 0.0)
-    e_f = _inf_norm(P["W1"]) * band2 + C.TC_REL * _abs_prod(y, P["W1"])          # relu is 1-Lipschitz
-    t3 = y + f @ D("W2").T + D("bf2")
-    band3 = C.ln_band(t3, P["g3"], P["b3"], eps, prod=_abs_prod(f, P["W2"]), upstream=band2 + _inf_norm(P["W2"]) * e_f)
-    xo = C.ln64(t3, P["g3"], P["b3"], eps)
-    qkv = xo @ D("Win").T + D("bin")
-    band_q = _inf_norm(P["Win"]) * band3 + C.TC_REL * _abs_prod(xo, P["Win"])
-    return xo, band3, qkv, band_q
-
-
 @pytest.mark.parametrize("with_qkv,inplace", [(True, False), (False, True), (True, True)])
 @pytest.mark.parametrize("stage,placement,v", CHAIN)
 def test_decoder_chain_layernorms_large_mean(ops, stage, placement, v, with_qkv, inplace):
     """One of LN1 / LN2 / LN3 conditioned at a time, R = 333 (a partial tile), in place or not, with and without the
     next layer's in_proj; x' and qkv' against the same fp64 chain."""
     attn, x, P, ratio = _chain_case(stage, placement, v)
-    want_x, band_x, want_q, band_q = _chain_bands(attn, x, P)
+    want_x, band_x, want_q, band_q = C.chain_bands(attn, x, P)
     Pd = {k: _d(a) for k, a in P.items()}
     xd = _d(x)
     prep = ops.decoder_chain_prepare(Pd["Wo"], Pd["W1"], Pd["W2"], Pd["Win"] if with_qkv else None)

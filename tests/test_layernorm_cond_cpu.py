@@ -2,6 +2,8 @@
 statistics stay inside it on every case, and the one-pass E[t^2] - mean^2 leaves it at every |mean|/std the GPU tests
 (tests/test_gpu_layernorm_cond.py) rely on, in both the linear_tc and the decoder-chain layouts.  So the GPU tests can
 tell the two apart."""
+import math
+
 import numpy as np
 import pytest
 
@@ -114,3 +116,24 @@ def test_kappa_has_its_margin():
         for meth, lay in _layouts(n):
             worst = max(worst, float((C.row_err(C.emulate_ln(t, g, b, 1e-5, meth, lay), want) / unit).max()))
     assert 4.0 < worst <= C.KAPPA / C.KAPPA_MARGIN, worst
+
+
+@pytest.mark.parametrize("placement", ["row", "bias"])
+@pytest.mark.parametrize("K,Nout", [(32, 16), (120, 120), (128, 128), (256, 256)])
+def test_one_pass_leaves_the_band_with_the_product_term(K, Nout, placement):
+    """The linear_tc cases of tests/test_gpu_layernorm_cond.py, band and all: the tensor-core product term (2 G(K) P,
+    up to about a fifth of the band at |mean|/std = 30) does not hide the one-pass statistics."""
+    import math
+    eps = 1e-5
+    for sign in (1.0, -1.0):
+        rows = C.ln_rows(Nout, placement, sign)
+        rng = np.random.default_rng(K + Nout)
+        A = (rng.standard_normal((rows.x.shape[0], K)) * rows.scale[:, None] * 0.01).astype(np.float32)
+        W = (rng.standard_normal((Nout, K)) / math.sqrt(K)).astype(np.float32)
+        g, b = C.ln_params(Nout)
+        prod64 = A.astype(np.float64) @ W.astype(np.float64).T
+        t64 = rows.t64 + prod64
+        band = C.ln_band(t64, g, b, eps, prod=C.abs_prod(A, W), k=K)
+        r = C.row_err(C.emulate_ln(C.emulate_input(rows, prod64), g, b, eps, "one-pass", "row"), C.ln64(t64, g, b, eps)) / band
+        for q in _ratio_groups(rows):
+            assert r[np.isclose(rows.ratio, q, rtol=0.05)].max() > 3.0, f"one-pass inside the band at |mean|/std = {q:g}"
