@@ -1,7 +1,28 @@
-// ABI bookkeeping: version, error strings, launch counter.
+// ABI bookkeeping: version, error strings, launch counter; the shared-memory opt-in table.
+#include <map>
+#include <mutex>
+#include <utility>
 #include "common.cuh"
 
-namespace irs { long long g_launches = 0; }
+namespace irs {
+
+long long g_launches = 0;
+
+cudaError_t opt_in_smem(const void* kernel, size_t bytes) {
+  static std::mutex mu;
+  static std::map<std::pair<const void*, int>, size_t> granted;
+  int dev;
+  const cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  std::lock_guard<std::mutex> lock(mu);
+  size_t& have = granted[{kernel, dev}];
+  if (bytes <= have) return cudaSuccess;
+  const cudaError_t r = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (r == cudaSuccess) have = bytes;
+  return r;
+}
+
+}  // namespace irs
 
 extern "C" int irs_abi_version(void) { return IRS_B200_ABI_VERSION; }
 

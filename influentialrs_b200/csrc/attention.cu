@@ -764,52 +764,11 @@ static int attn_drop_args(float p_drop, uint32_t* thresh, float* inv_keep) {
   return 0;
 }
 
-static int attn_fwd_blocked_launch(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
-                                   const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
-                                   float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
-                                   uint32_t drop_thresh, float inv_keep, unsigned long long seed, void* stream) {
-  if (L > IRS_ATTN_MAX_L || dh > irs::kBlkMaxDh) return IRS_E_SHAPE;
-  const size_t bytes = (size_t)irs::blk_smem_layout(dh, 1, 1).total_floats * sizeof(float);
-  static size_t configured = 0;
-  if (bytes > configured) {
-    IRS_CUDA(cudaFuncSetAttribute(irs::pim_attn_fwd_blocked_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    configured = bytes;
-  }
-  dim3 grid((unsigned)(B * H), (unsigned)((n_q + irs::kBlkRows - 1) / irs::kBlkRows));
-  irs::pim_attn_fwd_blocked_kernel<<<grid, irs::kAttWarps * 32, bytes, (cudaStream_t)stream>>>(
-      q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, L, H, dh, q_row0, n_q, seed, drop_thresh, inv_keep);
-  IRS_LAUNCHED();
-  return 0;
-}
-
-static int attn_bwd_blocked_launch(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
-                                   const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
-                                   const float* out, const float* lse, const float* d_out,
-                                   float* d_q, float* d_k, float* d_v, float* d_r_u, int B, int L, int H, int dh,
-                                   uint32_t drop_thresh, float inv_keep, unsigned long long seed, void* stream) {
-  if (L > IRS_ATTN_MAX_L || dh > irs::kBlkMaxDh) return IRS_E_SHAPE;
-  const size_t bytes_q = (size_t)irs::blk_smem_layout(dh, 2, 1).total_floats * sizeof(float);
-  const size_t bytes_kv = (size_t)irs::blk_smem_layout(dh, 2, 2).total_floats * sizeof(float);
-  static size_t configured = 0;
-  if (bytes_kv > configured) {
-    IRS_CUDA(cudaFuncSetAttribute(irs::pim_attn_bwd_dq_blocked_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes_q));
-    IRS_CUDA(cudaFuncSetAttribute(irs::pim_attn_bwd_dkv_blocked_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes_kv));
-    configured = bytes_kv;
-  }
-  dim3 grid((unsigned)(B * H), (unsigned)((L + irs::kBlkRows - 1) / irs::kBlkRows));
-  irs::pim_attn_bwd_dq_blocked_kernel<<<grid, irs::kAttWarps * 32, bytes_q, (cudaStream_t)stream>>>(
-      q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, d_out, d_q, d_r_u, L, H, dh, seed, drop_thresh, inv_keep);
-  IRS_LAUNCHED();
-  irs::pim_attn_bwd_dkv_blocked_kernel<<<grid, irs::kAttWarps * 32, bytes_kv, (cudaStream_t)stream>>>(
-      q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, d_out, d_k, d_v, L, H, dh, seed, drop_thresh, inv_keep);
-  IRS_LAUNCHED();
-  return 0;
-}
-
-extern "C" int irs_pim_attn_fwd(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
-                                const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
-                                float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
-                                float p_drop, unsigned long long seed, void* stream) {
+// The routed entry points stream the window in key blocks when it does not fit on chip; the _blocked ones always do.
+static int attn_fwd(bool blocked, const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
+                    const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
+                    float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
+                    float p_drop, unsigned long long seed, void* stream) {
   int rc = attn_check(q, k, v, ids, r_u, mode, B, L, H, dh);
   if (rc) return rc;
   if (!out || q_row0 < 0 || n_q <= 0 || q_row0 + n_q > L) return IRS_E_BADARG;
@@ -817,16 +776,19 @@ extern "C" int irs_pim_attn_fwd(const float* q, const float* k, const float* v, 
   float inv_keep;
   if ((rc = attn_drop_args(p_drop, &drop_thresh, &inv_keep))) return rc;
   if (L > IRS_ATTN_MAX_L) return IRS_E_SHAPE;
-  const irs::AttnSmem lay = irs::attn_smem_layout(L, dh);
-  const size_t bytes = (size_t)lay.total_floats * sizeof(float);
-  if (bytes > 227 * 1024)    // the window does not fit on chip: stream it in key blocks
-    return attn_fwd_blocked_launch(q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, B, L, H, dh, q_row0, n_q,
-                                   drop_thresh, inv_keep, seed, stream);
-  static size_t configured = 0;
-  if (bytes > configured) {
-    IRS_CUDA(cudaFuncSetAttribute(irs::pim_attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    configured = bytes;
+  const cudaStream_t s = (cudaStream_t)stream;
+  const size_t bytes = (size_t)irs::attn_smem_layout(L, dh).total_floats * sizeof(float);
+  if (blocked || bytes > 227 * 1024) {
+    if (dh > irs::kBlkMaxDh) return IRS_E_SHAPE;
+    const size_t bytes_blk = (size_t)irs::blk_smem_layout(dh, 1, 1).total_floats * sizeof(float);
+    IRS_CUDA(irs::opt_in_smem(irs::pim_attn_fwd_blocked_kernel, bytes_blk));
+    dim3 grid((unsigned)(B * H), (unsigned)((n_q + irs::kBlkRows - 1) / irs::kBlkRows));
+    irs::pim_attn_fwd_blocked_kernel<<<grid, irs::kAttWarps * 32, bytes_blk, s>>>(
+        q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, L, H, dh, q_row0, n_q, seed, drop_thresh, inv_keep);
+    IRS_LAUNCHED();
+    return 0;
   }
+  IRS_CUDA(irs::opt_in_smem(irs::pim_attn_fwd_kernel, bytes));
   // Enough CTAs to fill the machine: split the query rows when B*H alone is too few.
   int chunks = 1;
   const int per_pass = irs::kAttWarps * irs::kAttRows;
@@ -835,32 +797,18 @@ extern "C" int irs_pim_attn_fwd(const float* q, const float* k, const float* v, 
   rows_per_cta = ((rows_per_cta + irs::kAttRows - 1) / irs::kAttRows) * irs::kAttRows;
   chunks = (n_q + rows_per_cta - 1) / rows_per_cta;
   dim3 grid((unsigned)(B * H), (unsigned)chunks);
-  irs::pim_attn_fwd_kernel<<<grid, irs::kAttWarps * 32, bytes, (cudaStream_t)stream>>>(
+  irs::pim_attn_fwd_kernel<<<grid, irs::kAttWarps * 32, bytes, s>>>(
       q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, L, H, dh, q_row0, n_q, rows_per_cta,
       seed, drop_thresh, inv_keep);
   IRS_LAUNCHED();
   return 0;
 }
 
-extern "C" int irs_pim_attn_fwd_blocked(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
-                                        const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
-                                        float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
-                                        float p_drop, unsigned long long seed, void* stream) {
-  int rc = attn_check(q, k, v, ids, r_u, mode, B, L, H, dh);
-  if (rc) return rc;
-  if (!out || q_row0 < 0 || n_q <= 0 || q_row0 + n_q > L) return IRS_E_BADARG;
-  uint32_t drop_thresh;
-  float inv_keep;
-  if ((rc = attn_drop_args(p_drop, &drop_thresh, &inv_keep))) return rc;
-  return attn_fwd_blocked_launch(q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, B, L, H, dh, q_row0, n_q,
-                                 drop_thresh, inv_keep, seed, stream);
-}
-
-extern "C" int irs_pim_attn_bwd(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
-                                const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
-                                const float* out, const float* lse, const float* d_out,
-                                float* d_q, float* d_k, float* d_v, float* d_r_u,
-                                int B, int L, int H, int dh, float p_drop, unsigned long long seed, void* stream) {
+static int attn_bwd(bool blocked, const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
+                    const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
+                    const float* out, const float* lse, const float* d_out,
+                    float* d_q, float* d_k, float* d_v, float* d_r_u,
+                    int B, int L, int H, int dh, float p_drop, unsigned long long seed, void* stream) {
   int rc = attn_check(q, k, v, ids, r_u, mode, B, L, H, dh);
   if (rc) return rc;
   if (!out || !lse || !d_out || !d_q || !d_k || !d_v) return IRS_E_BADARG;
@@ -868,21 +816,54 @@ extern "C" int irs_pim_attn_bwd(const float* q, const float* k, const float* v, 
   float inv_keep;
   if ((rc = attn_drop_args(p_drop, &drop_thresh, &inv_keep))) return rc;
   if (L > IRS_ATTN_MAX_L) return IRS_E_SHAPE;
-  const irs::AttnBwdSmem lay = irs::attn_bwd_smem_layout(L, dh);
-  const size_t bytes = (size_t)lay.total_floats * sizeof(float);
-  if (bytes > 227 * 1024)
-    return attn_bwd_blocked_launch(q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, d_out, d_q, d_k, d_v, d_r_u,
-                                   B, L, H, dh, drop_thresh, inv_keep, seed, stream);
-  static size_t configured = 0;
-  if (bytes > configured) {
-    IRS_CUDA(cudaFuncSetAttribute(irs::pim_attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    configured = bytes;
+  const cudaStream_t s = (cudaStream_t)stream;
+  const size_t bytes = (size_t)irs::attn_bwd_smem_layout(L, dh).total_floats * sizeof(float);
+  if (blocked || bytes > 227 * 1024) {
+    if (dh > irs::kBlkMaxDh) return IRS_E_SHAPE;
+    const size_t bytes_q = (size_t)irs::blk_smem_layout(dh, 2, 1).total_floats * sizeof(float);
+    const size_t bytes_kv = (size_t)irs::blk_smem_layout(dh, 2, 2).total_floats * sizeof(float);
+    IRS_CUDA(irs::opt_in_smem(irs::pim_attn_bwd_dq_blocked_kernel, bytes_q));
+    IRS_CUDA(irs::opt_in_smem(irs::pim_attn_bwd_dkv_blocked_kernel, bytes_kv));
+    dim3 grid((unsigned)(B * H), (unsigned)((L + irs::kBlkRows - 1) / irs::kBlkRows));
+    irs::pim_attn_bwd_dq_blocked_kernel<<<grid, irs::kAttWarps * 32, bytes_q, s>>>(
+        q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, d_out, d_q, d_r_u, L, H, dh, seed, drop_thresh, inv_keep);
+    IRS_LAUNCHED();
+    irs::pim_attn_bwd_dkv_blocked_kernel<<<grid, irs::kAttWarps * 32, bytes_kv, s>>>(
+        q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, d_out, d_k, d_v, L, H, dh, seed, drop_thresh, inv_keep);
+    IRS_LAUNCHED();
+    return 0;
   }
-  irs::pim_attn_bwd_kernel<<<(unsigned)(B * H), irs::kAttWarps * 32, bytes, (cudaStream_t)stream>>>(
+  IRS_CUDA(irs::opt_in_smem(irs::pim_attn_bwd_kernel, bytes));
+  irs::pim_attn_bwd_kernel<<<(unsigned)(B * H), irs::kAttWarps * 32, bytes, s>>>(
       q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, d_out, d_q, d_k, d_v, d_r_u, L, H, dh,
       seed, drop_thresh, inv_keep);
   IRS_LAUNCHED();
   return 0;
+}
+
+extern "C" int irs_pim_attn_fwd(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
+                                const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
+                                float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
+                                float p_drop, unsigned long long seed, void* stream) {
+  return attn_fwd(false, q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, B, L, H, dh, q_row0, n_q,
+                  p_drop, seed, stream);
+}
+
+extern "C" int irs_pim_attn_fwd_blocked(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
+                                        const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
+                                        float* out, float* lse, int B, int L, int H, int dh, int q_row0, int n_q,
+                                        float p_drop, unsigned long long seed, void* stream) {
+  return attn_fwd(true, q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, B, L, H, dh, q_row0, n_q,
+                  p_drop, seed, stream);
+}
+
+extern "C" int irs_pim_attn_bwd(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
+                                const int64_t* ids, const float* r_u, float w_h, float w_obj, int mode,
+                                const float* out, const float* lse, const float* d_out,
+                                float* d_q, float* d_k, float* d_v, float* d_r_u,
+                                int B, int L, int H, int dh, float p_drop, unsigned long long seed, void* stream) {
+  return attn_bwd(false, q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, d_out, d_q, d_k, d_v, d_r_u,
+                  B, L, H, dh, p_drop, seed, stream);
 }
 
 extern "C" int irs_pim_attn_bwd_blocked(const float* q, const float* k, const float* v, int64_t ld_q, int64_t ld_k, int64_t ld_v,
@@ -890,12 +871,6 @@ extern "C" int irs_pim_attn_bwd_blocked(const float* q, const float* k, const fl
                                         const float* out, const float* lse, const float* d_out,
                                         float* d_q, float* d_k, float* d_v, float* d_r_u,
                                         int B, int L, int H, int dh, float p_drop, unsigned long long seed, void* stream) {
-  int rc = attn_check(q, k, v, ids, r_u, mode, B, L, H, dh);
-  if (rc) return rc;
-  if (!out || !lse || !d_out || !d_q || !d_k || !d_v) return IRS_E_BADARG;
-  uint32_t drop_thresh;
-  float inv_keep;
-  if ((rc = attn_drop_args(p_drop, &drop_thresh, &inv_keep))) return rc;
-  return attn_bwd_blocked_launch(q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, d_out, d_q, d_k, d_v, d_r_u,
-                                 B, L, H, dh, drop_thresh, inv_keep, seed, stream);
+  return attn_bwd(true, q, k, v, ld_q, ld_k, ld_v, ids, r_u, w_h, w_obj, mode, out, lse, d_out, d_q, d_k, d_v, d_r_u,
+                  B, L, H, dh, p_drop, seed, stream);
 }

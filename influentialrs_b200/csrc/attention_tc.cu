@@ -746,11 +746,7 @@ static tca::Params attn_tc_params(const float* q, const float* k, const float* v
 
 static int attn_tc_blocked_launch(const tca::Params& p, void* stream) {
   const tcb::Layout lay = tcb::make_layout(p.dh);
-  static uint32_t configured = 0;
-  if (lay.total > configured) {
-    IRS_CUDA(cudaFuncSetAttribute(tcb::pim_attn_tc_blocked_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.total));
-    configured = lay.total;
-  }
+  IRS_CUDA(opt_in_smem(tcb::pim_attn_tc_blocked_kernel, lay.total));
   const int tiles = (p.q_row0 + p.n_q - 1) / tcb::BM - p.q_row0 / tcb::BM + 1;
   dim3 grid((unsigned)(p.B * p.H), (unsigned)tiles);
   tcb::pim_attn_tc_blocked_kernel<<<grid, tcb::THREADS, lay.total, (cudaStream_t)stream>>>(p);
@@ -768,11 +764,7 @@ extern "C" int irs_pim_attn_fwd_tc(const float* q, const float* k, const float* 
                                        q_row0, n_q, error_flag);
   if (L > tca::KEYS_MAX - 1) return attn_tc_blocked_launch(p, stream);    // the head's K / V^T no longer fit on chip
   const tca::Layout lay = tca::make_layout(dh);
-  static uint32_t configured = 0;
-  if (lay.total > configured) {
-    IRS_CUDA(cudaFuncSetAttribute(tca::pim_attn_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.total));
-    configured = lay.total;
-  }
+  IRS_CUDA(opt_in_smem(tca::pim_attn_tc_kernel, lay.total));
   tca::pim_attn_tc_kernel<<<(unsigned)(B * H), tca::THREADS, lay.total, (cudaStream_t)stream>>>(p);
   IRS_LAUNCHED();
   return 0;

@@ -644,11 +644,6 @@ extern "C" int irs_pim_attn_fwd_img(const void* images, const int64_t* ids, cons
   if (!irs_pim_attn_img_supported(L, dh)) return IRS_E_SHAPE;
   if (!(n_q == L || n_q == 1)) return IRS_E_SHAPE;             // all rows, or exactly one
   if (((uintptr_t)images & 15) || ((uintptr_t)out & 31)) return IRS_E_SHAPE;
-  static bool configured = false;
-  if (!configured) {
-    IRS_CUDA(cudaFuncSetAttribute(tcp::pim_attn_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcp::SMEM_BYTES));
-    configured = true;
-  }
   tcp::Params p = {};
   p.images = (const uint8_t*)images; p.ids = ids; p.r_u = r_u; p.w_h = w_h; p.w_obj = w_obj; p.mode = mode;
   p.out = out; p.B = B; p.L = L; p.H = H; p.n_items = B * H; p.q_row = (n_q == L) ? -1 : q_row0;
@@ -663,6 +658,7 @@ extern "C" int irs_pim_attn_fwd_img(const void* images, const int64_t* ids, cons
     return 0;
   }
   const unsigned grid = (unsigned)(p.n_items < kNumSMs ? p.n_items : kNumSMs);
+  IRS_CUDA(opt_in_smem(tcp::pim_attn_persistent_kernel, tcp::SMEM_BYTES));
   tcp::pim_attn_persistent_kernel<<<grid, tcp::THREADS, tcp::SMEM_BYTES, (cudaStream_t)stream>>>(p);
   IRS_LAUNCHED();
   return 0;

@@ -22,6 +22,13 @@ extern long long g_launches;   // counted by IRS_LAUNCHED(), read through irs_la
     if (e__ != cudaSuccess) return (int)e__;             \
   } while (0)
 
+// Lets `kernel` use `bytes` of dynamic shared memory on the current device.  The attribute is held per device, so the
+// table of what was granted is keyed on (kernel address, device); the driver is called only to raise the limit, and
+// steady-state launches make no call.  Thread-safe.
+cudaError_t opt_in_smem(const void* kernel, size_t bytes);
+template <typename... Args>
+inline cudaError_t opt_in_smem(void (*kernel)(Args...), size_t bytes) { return opt_in_smem((const void*)kernel, bytes); }
+
 constexpr int kNumSMs = 148;   // B200: 2 dies x 74 SMs
 
 __host__ __device__ inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }

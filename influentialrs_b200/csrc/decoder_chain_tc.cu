@@ -667,11 +667,7 @@ static int chain_launch(tcl::Params& p, int64_t R, int* error_flag, void* stream
   p.R = R; p.n_tiles = ceil_div(R, tcl::BM);
   p.error_flag = error_flag;
   p.timeline = g_chain_timeline;
-  static bool configured = false;
-  if (!configured) {
-    IRS_CUDA(cudaFuncSetAttribute(tcl::decoder_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcl::SMEM_BYTES));
-    configured = true;
-  }
+  IRS_CUDA(opt_in_smem(tcl::decoder_chain_kernel, tcl::SMEM_BYTES));
   const unsigned grid = (unsigned)(p.n_tiles < kNumSMs ? p.n_tiles : kNumSMs);
   tcl::decoder_chain_kernel<<<grid, tcl::THREADS, tcl::SMEM_BYTES, (cudaStream_t)stream>>>(p);
   IRS_LAUNCHED();

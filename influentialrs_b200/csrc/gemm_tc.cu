@@ -418,19 +418,11 @@ extern "C" int irs_linear_tc(const float* A, int64_t lda, const void* prepared, 
   p.R = R; p.K = K; p.Nout = Nout; p.n_pad = pad16(Nout); p.n_chunks = (K + tcg::KC - 1) / tcg::KC;
   p.n_tiles = ceil_div(R, tcg::BM);
   p.error_flag = error_flag;
-  static bool configured = false;
-  if (!configured) {
-    IRS_CUDA(cudaFuncSetAttribute(tcg::linear_tc_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcg::SMEM_BYTES));
-    IRS_CUDA(cudaFuncSetAttribute(tcg::linear_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcg::SMEM_BYTES));
-    IRS_CUDA(cudaFuncSetAttribute(tcg::linear_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcg::SMEM_BYTES));
-    configured = true;
-  }
   const unsigned grid = (unsigned)(p.n_tiles < kNumSMs ? p.n_tiles : kNumSMs);
-  switch (epilogue) {
-    case 0: tcg::linear_tc_kernel<0><<<grid, tcg::THREADS, tcg::SMEM_BYTES, s>>>(p); break;
-    case 1: tcg::linear_tc_kernel<1><<<grid, tcg::THREADS, tcg::SMEM_BYTES, s>>>(p); break;
-    default: tcg::linear_tc_kernel<2><<<grid, tcg::THREADS, tcg::SMEM_BYTES, s>>>(p); break;
-  }
+  void (*const kernels[])(tcg::Params) = {tcg::linear_tc_kernel<0>, tcg::linear_tc_kernel<1>, tcg::linear_tc_kernel<2>};
+  const auto kernel = kernels[epilogue];
+  IRS_CUDA(opt_in_smem(kernel, tcg::SMEM_BYTES));
+  kernel<<<grid, tcg::THREADS, tcg::SMEM_BYTES, s>>>(p);
   IRS_LAUNCHED();
   return 0;
 }

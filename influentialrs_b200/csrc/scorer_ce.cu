@@ -199,18 +199,14 @@ extern "C" int irs_score_ce_bwd(const float* h, int64_t ld_h, const float* W, co
   if (d > ce::DMAX) return IRS_E_SHAPE;
   cudaStream_t s = (cudaStream_t)stream;
   const size_t bytes = sizeof(ce::Smem);
-  static bool configured = false;
-  if (!configured) {
-    IRS_CUDA(cudaFuncSetAttribute(ce_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    IRS_CUDA(cudaFuncSetAttribute(ce_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    configured = true;
-  }
   if (d_h != nullptr) {
+    IRS_CUDA(opt_in_smem(ce_bwd_kernel<true>, bytes));
     ce_bwd_kernel<true><<<(unsigned)ceil_div(M, 128), ce::kThreads, bytes, s>>>(
         h, ld_h, W, bias, target, lse, gscale, d_h, nullptr, nullptr, M, N, d);
     IRS_LAUNCHED();
   }
   if (d_W != nullptr || d_bias != nullptr) {             // d_bias comes out of the d_W pass
+    IRS_CUDA(opt_in_smem(ce_bwd_kernel<false>, bytes));
     ce_bwd_kernel<false><<<(unsigned)ceil_div(N, 128), ce::kThreads, bytes, s>>>(
         h, ld_h, W, bias, target, lse, gscale, nullptr, d_W, d_bias, M, N, d);
     IRS_LAUNCHED();

@@ -321,9 +321,17 @@ static void plan(int64_t RX, int64_t RY, int& n_x, int& n_y, int& n_splits, int&
 
 using namespace irs;
 
+// workspace: the bf16 operand image of h, then that of W, then the error flag
+struct CeBwdTcLayout { size_t wimg, flag, total; };
+static CeBwdTcLayout ce_bwd_tc_layout(int M, int64_t N) {
+  const size_t wimg = (size_t)ceil_div(M, cet::BM) * cet::TILE_BYTES;
+  const size_t flag = wimg + (size_t)ceil_div(N, cet::BM) * cet::TILE_BYTES;
+  return {wimg, flag, flag + 256};
+}
+
 extern "C" size_t irs_score_ce_bwd_tc_workspace_bytes(int M, int64_t N, int d) {
   if (M <= 0 || N <= 0 || d <= 0 || d > cet::DP) return 0;
-  return (size_t)(ceil_div(M, cet::BM) + ceil_div(N, cet::BM)) * cet::TILE_BYTES + 256;
+  return ce_bwd_tc_layout(M, N).total;
 }
 
 extern "C" int irs_score_ce_bwd_tc(const float* h, int64_t ld_h, const float* W, const float* bias,
@@ -336,19 +344,16 @@ extern "C" int irs_score_ce_bwd_tc(const float* h, int64_t ld_h, const float* W,
   if (workspace_bytes < irs_score_ce_bwd_tc_workspace_bytes(M, N, d)) return IRS_E_WORKSPACE;
   if ((uintptr_t)workspace & 15) return IRS_E_SHAPE;
   cudaStream_t s = (cudaStream_t)stream;
+  const CeBwdTcLayout lay = ce_bwd_tc_layout(M, N);
   uint8_t* himg = (uint8_t*)workspace;
-  uint8_t* wimg = himg + (size_t)ceil_div(M, cet::BM) * cet::TILE_BYTES;
-  int* error_flag = (int*)(wimg + (size_t)ceil_div(N, cet::BM) * cet::TILE_BYTES);
+  uint8_t* wimg = himg + lay.wimg;
+  int* error_flag = (int*)(himg + lay.flag);
   IRS_CUDA(cudaMemsetAsync(error_flag, 0, sizeof(int), s));
   cet::prepare_rows_kernel<<<kNumSMs * 8, 256, 0, s>>>(h, ld_h, M, d, (uint4*)himg);
   IRS_LAUNCHED();
   cet::prepare_rows_kernel<<<kNumSMs * 8, 256, 0, s>>>(W, d, N, d, (uint4*)wimg);
   IRS_LAUNCHED();
-  static bool configured = false;
-  if (!configured) {
-    IRS_CUDA(cudaFuncSetAttribute(cet::ce_bwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cet::SMEM_BYTES));
-    configured = true;
-  }
+  IRS_CUDA(opt_in_smem(cet::ce_bwd_tc_kernel, cet::SMEM_BYTES));
   if (d_h != nullptr) {                                  // X = users, Y = items
     cet::Params p = {};
     p.ximg = himg; p.yimg = wimg; p.rowb = lse; p.row_neg = 1; p.rowid64 = target; p.colb = bias; p.col_neg = 0; p.colid64 = nullptr;

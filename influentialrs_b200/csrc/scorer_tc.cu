@@ -959,10 +959,16 @@ static long long* g_scorer_timeline = nullptr;
 /* debug hook (not in the public header): device buffer of 3*64*4 int64 receiving CTA 0's per-tile time stamps */
 extern "C" void irs_scorer_debug_timeline(long long* buf) { g_scorer_timeline = buf; }
 
+static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
+
+// The prepared image is the weight tiles followed by a 256-byte tail holding max_j |W_j|^2; this is where the tail starts.
+static size_t wmax2_offset(int64_t N, int d) {
+  return (size_t)ceil_div(N, tc::BN) * ((d + tc::KC - 1) / tc::KC) * tc::STAGE_BYTES;
+}
+
 extern "C" size_t irs_scorer_prepared_bytes(int64_t N, int d) {
   if (N <= 0 || d <= 0 || d > tc::KMAX_SINGLE) return 0;      // d in (128, 256]: single-MMA consumers only (arg-max, top-k)
-  const int n_chunks = (d + tc::KC - 1) / tc::KC;
-  return (size_t)ceil_div(N, tc::BN) * n_chunks * tc::STAGE_BYTES + 256;      // + tail: max_j |W_j|^2
+  return wmax2_offset(N, d) + 256;
 }
 
 extern "C" int irs_scorer_prepare_weights(const float* W, int64_t N, int d, void* prepared, void* stream) {
@@ -971,19 +977,60 @@ extern "C" int irs_scorer_prepare_weights(const float* W, int64_t N, int d, void
   const int n_chunks = (d + tc::KC - 1) / tc::KC;
   tc::prepare_weights_kernel<<<kNumSMs * 8, 256, 0, (cudaStream_t)stream>>>(W, N, d, n_chunks, (uint4*)prepared);
   IRS_LAUNCHED();
-  float* wmax2 = (float*)((char*)prepared + (size_t)ceil_div(N, tc::BN) * n_chunks * tc::STAGE_BYTES);
+  float* wmax2 = (float*)((char*)prepared + wmax2_offset(N, d));
   IRS_CUDA(cudaMemsetAsync(wmax2, 0, 256, (cudaStream_t)stream));
   tc::weight_norm_kernel<<<kNumSMs * 4, 256, 0, (cudaStream_t)stream>>>(W, N, d, wmax2);
   IRS_LAUNCHED();
   return 0;
 }
 
-extern "C" size_t irs_score_argmax_tc_workspace_bytes(int M, int64_t N, int d) {
-  if (M <= 0 || N <= 0 || d <= 0) return 0;
+// The checks every tensor-core scorer entry point shares.  dmax: the largest d its MMA path takes.  `need` is the
+// entry's workspace query, which returns 0 for the sizes rejected here.
+static int score_tc_check(const float* h, const float* W, const void* prepared, const int32_t* excl_sorted,
+                          const int32_t* excl_count, int Lx, int M, int64_t N, int d, int dmax,
+                          const void* workspace, size_t workspace_bytes, size_t need) {
+  if (!h || !W || !prepared || !workspace) return IRS_E_BADARG;
+  if (M <= 0 || N <= 0 || d <= 0) return IRS_E_BADARG;
+  if (d > dmax || N > 0x7ffffffe) return IRS_E_SHAPE;
+  if (excl_sorted && (!excl_count || Lx <= 0)) return IRS_E_BADARG;
+  if (workspace_bytes < need) return IRS_E_WORKSPACE;
+  return 0;
+}
+
+// The Params fields every mode of score_tc_kernel reads, and the catalog split of tc::plan.
+static tc::Params score_tc_params(const float* h, int64_t ld_h, const void* prepared, const float* bias,
+                                  const int32_t* excl_sorted, const int32_t* excl_count, int Lx, int M, int64_t N, int d) {
+  tc::Params p = {};
+  p.h = h; p.ld_h = ld_h; p.Wt = (const uint4*)prepared; p.bias = bias; p.M = M; p.N = N; p.d = d;
+  p.n_chunks = (d + tc::KC - 1) / tc::KC;
+  p.excl_sorted = excl_sorted; p.excl_count = excl_count; p.Lx = Lx;
+  p.wmax2 = (const float*)((const char*)prepared + wmax2_offset(N, d));
+  tc::plan(M, N, p.m_tiles, p.n_tiles, p.tiles_per_split, p.n_splits);
+  return p;
+}
+
+template <int MODE>
+static int score_tc_launch(const tc::Params& p, cudaStream_t s) {
+  IRS_CUDA(cudaMemsetAsync(p.error_flag, 0, sizeof(int), s));
+  IRS_CUDA(opt_in_smem(tc::score_tc_kernel<MODE>, tc::SMEM_BYTES));
+  tc::score_tc_kernel<MODE><<<(unsigned)(p.m_tiles * p.n_splits), tc::THREADS, tc::SMEM_BYTES, s>>>(p);
+  IRS_LAUNCHED();
+  return 0;
+}
+
+// arg-max workspace: 6 candidate keys per (row, split, segment), then the error flag
+struct ArgmaxTcLayout { int n_segs; size_t flag, total; };
+static ArgmaxTcLayout argmax_tc_layout(int M, int64_t N) {
   int m_tiles, n_splits; int64_t n_tiles, tps;
   tc::plan(M, N, m_tiles, n_tiles, tps, n_splits);
-  const size_t n_segs = (size_t)ceil_div(tps, (int64_t)tc::SEG_TILES);
-  return (((size_t)M * n_splits * n_segs * 6 * 8 + 255) & ~(size_t)255) + 256;
+  const int n_segs = (int)ceil_div(tps, (int64_t)tc::SEG_TILES);
+  const size_t flag = align256((size_t)M * n_splits * n_segs * 6 * 8);
+  return {n_segs, flag, flag + 256};
+}
+
+extern "C" size_t irs_score_argmax_tc_workspace_bytes(int M, int64_t N, int d) {
+  if (M <= 0 || N <= 0 || d <= 0) return 0;
+  return argmax_tc_layout(M, N).total;
 }
 
 // phase 0: score + re-score (one shard = the whole catalog); phase 1: score + per-row shard leader -> lead[M+1];
@@ -992,39 +1039,24 @@ static int argmax_tc_run(int phase, const float* h, int64_t ld_h, const float* W
                          int64_t item_base, const int32_t* excl_sorted, const int32_t* excl_count, int Lx,
                          float* lead, float* vals, int64_t* items, int M, int64_t N, int d, int variant,
                          void* workspace, size_t workspace_bytes, void* stream) {
-  if (!h || !W || !prepared || !workspace) return IRS_E_BADARG;
   if ((phase != 1 && (!vals || !items)) || (phase != 0 && !lead)) return IRS_E_BADARG;
-  if (M <= 0 || N <= 0 || d <= 0) return IRS_E_BADARG;
-  if (d > tc::KMAX_SINGLE || N > 0x7ffffffe) return IRS_E_SHAPE;
-  if (d > tc::KMAX && !(variant & 2)) return IRS_E_SHAPE;       // 128 < d <= 256: single-MMA variant only (no lo image of h)
-  if (excl_sorted && (!excl_count || Lx <= 0)) return IRS_E_BADARG;
-  if (workspace_bytes < irs_score_argmax_tc_workspace_bytes(M, N, d)) return IRS_E_WORKSPACE;
+  // 128 < d <= 256: single-MMA variant only (no lo image of h)
+  int rc = score_tc_check(h, W, prepared, excl_sorted, excl_count, Lx, M, N, d, (variant & 2) ? tc::KMAX_SINGLE : tc::KMAX,
+                          workspace, workspace_bytes, irs_score_argmax_tc_workspace_bytes(M, N, d));
+  if (rc) return rc;
   cudaStream_t s = (cudaStream_t)stream;
-  tc::Params p = {};
-  p.h = h; p.ld_h = ld_h; p.Wt = (const uint4*)prepared; p.bias = bias; p.M = M; p.N = N; p.d = d;
-  p.n_chunks = (d + tc::KC - 1) / tc::KC;
-  p.excl_sorted = excl_sorted; p.excl_count = excl_count; p.Lx = Lx;
-  tc::plan(M, N, p.m_tiles, p.n_tiles, p.tiles_per_split, p.n_splits);
-  p.n_segs = (int)ceil_div(p.tiles_per_split, (int64_t)tc::SEG_TILES);
+  tc::Params p = score_tc_params(h, ld_h, prepared, bias, excl_sorted, excl_count, Lx, M, N, d);
+  const ArgmaxTcLayout lay = argmax_tc_layout(M, N);
+  p.n_segs = lay.n_segs;
   p.slice_keys = (unsigned long long*)workspace;
-  p.error_flag = (int*)((char*)workspace + (((size_t)M * p.n_splits * p.n_segs * 6 * 8 + 255) & ~(size_t)255));
+  p.error_flag = (int*)((char*)workspace + lay.flag);
   p.variant = variant;
   p.timeline = g_scorer_timeline;
   p.single = (variant & 2) ? 1 : 0;
-  p.wmax2 = (const float*)((const char*)prepared + (size_t)ceil_div(N, tc::BN) * p.n_chunks * tc::STAGE_BYTES);
   // floor of the band, relative to the leader's score: covers the fp32 rounding of the bias addition in both scores
   p.band_rel = 1e-4f;
   const int n_cand = p.n_splits * p.n_segs * 6;
-  if (phase != 2) {
-    IRS_CUDA(cudaMemsetAsync(p.error_flag, 0, sizeof(int), s));
-    static bool configured = false;
-    if (!configured) {
-      IRS_CUDA(cudaFuncSetAttribute(tc::score_tc_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::SMEM_BYTES));
-      configured = true;
-    }
-    tc::score_tc_kernel<0><<<(unsigned)(p.m_tiles * p.n_splits), tc::THREADS, tc::SMEM_BYTES, s>>>(p);
-    IRS_LAUNCHED();
-  }
+  if (phase != 2 && (rc = score_tc_launch<0>(p, s))) return rc;
   if (phase == 1) {
     tc::approx_leader_kernel<<<(unsigned)ceil_div((int64_t)M * 32, 256), 256, 0, s>>>(p.slice_keys, n_cand, M, p.wmax2, lead);
     IRS_LAUNCHED();
@@ -1063,96 +1095,87 @@ extern "C" int irs_score_argmax_tc_phase2(const float* h, int64_t ld_h, const fl
                        items, M, N, d, variant, workspace, workspace_bytes, stream);
 }
 
-extern "C" size_t irs_score_lse_gather_tc_workspace_bytes(int M, int64_t N, int d) {
-  if (M <= 0 || N <= 0 || d <= 0) return 0;
+// log-sum-exp workspace: a (max, sum) pair per (row, split), then the error flag
+struct LseTcLayout { size_t flag, total; };
+static LseTcLayout lse_tc_layout(int M, int64_t N) {
   int m_tiles, n_splits; int64_t n_tiles, tps;
   tc::plan(M, N, m_tiles, n_tiles, tps, n_splits);
-  return (((size_t)M * n_splits * 2 * 8 + 255) & ~(size_t)255) + 256;
+  const size_t flag = align256((size_t)M * n_splits * 2 * 8);
+  return {flag, flag + 256};
+}
+
+extern "C" size_t irs_score_lse_gather_tc_workspace_bytes(int M, int64_t N, int d) {
+  if (M <= 0 || N <= 0 || d <= 0) return 0;
+  return lse_tc_layout(M, N).total;
 }
 
 extern "C" int irs_score_lse_gather_tc(const float* h, int64_t ld_h, const float* W, const void* prepared, const float* bias,
                                        int64_t item_base, const int64_t* sel, int n_sel, float* lse, float* logit,
                                        int M, int64_t N, int d, void* workspace, size_t workspace_bytes, void* stream) {
-  if (!h || !W || !prepared || !lse || !workspace) return IRS_E_BADARG;
-  if (M <= 0 || N <= 0 || d <= 0 || n_sel < 0 || (n_sel > 0 && (!sel || !logit))) return IRS_E_BADARG;
-  if (d > tc::KMAX || N > 0x7ffffffe) return IRS_E_SHAPE;
-  if (workspace_bytes < irs_score_lse_gather_tc_workspace_bytes(M, N, d)) return IRS_E_WORKSPACE;
+  if (!lse || n_sel < 0 || (n_sel > 0 && (!sel || !logit))) return IRS_E_BADARG;
+  int rc = score_tc_check(h, W, prepared, nullptr, nullptr, 0, M, N, d, tc::KMAX, workspace, workspace_bytes,
+                          irs_score_lse_gather_tc_workspace_bytes(M, N, d));
+  if (rc) return rc;
   cudaStream_t s = (cudaStream_t)stream;
-  tc::Params p = {};
-  p.h = h; p.ld_h = ld_h; p.Wt = (const uint4*)prepared; p.bias = bias; p.M = M; p.N = N; p.d = d;
-  p.n_chunks = (d + tc::KC - 1) / tc::KC;
-  tc::plan(M, N, p.m_tiles, p.n_tiles, p.tiles_per_split, p.n_splits);
+  tc::Params p = score_tc_params(h, ld_h, prepared, bias, nullptr, nullptr, 0, M, N, d);
   p.slice_ms = (float2*)workspace;
-  p.error_flag = (int*)((char*)workspace + (((size_t)M * p.n_splits * 2 * 8 + 255) & ~(size_t)255));
-  IRS_CUDA(cudaMemsetAsync(p.error_flag, 0, sizeof(int), s));
-  static bool configured = false;
-  if (!configured) {
-    IRS_CUDA(cudaFuncSetAttribute(tc::score_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::SMEM_BYTES));
-    configured = true;
-  }
-  tc::score_tc_kernel<1><<<(unsigned)(p.m_tiles * p.n_splits), tc::THREADS, tc::SMEM_BYTES, s>>>(p);
-  IRS_LAUNCHED();
+  p.error_flag = (int*)((char*)workspace + lse_tc_layout(M, N).flag);
+  if ((rc = score_tc_launch<1>(p, s))) return rc;
   tc::lse_finalize_kernel<<<(unsigned)ceil_div((int64_t)M * 32, 256), 256, 0, s>>>(
       p.slice_ms, p.n_splits * 2, h, ld_h, W, bias, M, N, d, item_base, sel, n_sel, lse, logit);
   IRS_LAUNCHED();
   return 0;
 }
 
-static size_t rank_ws_layout(int M, int n_splits, size_t& off_above, size_t& off_unsure, size_t& off_flag) {
-  auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-  size_t o = al((size_t)M * 4);                                   // label scores
-  off_above = o; o += al((size_t)M * n_splits * 2 * 4);
-  off_unsure = o; o += al((size_t)M * n_splits * 2 * (1 + tc::RCAP) * 4);
-  off_flag = o; o += 256;
-  return o;
+// rank / count-ahead workspace: the label scores, then per (row, split) the columns surely ahead and the list of
+// uncertain ones, then the error flag
+struct RankTcLayout { size_t above, unsure, flag, total; };
+static RankTcLayout rank_tc_layout(int M, int64_t N) {
+  int m_tiles, n_splits; int64_t n_tiles, tps;
+  tc::plan(M, N, m_tiles, n_tiles, tps, n_splits);
+  const size_t above = align256((size_t)M * 4);
+  const size_t unsure = above + align256((size_t)M * n_splits * 2 * 4);
+  const size_t flag = unsure + align256((size_t)M * n_splits * 2 * (1 + tc::RCAP) * 4);
+  return {above, unsure, flag, flag + 256};
 }
 
 extern "C" size_t irs_score_rank_tc_workspace_bytes(int M, int64_t N, int d) {
   if (M <= 0 || N <= 0 || d <= 0) return 0;
-  int m_tiles, n_splits; int64_t n_tiles, tps;
-  tc::plan(M, N, m_tiles, n_tiles, tps, n_splits);
-  size_t a, b, c;
-  return rank_ws_layout(M, n_splits, a, b, c);
+  return rank_tc_layout(M, N).total;
+}
+
+// Counts, per row, the live columns ahead of label_score[m].  label_excluded null: writes the rank (0 when the label
+// is excluded or outside the catalog); otherwise the shard's count and whether the label is excluded here.
+static int rank_tc_run(tc::Params p, const float* W, int64_t item_base, const int64_t* label, const float* label_score,
+                       int64_t* out, int32_t* label_excluded, void* workspace, cudaStream_t s) {
+  const RankTcLayout lay = rank_tc_layout(p.M, p.N);
+  p.label_score = label_score;
+  p.rank_above = (int*)((char*)workspace + lay.above);
+  p.rank_unsure = (int*)((char*)workspace + lay.unsure);
+  p.error_flag = (int*)((char*)workspace + lay.flag);
+  const int rc = score_tc_launch<2>(p, s);
+  if (rc) return rc;
+  tc::rank_finalize_tc_kernel<<<(unsigned)ceil_div((int64_t)p.M * 32, 256), 256, 0, s>>>(
+      p.rank_above, p.rank_unsure, p.n_splits, p.tiles_per_split, label_score, label, p.h, p.ld_h, W, p.bias, p.M, p.N, p.d,
+      item_base, p.excl_sorted, p.excl_count, p.Lx, out, label_excluded);
+  IRS_LAUNCHED();
+  return 0;
 }
 
 extern "C" int irs_score_rank_tc(const float* h, int64_t ld_h, const float* W, const void* prepared, const float* bias,
                                  int64_t item_base, const int64_t* label, const int32_t* excl_sorted, const int32_t* excl_count,
                                  int Lx, int64_t* rank, int M, int64_t N, int d,
                                  void* workspace, size_t workspace_bytes, void* stream) {
-  if (!h || !W || !prepared || !label || !rank || !workspace) return IRS_E_BADARG;
-  if (M <= 0 || N <= 0 || d <= 0) return IRS_E_BADARG;
-  if (d > tc::KMAX || N > 0x7ffffffe) return IRS_E_SHAPE;
-  if (excl_sorted && (!excl_count || Lx <= 0)) return IRS_E_BADARG;
-  if (workspace_bytes < irs_score_rank_tc_workspace_bytes(M, N, d)) return IRS_E_WORKSPACE;
+  if (!label || !rank) return IRS_E_BADARG;
+  const int rc = score_tc_check(h, W, prepared, excl_sorted, excl_count, Lx, M, N, d, tc::KMAX, workspace, workspace_bytes,
+                                irs_score_rank_tc_workspace_bytes(M, N, d));
+  if (rc) return rc;
   cudaStream_t s = (cudaStream_t)stream;
-  tc::Params p = {};
-  p.h = h; p.ld_h = ld_h; p.Wt = (const uint4*)prepared; p.bias = bias; p.M = M; p.N = N; p.d = d;
-  p.n_chunks = (d + tc::KC - 1) / tc::KC;
-  p.excl_sorted = excl_sorted; p.excl_count = excl_count; p.Lx = Lx;
-  tc::plan(M, N, p.m_tiles, p.n_tiles, p.tiles_per_split, p.n_splits);
-  size_t off_above, off_unsure, off_flag;
-  rank_ws_layout(M, p.n_splits, off_above, off_unsure, off_flag);
   float* lab_s = (float*)workspace;
-  p.label_score = lab_s;
-  p.rank_above = (int*)((char*)workspace + off_above);
-  p.rank_unsure = (int*)((char*)workspace + off_unsure);
-  p.error_flag = (int*)((char*)workspace + off_flag);
-  p.wmax2 = (const float*)((const char*)prepared + (size_t)ceil_div(N, tc::BN) * p.n_chunks * tc::STAGE_BYTES);
-  IRS_CUDA(cudaMemsetAsync(p.error_flag, 0, sizeof(int), s));
   tc::rank_label_score_kernel<<<(unsigned)ceil_div(M, 256), 256, 0, s>>>(h, ld_h, W, bias, label, item_base, M, N, d, lab_s);
   IRS_LAUNCHED();
-  static bool configured = false;
-  if (!configured) {
-    IRS_CUDA(cudaFuncSetAttribute(tc::score_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::SMEM_BYTES));
-    configured = true;
-  }
-  tc::score_tc_kernel<2><<<(unsigned)(p.m_tiles * p.n_splits), tc::THREADS, tc::SMEM_BYTES, s>>>(p);
-  IRS_LAUNCHED();
-  tc::rank_finalize_tc_kernel<<<(unsigned)ceil_div((int64_t)M * 32, 256), 256, 0, s>>>(
-      p.rank_above, p.rank_unsure, p.n_splits, p.tiles_per_split, lab_s, label, h, ld_h, W, bias, M, N, d, item_base,
-      excl_sorted, excl_count, Lx, rank, nullptr);
-  IRS_LAUNCHED();
-  return 0;
+  return rank_tc_run(score_tc_params(h, ld_h, prepared, bias, excl_sorted, excl_count, Lx, M, N, d), W, item_base, label,
+                     lab_s, rank, nullptr, workspace, s);
 }
 
 extern "C" int irs_score_count_ahead_tc(const float* h, int64_t ld_h, const float* W, const void* prepared, const float* bias,
@@ -1160,85 +1183,48 @@ extern "C" int irs_score_count_ahead_tc(const float* h, int64_t ld_h, const floa
                                         const int32_t* excl_sorted, const int32_t* excl_count, int Lx,
                                         int64_t* count, int32_t* label_excluded, int M, int64_t N, int d,
                                         void* workspace, size_t workspace_bytes, void* stream) {
-  if (!h || !W || !prepared || !label || !label_score || !count || !label_excluded || !workspace) return IRS_E_BADARG;
-  if (M <= 0 || N <= 0 || d <= 0) return IRS_E_BADARG;
-  if (d > tc::KMAX || N > 0x7ffffffe) return IRS_E_SHAPE;
-  if (excl_sorted && (!excl_count || Lx <= 0)) return IRS_E_BADARG;
-  if (workspace_bytes < irs_score_rank_tc_workspace_bytes(M, N, d)) return IRS_E_WORKSPACE;
-  cudaStream_t s = (cudaStream_t)stream;
-  tc::Params p = {};
-  p.h = h; p.ld_h = ld_h; p.Wt = (const uint4*)prepared; p.bias = bias; p.M = M; p.N = N; p.d = d;
-  p.n_chunks = (d + tc::KC - 1) / tc::KC;
-  p.excl_sorted = excl_sorted; p.excl_count = excl_count; p.Lx = Lx;
-  tc::plan(M, N, p.m_tiles, p.n_tiles, p.tiles_per_split, p.n_splits);
-  size_t off_above, off_unsure, off_flag;
-  rank_ws_layout(M, p.n_splits, off_above, off_unsure, off_flag);
-  p.label_score = label_score;                         // the owning shard's exact fp32 score, given from outside
-  p.rank_above = (int*)((char*)workspace + off_above);
-  p.rank_unsure = (int*)((char*)workspace + off_unsure);
-  p.error_flag = (int*)((char*)workspace + off_flag);
-  p.wmax2 = (const float*)((const char*)prepared + (size_t)ceil_div(N, tc::BN) * p.n_chunks * tc::STAGE_BYTES);
-  IRS_CUDA(cudaMemsetAsync(p.error_flag, 0, sizeof(int), s));
-  static bool configured = false;
-  if (!configured) {
-    IRS_CUDA(cudaFuncSetAttribute(tc::score_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::SMEM_BYTES));
-    configured = true;
-  }
-  tc::score_tc_kernel<2><<<(unsigned)(p.m_tiles * p.n_splits), tc::THREADS, tc::SMEM_BYTES, s>>>(p);
-  IRS_LAUNCHED();
-  tc::rank_finalize_tc_kernel<<<(unsigned)ceil_div((int64_t)M * 32, 256), 256, 0, s>>>(
-      p.rank_above, p.rank_unsure, p.n_splits, p.tiles_per_split, label_score, label, h, ld_h, W, bias, M, N, d, item_base,
-      excl_sorted, excl_count, Lx, count, label_excluded);
-  IRS_LAUNCHED();
-  return 0;
+  if (!label || !label_score || !count || !label_excluded) return IRS_E_BADARG;
+  const int rc = score_tc_check(h, W, prepared, excl_sorted, excl_count, Lx, M, N, d, tc::KMAX, workspace, workspace_bytes,
+                                irs_score_rank_tc_workspace_bytes(M, N, d));
+  if (rc) return rc;
+  // the owning shard's exact fp32 score, given from outside
+  return rank_tc_run(score_tc_params(h, ld_h, prepared, bias, excl_sorted, excl_count, Lx, M, N, d), W, item_base, label,
+                     label_score, count, label_excluded, workspace, (cudaStream_t)stream);
 }
 
 
 // ---- top-k (k > 1) on the tensor cores ----------------------------------------------------------------------------------
-static size_t topk_tc_ws_layout(int M, int64_t N, size_t& off_flag, int64_t& ld_cm) {
-  ld_cm = ceil_div(N, (int64_t)tc::BN) * (tc::BN / 32);
-  size_t o = ((size_t)M * (size_t)ld_cm * 4 + 255) & ~(size_t)255;
-  off_flag = o;
-  return o + 256;
+// workspace: the best score of every 32-column chunk, [M, ld_cm] floats, then the error flag
+struct TopkTcLayout { int64_t ld_cm; size_t flag, total; };
+static TopkTcLayout topk_tc_layout(int M, int64_t N) {
+  const int64_t ld_cm = ceil_div(N, (int64_t)tc::BN) * (tc::BN / 32);
+  const size_t flag = align256((size_t)M * (size_t)ld_cm * 4);
+  return {ld_cm, flag, flag + 256};
 }
 
 extern "C" size_t irs_score_topk_tc_workspace_bytes(int M, int64_t N, int d, int k) {
   if (M <= 0 || N <= 0 || d <= 0 || k <= 0) return 0;
-  size_t off; int64_t ld;
-  return topk_tc_ws_layout(M, N, off, ld);
+  return topk_tc_layout(M, N).total;
 }
 
 extern "C" int irs_score_topk_tc(const float* h, int64_t ld_h, const float* W, const void* prepared, const float* bias,
                                  int64_t item_base, const int32_t* excl_sorted, const int32_t* excl_count, int Lx, int k,
                                  float* vals, int64_t* items, int M, int64_t N, int d,
                                  void* workspace, size_t workspace_bytes, void* stream) {
-  if (!h || !W || !prepared || !vals || !items || !workspace) return IRS_E_BADARG;
-  if (M <= 0 || N <= 0 || d <= 0 || k < 1 || k > 1024) return IRS_E_BADARG;
-  if (d > tc::KMAX_SINGLE || N > 0x7ffffffe) return IRS_E_SHAPE;
-  if (excl_sorted && (!excl_count || Lx <= 0)) return IRS_E_BADARG;
-  if (workspace_bytes < irs_score_topk_tc_workspace_bytes(M, N, d, k)) return IRS_E_WORKSPACE;
+  if (!vals || !items || k < 1 || k > 1024) return IRS_E_BADARG;
+  int rc = score_tc_check(h, W, prepared, excl_sorted, excl_count, Lx, M, N, d, tc::KMAX_SINGLE, workspace, workspace_bytes,
+                          irs_score_topk_tc_workspace_bytes(M, N, d, k));
+  if (rc) return rc;
   cudaStream_t s = (cudaStream_t)stream;
-  tc::Params p = {};
-  p.h = h; p.ld_h = ld_h; p.Wt = (const uint4*)prepared; p.bias = bias; p.M = M; p.N = N; p.d = d;
-  p.n_chunks = (d + tc::KC - 1) / tc::KC;
-  p.excl_sorted = excl_sorted; p.excl_count = excl_count; p.Lx = Lx;
-  tc::plan(M, N, p.m_tiles, p.n_tiles, p.tiles_per_split, p.n_splits);
-  size_t off_flag;
-  topk_tc_ws_layout(M, N, off_flag, p.ld_cm);
+  tc::Params p = score_tc_params(h, ld_h, prepared, bias, excl_sorted, excl_count, Lx, M, N, d);
+  const TopkTcLayout lay = topk_tc_layout(M, N);
+  p.ld_cm = lay.ld_cm;
   p.chunk_max = (float*)workspace;
-  p.error_flag = (int*)((char*)workspace + off_flag);
+  p.error_flag = (int*)((char*)workspace + lay.flag);
   p.single = 1;
   p.variant = 2;
   p.band_rel = 1e-4f;
-  p.wmax2 = (const float*)((const char*)prepared + (size_t)ceil_div(N, tc::BN) * p.n_chunks * tc::STAGE_BYTES);
-  IRS_CUDA(cudaMemsetAsync(p.error_flag, 0, sizeof(int), s));
-  static bool configured = false;
-  if (!configured) {
-    IRS_CUDA(cudaFuncSetAttribute(tc::score_tc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::SMEM_BYTES));
-    configured = true;
-  }
-  tc::score_tc_kernel<3><<<(unsigned)(p.m_tiles * p.n_splits), tc::THREADS, tc::SMEM_BYTES, s>>>(p);
-  IRS_LAUNCHED();
+  if ((rc = score_tc_launch<3>(p, s))) return rc;
   tc::topk_select_kernel<<<(unsigned)M, 256, 0, s>>>(p.chunk_max, p.ld_cm, p.ld_cm, h, ld_h, W, bias, M, N, d, item_base,
                                                    p.band_rel, p.wmax2, excl_sorted, excl_count, Lx, k, vals, items);
   IRS_LAUNCHED();

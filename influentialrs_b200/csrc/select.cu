@@ -339,42 +339,49 @@ static int cand_cap_for(int k) {
   return c;
 }
 
-static int score_common_check(const float* h, const float* W, int M, int64_t N, int d) {
+// The checks every fp32 scorer entry point shares, in the order of their error codes.  args_ok: the entry's own pointer
+// and size arguments are valid.  `need` is the entry's workspace query, which returns 0 for the sizes rejected here.
+static int score_check(const float* h, const float* W, int M, int64_t N, int d, bool args_ok,
+                       const int32_t* excl_sorted, const int32_t* excl_count, int Lx, size_t workspace_bytes, size_t need) {
   if (!h || !W) return IRS_E_BADARG;
   if (M <= 0 || N <= 0 || d <= 0) return IRS_E_BADARG;
   if (N > 0x7ffffffe) return IRS_E_SHAPE;
+  if (!args_ok) return IRS_E_BADARG;
+  if (excl_sorted && (!excl_count || Lx <= 0)) return IRS_E_BADARG;
+  if (workspace_bytes < need) return IRS_E_WORKSPACE;
   return 0;
+}
+
+// top-k workspace: the slice keys; for k > 1 (16 slice keys per split) the per-row thresholds, candidate counts and
+// candidate keys follow
+struct TopkLayout { size_t thr, cnt, cand, total; };
+static TopkLayout topk_layout(int M, int64_t N, int k) {
+  const int splits = score_simt_max_splits(M, N);
+  const size_t thr = align256((size_t)M * splits * 16 * 8);
+  const size_t cnt = thr + align256((size_t)M * 8);
+  const size_t cand = cnt + align256((size_t)M * 4);
+  return {thr, cnt, cand, k == 1 ? align256((size_t)M * splits * 8) : cand + align256((size_t)M * cand_cap_for(k) * 8)};
 }
 
 extern "C" size_t irs_score_topk_workspace_bytes(int M, int64_t N, int d, int k) {
   (void)d;
   if (M <= 0 || N <= 0 || k <= 0) return 0;
-  const int splits = score_simt_max_splits(M, N);
-  if (k == 1) return align256((size_t)M * splits * 8);
-  size_t b = align256((size_t)M * splits * 16 * 8);      // slice keys
-  b += align256((size_t)M * 8);                          // thresholds
-  b += align256((size_t)M * 4);                          // candidate counts
-  b += align256((size_t)M * cand_cap_for(k) * 8);        // candidate keys
-  return b;
+  return topk_layout(M, N, k).total;
 }
 
 extern "C" int irs_score_topk(const float* h, int64_t ld_h, const float* W, const float* bias, int64_t item_base,
                               const int32_t* excl_sorted, const int32_t* excl_count, int Lx, int k,
                               float* vals, int64_t* items, int M, int64_t N, int d,
                               void* workspace, size_t workspace_bytes, void* stream) {
-  int rc = score_common_check(h, W, M, N, d);
+  int rc = score_check(h, W, M, N, d, vals && items && workspace && k >= 1 && k <= 1024, excl_sorted, excl_count, Lx,
+                       workspace_bytes, irs_score_topk_workspace_bytes(M, N, d, k));
   if (rc) return rc;
-  if (!vals || !items || !workspace || k < 1 || k > 1024) return IRS_E_BADARG;
-  if (excl_sorted && (!excl_count || Lx <= 0)) return IRS_E_BADARG;
-  if (workspace_bytes < irs_score_topk_workspace_bytes(M, N, d, k)) return IRS_E_WORKSPACE;
   cudaStream_t s = (cudaStream_t)stream;
   ScoreParams p = {};
   p.h = h; p.ld_h = ld_h; p.W = W; p.bias = bias; p.M = M; p.N = N; p.d = d; p.item_base = item_base;
   p.excl_sorted = excl_sorted; p.excl_count = excl_count; p.Lx = Lx;
-  char* ws = (char*)workspace;
-  const int splits = score_simt_max_splits(M, N);
-  p.max_splits = splits;
-  p.slice_keys = (unsigned long long*)ws;
+  p.max_splits = score_simt_max_splits(M, N);
+  p.slice_keys = (unsigned long long*)workspace;
   if (k == 1) {
     p.slices_per_split = 1;
     rc = launch_score_simt(MODE_MAX, p, s);
@@ -383,10 +390,10 @@ extern "C" int irs_score_topk(const float* h, int64_t ld_h, const float* W, cons
     IRS_LAUNCHED();
     return 0;
   }
-  ws += align256((size_t)M * splits * 16 * 8);
-  unsigned long long* thr = (unsigned long long*)ws; ws += align256((size_t)M * 8);
-  int* cnt = (int*)ws; ws += align256((size_t)M * 4);
-  unsigned long long* cand = (unsigned long long*)ws;
+  const TopkLayout lay = topk_layout(M, N, k);
+  unsigned long long* thr = (unsigned long long*)((char*)workspace + lay.thr);
+  int* cnt = (int*)((char*)workspace + lay.cnt);
+  unsigned long long* cand = (unsigned long long*)((char*)workspace + lay.cand);
   const int cap = cand_cap_for(k);
   p.slices_per_split = 16;
   if (p.max_splits > 256) p.max_splits = 256;       // the threshold kernel sorts <= 4096 slice keys per row (few rows x large catalog)
@@ -404,64 +411,32 @@ extern "C" int irs_score_topk(const float* h, int64_t ld_h, const float* W, cons
   return 0;
 }
 
+// log-sum-exp workspace: the per-(row, split) maxima, then the sums
+static size_t lse_sum_offset(int M, int64_t N) { return align256((size_t)M * score_simt_max_splits(M, N) * 4); }
+
 extern "C" size_t irs_score_lse_gather_workspace_bytes(int M, int64_t N, int d, int n_sel) {
   (void)d; (void)n_sel;
   if (M <= 0 || N <= 0) return 0;
-  return 2 * align256((size_t)M * score_simt_max_splits(M, N) * 4);
+  return 2 * lse_sum_offset(M, N);
 }
 
 extern "C" int irs_score_lse_gather(const float* h, int64_t ld_h, const float* W, const float* bias, int64_t item_base,
                                     const int64_t* sel, int n_sel, float* lse, float* logit,
                                     int M, int64_t N, int d, void* workspace, size_t workspace_bytes, void* stream) {
-  int rc = score_common_check(h, W, M, N, d);
+  int rc = score_check(h, W, M, N, d, lse && workspace && n_sel >= 0 && (n_sel == 0 || (sel && logit)), nullptr, nullptr, 0,
+                       workspace_bytes, irs_score_lse_gather_workspace_bytes(M, N, d, n_sel));
   if (rc) return rc;
-  if (!lse || !workspace || n_sel < 0 || (n_sel > 0 && (!sel || !logit))) return IRS_E_BADARG;
-  if (workspace_bytes < irs_score_lse_gather_workspace_bytes(M, N, d, n_sel)) return IRS_E_WORKSPACE;
   cudaStream_t s = (cudaStream_t)stream;
   ScoreParams p = {};
   p.h = h; p.ld_h = ld_h; p.W = W; p.bias = bias; p.M = M; p.N = N; p.d = d; p.item_base = item_base;
-  const int splits = score_simt_max_splits(M, N);
-  p.max_splits = splits;
+  p.max_splits = score_simt_max_splits(M, N);
   p.part_max = (float*)workspace;
-  p.part_sum = (float*)((char*)workspace + align256((size_t)M * splits * 4));
+  p.part_sum = (float*)((char*)workspace + lse_sum_offset(M, N));
   p.sel = sel; p.n_sel = n_sel; p.sel_logit = logit;
   if (n_sel > 0) IRS_CUDA(cudaMemsetAsync(logit, 0, (size_t)M * n_sel * 4, s));
   rc = launch_score_simt(MODE_LSE, p, s);
   if (rc) return rc;
   lse_finalize_kernel<<<(unsigned)ceil_div(M, 256), 256, 0, s>>>(p.part_max, p.part_sum, p.n_splits, M, lse);
-  IRS_LAUNCHED();
-  return 0;
-}
-
-extern "C" size_t irs_score_rank_workspace_bytes(int M, int64_t N, int d) {
-  (void)N; (void)d;
-  if (M <= 0) return 0;
-  return 3 * align256((size_t)M * 4);
-}
-
-extern "C" int irs_score_rank(const float* h, int64_t ld_h, const float* W, const float* bias, int64_t item_base,
-                              const int64_t* label, const int32_t* excl_sorted, const int32_t* excl_count, int Lx,
-                              int64_t* rank, int M, int64_t N, int d,
-                              void* workspace, size_t workspace_bytes, void* stream) {
-  int rc = score_common_check(h, W, M, N, d);
-  if (rc) return rc;
-  if (!label || !rank || !workspace) return IRS_E_BADARG;
-  if (excl_sorted && (!excl_count || Lx <= 0)) return IRS_E_BADARG;
-  if (workspace_bytes < irs_score_rank_workspace_bytes(M, N, d)) return IRS_E_WORKSPACE;
-  cudaStream_t s = (cudaStream_t)stream;
-  char* ws = (char*)workspace;
-  float* lab_s = (float*)ws; ws += align256((size_t)M * 4);
-  int* cnt = (int*)ws; ws += align256((size_t)M * 4);
-  int* exc = (int*)ws;
-  label_score_kernel<<<(unsigned)ceil_div(M, 256), 256, 0, s>>>(h, ld_h, W, bias, label, item_base, M, N, d, lab_s, cnt, exc);
-  IRS_LAUNCHED();
-  ScoreParams p = {};
-  p.h = h; p.ld_h = ld_h; p.W = W; p.bias = bias; p.M = M; p.N = N; p.d = d; p.item_base = item_base;
-  p.excl_sorted = excl_sorted; p.excl_count = excl_count; p.Lx = Lx;
-  p.label = label; p.label_score = lab_s; p.rank_count = cnt; p.rank_excluded = exc;
-  rc = launch_score_simt(MODE_RANK, p, s);
-  if (rc) return rc;
-  rank_finalize_kernel<<<(unsigned)ceil_div(M, 256), 256, 0, s>>>(cnt, exc, M, rank);
   IRS_LAUNCHED();
   return 0;
 }
@@ -496,18 +471,61 @@ count_finalize_kernel(const int* __restrict__ cnt, const int* __restrict__ exc, 
 
 extern "C" int irs_score_select(const float* h, int64_t ld_h, const float* W, const float* bias, int64_t item_base,
                                 const int64_t* sel, int n_sel, float* out, int M, int64_t N, int d, void* stream) {
-  int rc = score_common_check(h, W, M, N, d);
+  const int rc = score_check(h, W, M, N, d, sel && out && n_sel > 0, nullptr, nullptr, 0, 0, 0);
   if (rc) return rc;
-  if (!sel || !out || n_sel <= 0) return IRS_E_BADARG;
   score_select_kernel<<<(unsigned)ceil_div((int64_t)M * n_sel, 256), 256, 0, (cudaStream_t)stream>>>(
       h, ld_h, W, bias, item_base, sel, n_sel, out, M, N, d);
   IRS_LAUNCHED();
   return 0;
 }
 
+// rank / count-ahead workspace: slot 0 the per-row counts, slot 1 the label-excluded flags, slot 2 (rank only) the
+// label scores
+static size_t rank_slot(int M) { return align256((size_t)M * 4); }
+
+extern "C" size_t irs_score_rank_workspace_bytes(int M, int64_t N, int d) {
+  (void)N; (void)d;
+  return M > 0 ? 3 * rank_slot(M) : 0;
+}
+
 extern "C" size_t irs_score_count_ahead_workspace_bytes(int M, int64_t N, int d) {
   (void)N; (void)d;
-  return M > 0 ? 2 * align256((size_t)M * 4) : 0;
+  return M > 0 ? 2 * rank_slot(M) : 0;
+}
+
+// Counts, per row, the live columns ahead of label_score[m] into slot 0 (slot 1: the label is excluded); the caller has
+// initialised both.  label_excluded null: writes the rank; otherwise the shard's count and label-excluded flags.
+static int rank_run(const float* h, int64_t ld_h, const float* W, const float* bias, int64_t item_base,
+                    const int64_t* label, const float* label_score, const int32_t* excl_sorted, const int32_t* excl_count,
+                    int Lx, int M, int64_t N, int d, void* workspace, int64_t* out, int32_t* label_excluded, cudaStream_t s) {
+  int* cnt = (int*)workspace;
+  int* exc = (int*)((char*)workspace + rank_slot(M));
+  ScoreParams p = {};
+  p.h = h; p.ld_h = ld_h; p.W = W; p.bias = bias; p.M = M; p.N = N; p.d = d; p.item_base = item_base;
+  p.excl_sorted = excl_sorted; p.excl_count = excl_count; p.Lx = Lx;
+  p.label = label; p.label_score = label_score; p.rank_count = cnt; p.rank_excluded = exc;
+  const int rc = launch_score_simt(MODE_RANK, p, s);
+  if (rc) return rc;
+  if (label_excluded) count_finalize_kernel<<<(unsigned)ceil_div(M, 256), 256, 0, s>>>(cnt, exc, M, out, label_excluded);
+  else rank_finalize_kernel<<<(unsigned)ceil_div(M, 256), 256, 0, s>>>(cnt, exc, M, out);
+  IRS_LAUNCHED();
+  return 0;
+}
+
+extern "C" int irs_score_rank(const float* h, int64_t ld_h, const float* W, const float* bias, int64_t item_base,
+                              const int64_t* label, const int32_t* excl_sorted, const int32_t* excl_count, int Lx,
+                              int64_t* rank, int M, int64_t N, int d,
+                              void* workspace, size_t workspace_bytes, void* stream) {
+  const int rc = score_check(h, W, M, N, d, label && rank && workspace, excl_sorted, excl_count, Lx, workspace_bytes,
+                             irs_score_rank_workspace_bytes(M, N, d));
+  if (rc) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  char* ws = (char*)workspace;
+  float* lab_s = (float*)(ws + 2 * rank_slot(M));
+  label_score_kernel<<<(unsigned)ceil_div(M, 256), 256, 0, s>>>(h, ld_h, W, bias, label, item_base, M, N, d, lab_s,
+                                                                (int*)ws, (int*)(ws + rank_slot(M)));
+  IRS_LAUNCHED();
+  return rank_run(h, ld_h, W, bias, item_base, label, lab_s, excl_sorted, excl_count, Lx, M, N, d, workspace, rank, nullptr, s);
 }
 
 extern "C" int irs_score_count_ahead(const float* h, int64_t ld_h, const float* W, const float* bias, int64_t item_base,
@@ -515,25 +533,13 @@ extern "C" int irs_score_count_ahead(const float* h, int64_t ld_h, const float* 
                                      const int32_t* excl_sorted, const int32_t* excl_count, int Lx,
                                      int64_t* count, int32_t* label_excluded, int M, int64_t N, int d,
                                      void* workspace, size_t workspace_bytes, void* stream) {
-  int rc = score_common_check(h, W, M, N, d);
+  const int rc = score_check(h, W, M, N, d, label && label_score && count && label_excluded && workspace, excl_sorted,
+                             excl_count, Lx, workspace_bytes, irs_score_count_ahead_workspace_bytes(M, N, d));
   if (rc) return rc;
-  if (!label || !label_score || !count || !label_excluded || !workspace) return IRS_E_BADARG;
-  if (excl_sorted && (!excl_count || Lx <= 0)) return IRS_E_BADARG;
-  if (workspace_bytes < irs_score_count_ahead_workspace_bytes(M, N, d)) return IRS_E_WORKSPACE;
   cudaStream_t s = (cudaStream_t)stream;
-  char* ws = (char*)workspace;
-  int* cnt = (int*)ws; ws += align256((size_t)M * 4);
-  int* exc = (int*)ws;
-  IRS_CUDA(cudaMemsetAsync(workspace, 0, 2 * align256((size_t)M * 4), s));
-  ScoreParams p = {};
-  p.h = h; p.ld_h = ld_h; p.W = W; p.bias = bias; p.M = M; p.N = N; p.d = d; p.item_base = item_base;
-  p.excl_sorted = excl_sorted; p.excl_count = excl_count; p.Lx = Lx;
-  p.label = label; p.label_score = label_score; p.rank_count = cnt; p.rank_excluded = exc;
-  rc = launch_score_simt(MODE_RANK, p, s);
-  if (rc) return rc;
-  count_finalize_kernel<<<(unsigned)ceil_div(M, 256), 256, 0, s>>>(cnt, exc, M, count, label_excluded);
-  IRS_LAUNCHED();
-  return 0;
+  IRS_CUDA(cudaMemsetAsync(workspace, 0, 2 * rank_slot(M), s));
+  return rank_run(h, ld_h, W, bias, item_base, label, label_score, excl_sorted, excl_count, Lx, M, N, d, workspace, count,
+                  label_excluded, s);
 }
 
 extern "C" int irs_topk_merge(const float* vals, const int64_t* items, int G, int M, int k,
